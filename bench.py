@@ -124,6 +124,41 @@ def measured_traffic(cfg, kernel):
         return None, None
 
 
+DUMP_MAX = 1 << 21  # elements per array written by --dump-outputs (16 MB of float64; at most three arrays per run)
+
+
+def dump_rows(n_rows, ncols):
+    """Global row indices that --dump-outputs keeps of an n_rows x ncols output: all of them when the output fits
+    DUMP_MAX, else a fixed, seeded sample (the same for every build and every sharding)."""
+    k = max(1, DUMP_MAX // max(1, ncols))
+    if n_rows <= k:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(0).choice(n_rows, size=k, replace=False))
+
+
+def write_outputs(outdir, rank, world, lo, hi, N, sharded, whole):
+    """--dump-outputs: `sharded` maps names to this rank's rows [lo, hi) of an N-row output, `whole` to outputs that
+    every rank holds in full.  Rank 0 writes each as DIR/<name>.npy in float64, rows sampled by dump_rows."""
+    arrays = {}
+    for name, a in sharded.items():
+        a = np.asarray(a, dtype=np.float64)
+        idx = dump_rows(N, a.size // max(1, a.shape[0]))
+        part = a[idx[(idx >= lo) & (idx < hi)] - lo]
+        if world > 1:
+            import torch.distributed as dist
+            parts = [None] * world if rank == 0 else None
+            dist.gather_object(part, parts, dst=0)
+            part = np.concatenate(parts) if rank == 0 else None
+        arrays[name] = part
+    if rank != 0:
+        return
+    arrays.update((name, np.asarray(a, dtype=np.float64)) for name, a in whole.items())
+    outdir = Path(outdir)
+    outdir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(outdir / f"{name}.npy", a)
+
+
 def term_stats(terms):
     nnz = (terms > 0).sum(1)
     return int((nnz + 1).sum()), int(terms.max(0).sum())
@@ -249,7 +284,7 @@ def hbm_peak():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
-def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
+def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols, lo, hi):
     """c5: Phi.A with 64 right-hand sides (prodmm_(mat), src/linalg.cpp:527-557) and its transpose; build: the basis
     rebuild with gradients (outerbase::build, src/modandbase.cpp:547-626).  Same JSON contract, own metric."""
     import torch
@@ -295,6 +330,8 @@ def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
         barrier()
         ms_mm, l1 = timed(f_mm, args.steps)
         ms_tm, l2 = timed(f_tm, args.steps)
+        if args.dump_outputs:  # the last timed products: Phi.A (column-major, leading dimension nloc) and Phi^T.R (K x C)
+            dumped = ({"phi_a_mat": out[:Ccols * nloc].view(Ccols, nloc).T.cpu().numpy()}, {"phi_t_mat": G.view(Ccols, K).T.cpu().numpy()})
         # e2e: host matrices in, host results out, every call
         Ah = np.asfortranarray(rng.normal(size=(K, Ccols))); Rh = np.asfortranarray(rng.normal(size=(nloc, Ccols)))
         ob.matmul(terms, Ah); barrier()
@@ -303,6 +340,8 @@ def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
             ob.matmul(terms, Ah)
         barrier(); e2e_ms = (time.perf_counter() - t0) / n_e2e * 1e3
         clk = clocks.stop() if clocks else None
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, rank, world, lo, hi, N, *dumped)
         if rank != 0:
             return
         flop = 2.0 * (-(-N // world)) * K * Ccols
@@ -335,6 +374,8 @@ def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
     barrier()
     ms = (time.perf_counter() - t0) / args.steps * 1e3
     launches = lib.launch_count() - n0
+    if args.dump_outputs:  # the basis the last timed rebuild left in the object
+        dumped = ({"basemat": ob.real("basemat"), "basescale": ob.real("basescale")}, {})
     # what a BFGS objective evaluation pays (R/outersupport.R:215-216 -> loglik_gauss::updateom): the same rebuild on the
     # columns the terms table reads (compact layout, DESIGN 2)
     yv = wingweight(x); yv = (yv - yv.mean()) / yv.std(ddof=1)
@@ -348,6 +389,8 @@ def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
     barrier()
     ms_pruned = (time.perf_counter() - t0) / args.steps * 1e3
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, rank, world, lo, hi, N, *dumped)
     if rank != 0:
         return
     d, H, M, nge = om.sizes()
@@ -375,7 +418,9 @@ def run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the measured path (--impl reference stops after 90 s; the e2e and optcg "
+                         "side measurements use their own counts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--rows", type=int, default=0, help="total rows over all ranks (default: the configuration's)")
@@ -384,7 +429,14 @@ def main():
     ap.add_argument("--no-optcg", action="store_true")
     ap.add_argument("--spec", default="1", choices=["0", "1"],
                     help="1: terms-specialised kernels, compiled during set-up (default); 0: interpreter kernels only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64; outputs "
+                         "above 2M elements as a fixed, seeded sample of their rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path computed: not available with --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
@@ -418,7 +470,7 @@ def main():
     x = config_rows(cfg, lo, hi)
     lib.set_option("spec", float(args.spec))
     if cfg in ("c5", "build"):
-        run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols)
+        run_special(args, lib, om, terms, x, cfg, rank, world, local, N, W, Lcols, lo, hi)
         if world > 1:
             dist.destroy_process_group()
         return
@@ -470,6 +522,8 @@ def main():
     t_issue = (time.perf_counter() - t_issue) / args.steps * 1e3  # host time to ISSUE one step (launch-bound check)
     barrier()
     launches = lib.launch_count() - n0
+    if args.dump_outputs:  # what the last timed step returned: Phi a on this rank's rows, Phi^T r summed over the ranks
+        dumped = ({"phi_a": yhat_d[:nloc].cpu().numpy()}, {"phi_t": g_d.cpu().numpy()})
     ms = e0.elapsed_time(e1)
     t_a = float(np.mean([evs[s][0][i].elapsed_time(evs[s][1][i]) for s in range(args.steps) for i in range(2)]))
     t_t = float(np.mean([evs[s][1][i].elapsed_time(evs[s][2][i]) for s in range(args.steps) for i in range(2)]))
@@ -569,6 +623,8 @@ def main():
         del vec, loglik, logpr
 
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, rank, world, lo, hi, N, *dumped)
     if rank == 0:
         hbm_peak, hbm_src = 6650.0, "fallback"
         mp = REPO / "MEASURED_PEAKS.json"
