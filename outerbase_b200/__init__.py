@@ -19,6 +19,7 @@ CSRC = ROOT / "csrc"
 LIBDIR = ROOT / "_lib"
 LIBPATH = LIBDIR / "libouterbase_b200.so"
 HEADER = REPO / "include" / "outerbase_b200.h"
+MULTI_HEADER = REPO / "include" / "outerbase_b200_multi.h"  # the multi-response extension
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -32,7 +33,7 @@ def _stale() -> bool:
     if not LIBPATH.exists():
         return True
     t = LIBPATH.stat().st_mtime
-    deps = list(CSRC.glob("*")) + [HEADER]
+    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

@@ -217,10 +217,20 @@ class Library:
     def logpr_gauss(self, om, terms):
         return logpr_gauss(self, om, terms)
 
+    def loglik_gauss_multi(self, om, terms, Y, x):
+        return loglik_gauss_multi(self, om, terms, Y, x)
+
+    def logpr_gauss_multi(self, om, terms, ncol):
+        return logpr_gauss_multi(self, om, terms, ncol)
+
     def lpdfvec(self, a, b):
+        if isinstance(a, _multi) or isinstance(b, _multi):
+            return lpdfvec_multi(self, a, b)
         return lpdfvec(self, a, b)
 
     def predictor(self, loglik):
+        if isinstance(loglik, loglik_gauss_multi):
+            return predictor_multi(self, loglik)
         return predictor(self, loglik)
 
     # -- stateless linalg.h seam (src/linalg.h:9-58)
@@ -775,6 +785,45 @@ class lpdfvec(lpdf):
     domarg = property(fset=lambda s, v: s._flag("domarg", v))
 
 
+class _multi:
+    """Multi-response objects (C responses on one basis): coefficients and gradients are K x C (column c belongs to
+    response c); every other quantity is as for the flat K*C vector of the C ABI."""
+    ncol = property(lambda s: int(s._get("ncol")[0]))
+    coeff = property(lambda s: s._get("coeff").reshape((-1, s.ncol), order="F"))
+    grad = property(lambda s: s._get("grad").reshape((-1, s.ncol), order="F"))
+
+
+class loglik_gauss_multi(_multi, lpdf):
+    """loglik_gauss on each column of Y (N x C), all columns on one basis (include/outerbase_b200.h)."""
+
+    def __init__(self, lib, om, terms, Y, x):
+        super().__init__(lib)
+        self._om = om
+        t, Y, x = _terms(terms), _f64(Y), _f64(x)
+        if Y.ndim != 2:
+            raise ValueError("Y must be N x C")
+        if x.shape[0] != Y.shape[0]:
+            raise ValueError("x and Y dims do not align")
+        lib.call("loglik_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _p(Y), _u(Y.shape[1]), _p(x), _u(Y.shape[0]),
+                 C.byref(self._h))
+
+
+class logpr_gauss_multi(_multi, lpdf):
+    """An independent logpr_gauss on each of ncol coefficient columns, shared coeffscale."""
+
+    def __init__(self, lib, om, terms, ncol):
+        super().__init__(lib)
+        self._om = om
+        t = _terms(terms)
+        lib.call("logpr_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.byref(self._h))
+
+
+class lpdfvec_multi(_multi, lpdfvec):
+    """lpdfvec of two multi-response children; optcg runs one independent CG per column."""
+    cg_iters_per_column = property(lambda s: s._get("cg_iters").astype(int))
+    cg_iters = property(lambda s: int(s._get("cg_iters").max()))
+
+
 class predictor(_Handle):
     """new(predictor, loglik) -- src/fit.h:352-361."""
     _destroy = "predictor_destroy"
@@ -798,4 +847,13 @@ class predictor(_Handle):
     def var(self):
         out = np.empty(self._n)
         self._lib.call("predictor_var", self._h, _p(out))
+        return out
+
+
+class predictor_multi(predictor):
+    """predictor(loglik_gauss_multi): mean N x C; var is one N-vector shared by all columns."""
+
+    def mean(self):
+        out = np.empty((self._n, self._loglik.ncol), order="F")
+        self._lib.call("predictor_mean", self._h, _p(out))
         return out

@@ -4,6 +4,7 @@
  * computes: host model calls go to ob_model.hpp, everything N-sized to the CUDA kernels.
  */
 #include "../../include/outerbase_b200.h"
+#include "../../include/outerbase_b200_multi.h"
 
 #include "ob_engine.hpp"
 
@@ -455,6 +456,26 @@ int ob_logpr_gauss_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, u
   *out = h;
   OB_CATCH
 }
+int ob_loglik_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* Y, uint64_t C,
+                                 const double* x, uint64_t N, ob_lpdf** out) {
+  OB_TRY
+  need(ctx, "ctx"); need(om, "om");
+  if (C == 0) throw std::invalid_argument("ncol must be at least 1");
+  auto* h = new ob_lpdf();
+  h->ctx = ctx;
+  try { h->p.reset(new obe::LoglikGaussMulti(ctx->c, &om->om, terms, K, Y, C, x, N)); } catch (...) { delete h; throw; }
+  *out = h;
+  OB_CATCH
+}
+int ob_logpr_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, uint64_t C, ob_lpdf** out) {
+  OB_TRY
+  need(om, "om");
+  auto* h = new ob_lpdf();
+  h->ctx = ctx;
+  try { h->p.reset(new obe::LogprGaussMulti(&om->om, terms, K, C)); } catch (...) { delete h; throw; }
+  *out = h;
+  OB_CATCH
+}
 int ob_lpdfvec_create(ob_lpdf* a, ob_lpdf* b, ob_lpdf** out) {
   OB_TRY
   need(a, "a"); need(b, "b");
@@ -516,7 +537,11 @@ int ob_lpdf_get(ob_lpdf* l, const char* which, double* out, uint64_t* n) {
   else if (w == "para") v = l->p->para;
   else if (w == "totdiaghess") v = l->p->totdiaghess;
   else if (w == "tothess") v = l->p->tothess;
-  else if (w == "cg_iters") v = {double(l->p->cg_iters)};
+  else if (w == "cg_iters") {
+    auto* mv = dynamic_cast<obe::LpdfVec*>(l->p.get());
+    if (mv && mv->multi()) v.assign(mv->cg_iters_cols.begin(), mv->cg_iters_cols.end());
+    else v = {double(l->p->cg_iters)};
+  } else if (w == "ncol") v = {double(l->p->ncol())};
   else if (w == "yhat") {
     if (auto* g = dynamic_cast<obe::LoglikGauss*>(l->p.get())) v = g->get_yhat();
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(l->p.get())) v = g2->yhat;
@@ -538,6 +563,7 @@ int ob_predictor_create(ob_lpdf* loglik, ob_predictor** out) {
   try {
     if (auto* g3 = dynamic_cast<obe::LoglikStd*>(loglik->p.get())) h->ps.reset(new obe::PredrStd(*g3)); /* before its base class */
     else if (auto* g = dynamic_cast<obe::LoglikGauss*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*g));
+    else if (auto* gm = dynamic_cast<obe::LoglikGaussMulti*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*gm));
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(loglik->p.get())) h->pg.reset(new obe::PredGda(*g2));
     else throw std::invalid_argument("cannot produce a predictor from this obj.");
   } catch (...) { delete h; throw; }

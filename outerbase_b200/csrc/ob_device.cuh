@@ -283,16 +283,26 @@ enum CgStage : int {
   CG_STEP = 2,              /* q as above; num = grad.rm ; stop test ; denom = q.p ; alpha ; coeff += alpha p ; valo (:72-77) */
   CG_POST_UPDATE = 3        /* grad, val ; valdiff ; rm ; num2 = -(alpha q).rm ; beta ; p = rm + beta p             (:79-83) */
 };
+/* Column-batched form (loglik_gauss_multi): the launch runs one CTA per column; coeff, grad, m, rm, p, q and red are K x C
+ * column-major, scal holds CG_NSCAL scalars per column, sds is shared.  ncol = 1 with ssq = running = null is the
+ * single-response launch. */
 struct CgParams {
   int K, stage, lik_first, domarg;
   double* coeff; double* grad; const double* m; double* rm; double* p; double* q;
   const double* red;    /* K + 1: likelihood part of grad (update) or of the Hessian product (hessmult) | sum of squared residuals */
   const double* sds;    /* K: coeffsd (logpr_gauss.cpp:57) */
   double sca, obssd, nglobal, val_margadj, tol;
-  double* scal;         /* [0] num [1] denom [2] alpha [3] beta [4] val [5] valo [6] valdiff [7] stop [8] val_lik [9] val_pr */
+  double* scal;         /* [0] num [1] denom [2] alpha [3] beta [4] val [5] valo [6] valdiff [7] stop [8] val_lik [9] val_pr [10] iter */
+  const double* ssq = nullptr;  /* batched: per-column sums of squared residuals (red then holds K per column) */
+  unsigned* running = nullptr;  /* batched: running[iter & 1] counts the columns that did not stop in CG_STEP of iteration iter */
+  int iter = 0;
 };
-enum { CG_NUM = 0, CG_DENOM, CG_ALPHA, CG_BETA, CG_VAL, CG_VALO, CG_VALDIFF, CG_STOP, CG_VAL_LIK, CG_VAL_PR, CG_NSCAL = 16 };
-void launch_cg_stage(Ctx& c, const CgParams& p);
+enum { CG_NUM = 0, CG_DENOM, CG_ALPHA, CG_BETA, CG_VAL, CG_VALO, CG_VALDIFF, CG_STOP, CG_VAL_LIK, CG_VAL_PR, CG_ITER, CG_NSCAL = 16 };
+void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol = 1);
+/* after mm_mat_dev on C columns (leading dimension ld): update: w = -((yhat - y)/sd)/sd, ssq_out[c] = sum of
+ * ((yhat - y)/sd)^2 over column c (fixed order); hessmult: w = (yhat/sd)/sd.  Pad rows of w are zero; yhat may alias w. */
+void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
+                        DevBuf<double>& partial, double* ssq_out);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

@@ -735,6 +735,10 @@ struct Lpdf {
   virtual std::vector<double> hessgradpara() { return {}; }
   virtual u64 nhyp() const { return 0; }
   virtual u64 nrow() const { return 0; }
+  /* multi-response objects (loglik_gauss_multi, logpr_gauss_multi, an lpdfvec of them): ncol responses, coefficients
+   * K x ncol column-major, nterms = K * ncol */
+  virtual bool multi() const { return false; }
+  virtual u64 ncol() const { return 1; }
 
   /* dense K x K algebra of the full-Hessian branch: host side, like every other K-sized object of the lpdf family */
   /* solve A X = B by elimination with partial pivoting (Armadillo solve(): LAPACK dgesv); B is n x m */
@@ -1112,17 +1116,21 @@ struct LoglikGauss : Lpdf { /* loglik_gauss.cpp:41-179 */
   }
   bool can_diaghessgradhyp_dot() const override { return ctx.dsweep; }
   bool diaghessgradhyp_dot(const std::vector<double>& c, std::vector<double>& out) override {
-    /* sum_k c_k sum_n d(Phi^2)[n,k]/dhyp = sum_n d(Phi^2 c)[n]/dhyp: the hyper-gradient sweep on the squared operator.
-     * The swept / not-swept decision is COLLECTIVE: slot H of the reduction buffer counts the ranks whose sweep was
-     * unavailable (module build failure, table not specialised, geometry), so every rank takes the same branch and the
-     * allreduce sequence stays aligned (the fallback is a K*(1+H) allreduce in diaghessgradhyp()). */
-    const u64 K = nterms, H = ob.H;
-    if (!ctx.dsweep || c.size() != K || H == 0) return false;
+    if (!ctx.dsweep || c.size() != nterms || ob.H == 0) return false;
+    return sq_sweep_dot(ctx, ob, terms.data(), nterms, c, kbuf, red, para[0], out);
+  }
+  /* sum_k c_k sum_n d(Phi^2)[n,k]/dhyp = sum_n d(Phi^2 c)[n]/dhyp: the hyper-gradient sweep on the squared operator.
+   * The swept / not-swept decision is COLLECTIVE: slot H of the reduction buffer counts the ranks whose sweep was
+   * unavailable (module build failure, table not specialised, geometry), so every rank takes the same branch and the
+   * allreduce sequence stays aligned (the fallback is a K*(1+H) allreduce in diaghessgradhyp()). */
+  static bool sq_sweep_dot(Ctx& ctx, OuterBase& ob, const u64* terms, u64 K, const std::vector<double>& c, DevBuf<double>& kbuf,
+                           DevBuf<double>& red, double para0, std::vector<double>& out) {
+    const u64 H = ob.H;
     kbuf.upload(c, ctx.stream);
     red.ensure(H + 1);
     OB_CUDA(cudaMemsetAsync(red.p, 0, (H + 1) * sizeof(double), ctx.stream));
     bool done = false;
-    try { done = ob.gradhyp_sweep(terms.data(), K, 1, kbuf.p, nullptr, red.p); } catch (const std::exception&) { done = false; }
+    try { done = ob.gradhyp_sweep(terms, K, 1, kbuf.p, nullptr, red.p); } catch (const std::exception&) { done = false; }
     ctx.sync(); /* c must outlive the upload */
     if (ctx.nranks > 1) {
       if (!done) obd::launch_fill(ctx, red.p, H + 1, 0.0), obd::launch_fill(ctx, red.p + H, 1, 1.0);
@@ -1132,7 +1140,7 @@ struct LoglikGauss : Lpdf { /* loglik_gauss.cpp:41-179 */
     ob.d2h(r.data(), red.p, H + 1);
     if (r[H] != 0.0) return false; /* some rank could not sweep: all ranks fall back together */
     out.assign(r.begin(), r.begin() + H);
-    const double sc = std::exp(-2 * para[0]);
+    const double sc = std::exp(-2 * para0);
     for (double& v : out) v = sc * v;
     return true;
   }
@@ -1337,6 +1345,255 @@ struct LoglikGda : Lpdf {
   u64 nrow() const override { return N; }
 };
 
+/* ------------------------------------------------------------------ multi-response: C responses observed at the same rows
+ * Every column is the single-response model on its own response, all columns share the basis, the terms table, the
+ * hyper-parameters and both para entries.  val, gradhyp and gradpara are the sums over the columns (in column order) of
+ * what the single-response object returns at that column, grad is K x C, the Hessian product is block-diagonal and the
+ * Hessian diagonals are the single-response ones repeated C times.  The objective is meant for lpdfvec's diagonal
+ * branch and its column-batched CG (LpdfVec::optcg_multi); the full Hessian, optnewton and the host optcg are refused. */
+[[noreturn]] inline void refuse_multi(const char* what) {
+  throw std::invalid_argument(std::string(what) + " is not available for multi-response objects");
+}
+/* K x S -> (K C) x S: each length-K column repeated C times */
+inline std::vector<double> tile_cols(const std::vector<double>& v, u64 K, u64 C) {
+  const u64 S = K ? v.size() / K : 0;
+  std::vector<double> o(K * C * S);
+  for (u64 s = 0; s < S; ++s)
+    for (u64 c = 0; c < C; ++c) std::copy(v.begin() + s * K, v.begin() + (s + 1) * K, o.begin() + (s * C + c) * K);
+  return o;
+}
+
+struct LogprGaussMulti : Lpdf { /* an independent logpr_gauss on each column, shared coeffscale */
+  LogprGauss one;
+  u64 K, C;
+  std::vector<double> val_cols;
+  LogprGaussMulti(const OuterMod* om_, const u64* t, u64 K_, u64 C_) : one(om_, t, K_), K(K_), C(C_) {
+    if (C == 0) throw std::invalid_argument("ncol must be at least 1");
+    d = one.d; npara = one.npara; terms = one.terms; para0 = one.para0; paravar = one.paravar; para = one.para;
+    nterms = K * C;
+  }
+  bool multi() const override { return true; }
+  u64 ncol() const override { return C; }
+  u64 nhyp() const override { return one.nhyp(); }
+  void updateom() override { one.updateom(); }
+  void updatepara(const double* p, u64 n) override { one.updatepara(p, n); para = one.para; }
+  void updateterms(const u64* t, u64 K_) override { one.updateterms(t, K_); terms = one.terms; K = K_; nterms = K * C; }
+  std::vector<double> column(const std::vector<double>& v, u64 c) const { return std::vector<double>(v.begin() + c * K, v.begin() + (c + 1) * K); }
+  void update(const std::vector<double>& cf) override {
+    if (cf.size() != K * C) throw std::range_error("coeff must have K x ncol entries");
+    coeff = cf;
+    one.compute_val = compute_val; one.compute_grad = compute_grad; one.compute_gradhyp = compute_gradhyp; one.compute_gradpara = compute_gradpara;
+    if (compute_val) { val = 0; val_cols.assign(C, 0.0); }
+    if (compute_grad) grad.assign(K * C, 0.0);
+    if (compute_gradhyp) gradhyp.assign(one.nhyp(), 0.0);
+    if (compute_gradpara) gradpara.assign(1, 0.0);
+    for (u64 c = 0; c < C; ++c) {
+      one.update(column(cf, c));
+      if (compute_val) { val += one.val; val_cols[c] = one.val; }
+      if (compute_grad) std::copy(one.grad.begin(), one.grad.end(), grad.begin() + c * K);
+      if (compute_gradhyp) for (u64 h = 0; h < gradhyp.size(); ++h) gradhyp[h] += one.gradhyp[h];
+      if (compute_gradpara) gradpara[0] += one.gradpara[0];
+    }
+  }
+  std::vector<double> hessmult(const std::vector<double>& g) override {
+    if (g.size() != K * C) throw std::range_error("g must have K x ncol entries");
+    std::vector<double> o(K * C);
+    for (u64 c = 0; c < C; ++c) { const std::vector<double> h = one.hessmult(column(g, c)); std::copy(h.begin(), h.end(), o.begin() + c * K); }
+    return o;
+  }
+  std::vector<double> diaghess() override { return tile_cols(one.diaghess(), K, C); }
+  std::vector<double> diaghessgradhyp() override { return tile_cols(one.diaghessgradhyp(), K, C); }
+  std::vector<double> diaghessgradpara() override { return tile_cols(one.diaghessgradpara(), K, C); }
+  bool can_diaghessgradhyp_dot() const override { return true; }
+  bool diaghessgradhyp_dot(const std::vector<double>& cv, std::vector<double>& out) override {
+    if (cv.size() != K * C) return false;
+    out.assign(one.nhyp(), 0.0);
+    std::vector<double> o;
+    for (u64 c = 0; c < C; ++c) {
+      one.diaghessgradhyp_dot(column(cv, c), o);
+      for (u64 h = 0; h < out.size(); ++h) out[h] += o[h];
+    }
+    return true;
+  }
+  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
+  void optnewton() override { refuse_multi("optnewton"); }
+  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi)"); }
+};
+
+struct LoglikGaussMulti : Lpdf { /* loglik_gauss (loglik_gauss.cpp:41-179) on each of C responses */
+  Ctx& ctx;
+  const OuterMod* om;
+  OuterBase ob;
+  std::vector<double> x_host;
+  u64 N = 0, K = 0, C = 0;
+  double Nglobal = 0;
+  double obssd = 1;
+  /* Y, yhat, w: ld x C (pad rows zero) */
+  DevBuf<double> Y, yhat, w, kbuf, red, ssq, partial, gh, gebuf, ones;
+  std::vector<double> ssq_host; /* per-column sums of squared standardised residuals of the last update (all ranks) */
+
+  LoglikGaussMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
+      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_) {
+    if (C == 0) throw std::invalid_argument("ncol must be at least 1");
+    d = om->d; npara = 1;
+    terms.assign(t, t + K * d);
+    nterms = K * C;
+    x_host.assign(xh, xh + N * d);
+    const u64 ld = ob.ld;
+    Y.ensure(ld * C);
+    OB_CUDA(cudaMemsetAsync(Y.p, 0, ld * C * sizeof(double), ctx.stream));
+    for (u64 j = 0; j < C; ++j)
+      if (N) OB_CUDA(cudaMemcpyAsync(Y.p + j * ld, yh + j * N, N * sizeof(double), cudaMemcpyHostToDevice, ctx.stream));
+    yhat.ensure(ld * C); w.ensure(ld * C); ssq.ensure(C);
+    ctx.sync();
+    /* para0 = log(0.01 * mean over the columns of var(Y[:,c])), Armadillo two-pass variance over ALL ranks' rows; for
+     * C = 1 this is loglik_gauss's default (loglik_gauss.cpp:48) */
+    std::vector<double> var(C);
+    if (ctx.nranks > 1) {
+      std::vector<double> st(C + 1, 0.0), ss(C, 0.0);
+      st[0] = double(N);
+      for (u64 j = 0; j < C; ++j) for (u64 i = 0; i < N; ++i) st[1 + j] += yh[i + j * N];
+      allreduce_host(st.data(), C + 1);
+      Nglobal = st[0];
+      for (u64 j = 0; j < C; ++j) {
+        const double mean = st[1 + j] / st[0];
+        for (u64 i = 0; i < N; ++i) ss[j] += (yh[i + j * N] - mean) * (yh[i + j * N] - mean);
+      }
+      allreduce_host(ss.data(), C);
+      for (u64 j = 0; j < C; ++j) var[j] = ss[j] / (Nglobal - 1);
+    } else {
+      Nglobal = double(N);
+      for (u64 j = 0; j < C; ++j) var[j] = LoglikGauss::arma_var(yh + j * N, N);
+    }
+    double vs = 0;
+    for (double v : var) vs += v;
+    para0 = {std::log(0.01 * (vs / double(C)))};
+    paravar = {1};
+    para = para0;
+    obssd = std::exp(para[0]);
+  }
+  void allreduce_host(double* v, u64 n) {
+    red.upload(v, n, ctx.stream);
+    ctx.allreduce_sum(red.p, n);
+    OB_CUDA(cudaMemcpyAsync(v, red.p, n * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
+    ctx.sync();
+  }
+  bool multi() const override { return true; }
+  u64 ncol() const override { return C; }
+  u64 nhyp() const override { return ob.H; }
+  u64 nrow() const override { return N; }
+  void setnthreads(int k) override { ob.nthreads = k; }
+  void updateom() override { ob.build(); }
+  void updatepara(const double* p, u64 n) override { para.assign(p, p + n); obssd = std::exp(para[0]); }
+  void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; }
+  double val_col(u64 c) const { return -0.5 * ssq_host[c] - Nglobal * std::log(obssd); }
+
+  /* ---- device forms (stream ordered): red[0 .. K C) = the likelihood part of grad (update) or of the Hessian product
+   * (hessmult), summed over ranks; update also leaves ssq[c], summed over ranks.  The products are mm_mat_dev /
+   * tmm_mat_dev: the FP64 tensor-core kernels for C >= 8 on a specialised table, else column loops. */
+  void update_dev(const double* coeff_dev) {
+    ob.mm_mat_dev(terms.data(), K, 0, coeff_dev, C, yhat.p, ob.ld);
+    obd::launch_resid_multi(ctx, yhat.p, Y.p, w.p, N, ob.ld, C, obssd, true, partial, ssq.p);
+    red.ensure(K * C);
+    ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
+    ctx.allreduce_sum(ssq.p, C);
+  }
+  void hessmult_dev(const double* g_dev) { /* loglik_gauss.cpp:137-145 per column; w holds Phi g until the residual pass */
+    ob.mm_mat_dev(terms.data(), K, 0, g_dev, C, w.p, ob.ld);
+    obd::launch_resid_multi(ctx, w.p, nullptr, w.p, N, ob.ld, C, obssd, false, partial, nullptr);
+    red.ensure(K * C);
+    ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
+  }
+  void update(const std::vector<double>& cf) override { /* loglik_gauss.cpp:110-130 per column */
+    if (cf.size() != K * C) throw std::range_error("coeff must have K x ncol entries");
+    coeff = cf;
+    const u64 H = ob.H, ld = ob.ld;
+    kbuf.upload(coeff, ctx.stream);
+    update_dev(kbuf.p);
+    ssq_host.resize(C);
+    ob.d2h(ssq_host.data(), ssq.p, C);
+    if (compute_val) { val = 0; for (u64 c = 0; c < C; ++c) val += val_col(c); }
+    if (!compute_grad) return;
+    grad.resize(K * C);
+    ob.d2h(grad.data(), red.p, K * C);
+    if (compute_gradhyp) { /* one hyper-gradient pass per column (:127) */
+      gh.ensure(std::max<u64>(H * C, 1));
+      OB_CUDA(cudaMemsetAsync(gh.p, 0, std::max<u64>(H * C, 1) * sizeof(double), ctx.stream));
+      for (u64 c = 0; c < C && H > 0; ++c) {
+        const std::vector<double> a(coeff.begin() + c * K, coeff.begin() + (c + 1) * K);
+        if (ob.gradhyp_dots_spec(terms.data(), K, a, w.p + c * ld, yhat.p + c * ld, gh.p + c * H)) continue;
+        gebuf.ensure(ld + 4 * ctx.sms);
+        for (u64 h = 0; h < H; ++h) {
+          obd::PhiAArgs g; g.a = kbuf.p + c * K; g.out = gebuf.p; g.mode = obd::PHI_PLAIN;
+          obd::launch_phi_a(ctx, ob.plan(ob.program(terms.data(), K, (int)ob.hypmatch[h]), 0, (int)h), g, ob.ws, nullptr);
+          int nb = 0;
+          obd::launch_dot_partials(ctx, w.p + c * ld, gebuf.p, N, gebuf.p + ld, &nb);
+          obd::launch_sum_partials(ctx, gebuf.p + ld, nb, gh.p + c * H + h);
+        }
+      }
+      ctx.allreduce_sum(gh.p, H * C);
+      std::vector<double> r(H * C);
+      ob.d2h(r.data(), gh.p, H * C);
+      gradhyp.assign(H, 0.0);
+      for (u64 c = 0; c < C; ++c) for (u64 h = 0; h < H; ++h) gradhyp[h] += r[c * H + h];
+    }
+    if (compute_gradpara) { gradpara = {0.0}; for (u64 c = 0; c < C; ++c) gradpara[0] += ssq_host[c] - Nglobal; }
+  }
+  std::vector<double> hessmult(const std::vector<double>& g) override {
+    if (g.size() != K * C) throw std::range_error("g must have K x ncol entries");
+    kbuf.upload(g, ctx.stream);
+    hessmult_dev(kbuf.p);
+    std::vector<double> o(K * C);
+    ob.d2h(o.data(), red.p, K * C);
+    return o;
+  }
+  const double* ones_dev() {
+    if (ones.cap < ob.ld) { ones.ensure(ob.ld); obd::launch_fill(ctx, ones.p, ob.ld, 1.0); }
+    return ones.p;
+  }
+  /* the Hessian diagonals do not depend on the response: computed once (K long) and repeated over the columns */
+  std::vector<double> diaghess() override { /* :154-157 */
+    red.ensure(K);
+    ob.tmm_dev(terms.data(), K, 1, ones_dev(), red.p);
+    std::vector<double> lh(K);
+    ob.d2h(lh.data(), red.p, K);
+    const double c = std::exp(-2 * para[0]);
+    for (double& v : lh) v = c * v;
+    return tile_cols(lh, K, C);
+  }
+  std::vector<double> diaghessgradpara() override { /* :176-179 */
+    std::vector<double> lh = diaghess();
+    for (double& v : lh) v = -2 * v;
+    return lh;
+  }
+  std::vector<double> diaghessgradhyp() override { /* :165-168 */
+    const u64 H = ob.H;
+    red.ensure(K * (1 + H));
+    ob.tmm_ge_dev(terms.data(), K, 1, ones_dev(), red.p);
+    std::vector<double> all(K * (1 + H));
+    ob.d2h(all.data(), red.p, K * (1 + H));
+    std::vector<double> o(all.begin() + K, all.end());
+    const double c = std::exp(-2 * para[0]);
+    for (double& v : o) v = c * v;
+    return tile_cols(o, K, C);
+  }
+  bool can_diaghessgradhyp_dot() const override { return ctx.dsweep; }
+  bool diaghessgradhyp_dot(const std::vector<double>& cv, std::vector<double>& out) override {
+    /* linear in cv: the columns' weights are summed first, then ONE sweep of the squared operator */
+    if (!ctx.dsweep || cv.size() != K * C || ob.H == 0) return false;
+    std::vector<double> s(K, 0.0);
+    for (u64 c = 0; c < C; ++c) for (u64 i = 0; i < K; ++i) s[i] += cv[c * K + i];
+    return LoglikGauss::sq_sweep_dot(ctx, ob, terms.data(), K, s, kbuf, red, para[0], out);
+  }
+  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
+  void optnewton() override { refuse_multi("optnewton"); }
+  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi)"); }
+};
+
 struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   double val_margadj = 0;
   std::vector<double> gradhyp_margadj, gradpara_margadj;
@@ -1348,6 +1605,8 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   Lpdf* kid[2];
   u64 parasrt[2], paraend[2];
   LpdfVec(Lpdf* a, Lpdf* b) {
+    if (a->multi() != b->multi() || a->ncol() != b->ncol())
+      throw std::invalid_argument("lpdfvec: children must both be single-response, or multi-response with the same number of columns");
     kid[0] = a; kid[1] = b;
     terms = a->terms; d = a->d;
     nterms = a->nterms;
@@ -1417,6 +1676,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
    * Hessian is positive definite (it is at every point optnewton reaches), else from the symmetric eigen-decomposition
    * the reference uses for both */
   void buildhess_full() {
+    if (multi()) refuse_multi("the full-Hessian branch");
     const u64 K = nterms, KK = K * K;
     hessv = sum_same_size(kid[0]->hess(), kid[1]->hess(), "hess");
     settothess(hessv);
@@ -1609,10 +1869,95 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     compute_gradhyp = false; compute_gradpara = false;
     return true;
   }
+  /* optcg of lpdfvec(logpr_gauss_multi, loglik_gauss_multi), either order: C independent runs of lpdf::optcg
+   * (fit.cpp:37-96), column c on column c's own objective (its loglik, its prior, the single-response marginal
+   * adjustment) with its own num, alpha, beta, val / valdiff and stop test -- NOT one CG on the K C system, which would
+   * share alpha and beta over the columns.  The column-batched cg_stage_kernel runs one CTA per column; a column whose
+   * stop test passes is frozen as the reference `break`s, and the loop ends when no column runs (the host reads one
+   * count per iteration) or after maxepch.  The products of an iteration are matrix products over all C columns
+   * (frozen ones included), the first update() / diaghess() and the final update() with gradients run once for the
+   * whole object. */
+  DevBuf<unsigned> cg_running;
+  std::vector<u64> cg_iters_cols;
+  void optcg_multi(double tol, u64 maxepch) {
+    LoglikGaussMulti* lk = dynamic_cast<LoglikGaussMulti*>(kid[0]);
+    LogprGaussMulti* pr = dynamic_cast<LogprGaussMulti*>(kid[1]);
+    const bool lik_first = lk && pr;
+    if (!lik_first) { lk = dynamic_cast<LoglikGaussMulti*>(kid[1]); pr = dynamic_cast<LogprGaussMulti*>(kid[0]); }
+    if (!lk || !pr) throw std::invalid_argument("optcg on multi-response objects needs lpdfvec(logpr_gauss_multi, loglik_gauss_multi)");
+    Ctx& ctx = lk->ctx;
+    const u64 K = lk->K, C = lk->C, NS = obd::CG_NSCAL;
+    compute_val = true; compute_grad = true; compute_gradhyp = false; compute_gradpara = false;
+    if (coeff.size() != nterms) coeff.assign(nterms, 0.0);
+    update(std::vector<double>(coeff));
+    std::vector<double> m = diaghess();
+    cg_iters = 0;
+    cg_iters_cols.assign(C, 0);
+    if (!all_finite(m) && !all_finite(grad)) { val = -std::numeric_limits<double>::infinity(); return; }
+    /* column c's value as the single-response lpdfvec forms it (fit.cpp:352-380): children in order, then its own
+     * marginal adjustment -- the first K entries of the repeated diagonal are the single-response diagonal */
+    double vma = 0;
+    if (domargadj) {
+      std::vector<double> t(K);
+      for (u64 i = 0; i < K; ++i) t[i] = std::log(diaghessv[i]);
+      vma = -0.5 * obh::sum2(t.data(), K);
+    }
+    std::vector<double> scal(C * NS, 0.0);
+    for (u64 c = 0; c < C; ++c) {
+      const double vl = lk->val_col(c), vp = pr->val_cols[c];
+      double v = lik_first ? (0.0 + vl) + vp : (0.0 + vp) + vl;
+      if (domargadj) v += vma;
+      double* S = scal.data() + c * NS;
+      S[obd::CG_VAL] = v; S[obd::CG_VALO] = v; S[obd::CG_VALDIFF] = 10; S[obd::CG_DENOM] = 1;
+    }
+    cg_coeff.upload(coeff, ctx.stream); cg_grad.upload(grad, ctx.stream); cg_m.upload(m, ctx.stream);
+    cg_sds.upload(pr->one.coeffsd, ctx.stream);
+    cg_rm.ensure(K * C); cg_p.ensure(K * C); cg_q.ensure(K * C);
+    cg_scal.upload(scal, ctx.stream);
+    cg_running.ensure(2);
+    ctx.sync(); /* the host images above must outlive the uploads */
+    obd::CgParams c{};
+    c.K = (int)K; c.lik_first = lik_first ? 1 : 0; c.domarg = domargadj ? 1 : 0;
+    c.coeff = cg_coeff.p; c.grad = cg_grad.p; c.m = cg_m.p; c.rm = cg_rm.p; c.p = cg_p.p; c.q = cg_q.p; c.sds = cg_sds.p;
+    c.sca = pr->one.sca; c.obssd = lk->obssd; c.nglobal = lk->Nglobal; c.val_margadj = vma; c.tol = tol; c.scal = cg_scal.p;
+    c.ssq = lk->ssq.p; c.running = cg_running.p;
+    auto stage = [&](int st) { c.stage = st; c.red = lk->red.p; obd::launch_cg_stage(ctx, c, C); };
+    stage(obd::CG_INIT);
+    lk->hessmult_dev(cg_p.p);
+    u64 k;
+    for (k = 0; k < maxepch; k++) {
+      c.iter = (int)k;
+      OB_CUDA(cudaMemsetAsync(cg_running.p + (k & 1), 0, sizeof(unsigned), ctx.stream));
+      stage(obd::CG_STEP);
+      OB_CUDA(cudaMemcpyAsync(ctx.pinned, cg_running.p + (k & 1), sizeof(unsigned), cudaMemcpyDeviceToHost, ctx.stream));
+      ctx.sync();
+      unsigned running = 0;
+      std::memcpy(&running, ctx.pinned, sizeof(running));
+      if (running == 0) break;
+      lk->update_dev(cg_coeff.p);
+      stage(obd::CG_POST_UPDATE);
+      lk->hessmult_dev(cg_p.p);
+    }
+    cg_iters = k;
+    OB_CUDA(cudaMemcpyAsync(scal.data(), cg_scal.p, C * NS * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
+    OB_CUDA(cudaMemcpyAsync(coeff.data(), cg_coeff.p, K * C * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
+    ctx.sync();
+    for (u64 j = 0; j < C; ++j) cg_iters_cols[j] = scal[j * NS + obd::CG_STOP] != 0.0 ? (u64)scal[j * NS + obd::CG_ITER] : k;
+    compute_gradhyp = true; compute_gradpara = true;
+    update(std::vector<double>(coeff));
+    compute_gradhyp = false; compute_gradpara = false;
+  }
   void optcg(double tol, u64 maxepch) override {
     fullhess = false; /* fit.cpp:38 */
+    if (multi()) { optcg_multi(tol, maxepch); return; }
     if (!optcg_device(tol, maxepch)) Lpdf::optcg(tol, maxepch);
   }
+  void optnewton() override {
+    if (multi()) refuse_multi("optnewton");
+    Lpdf::optnewton();
+  }
+  bool multi() const override { return kid[0]->multi(); }
+  u64 ncol() const override { return kid[0]->ncol(); }
   std::vector<double> diaghess() override { return diaghessv; }
   std::vector<double> diaghessgradhyp() override {
     if (hyp_matrix_stale) { diaghessgradhypv = diaghessgradhyp_(); hyp_matrix_stale = false; }
@@ -1640,6 +1985,7 @@ struct PredGauss { /* loglik_gauss.cpp:196-227 */
   std::vector<double> para, coeff, coeffvar;
   std::vector<u64> terms;
   u64 K, d;
+  u64 C = 1; /* columns of the mean (loglik_gauss_multi) */
   int nthreads = 0;
   std::unique_ptr<OuterBase> ob;
   PredGauss(LoglikGauss& lk) : ctx(lk.ctx), om(lk.om), para(lk.para), coeff(lk.coeff), terms(lk.terms), K(lk.nterms), d(lk.d) {
@@ -1651,8 +1997,21 @@ struct PredGauss { /* loglik_gauss.cpp:196-227 */
       for (u64 i = 0; i < coeffvar.size(); ++i) coeffvar[i] = 1 / lk.totdiaghess[i];
     } else coeffvar.assign(coeff.size(), 0.0);
   }
+  /* multi-response: mean N x C; the variance is one N-vector for all columns (the total Hessian diagonal is the same
+   * K-vector repeated over the columns) */
+  PredGauss(LoglikGaussMulti& lk) : ctx(lk.ctx), om(lk.om), para(lk.para), coeff(lk.coeff), terms(lk.terms), K(lk.K), d(lk.d), C(lk.C) {
+    ob.reset(new OuterBase(ctx, om, lk.x_host.data(), lk.N, false, terms.data(), K));
+    nthreads = (int)lk.ob.nthreads;
+    if (coeff.size() != K * C) coeff.assign(K * C, 0.0);
+    coeffvar.assign(K, 0.0);
+    if (!lk.didnotothess && lk.totdiaghess.size() >= K)
+      for (u64 i = 0; i < K; ++i) coeffvar[i] = 1 / lk.totdiaghess[i];
+  }
   void update(const double* x, u64 N) { ob.reset(new OuterBase(ctx, om, x, N, false, terms.data(), K)); }
-  void mean(double* out) { ob->mm(0, terms.data(), K, coeff.data(), out); }
+  void mean(double* out) {
+    if (C == 1) ob->mm(0, terms.data(), K, coeff.data(), out);
+    else ob->mm_mat(0, terms.data(), K, coeff.data(), C, out);
+  }
   void var(double* out) {
     ob->mm(1, terms.data(), K, coeffvar.data(), out);
     const double c = std::exp(2 * para[0]);

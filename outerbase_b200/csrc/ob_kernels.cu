@@ -1330,10 +1330,16 @@ __device__ double cg_block_sum(double v, double* sm) {
   return sm[32];
 }
 
-__global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(const CgParams c) {
+/* One CTA per column (blockIdx.x): the column's K-slices of every vector and its own CG_NSCAL scalars.  c.running is
+ * set only by the column-batched caller; there a column whose stop test has passed is frozen (the reference `break`s,
+ * fit.cpp:73) -- its stages return before touching anything. */
+__global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
   __shared__ double sm[33];
   const int K = c.K, tid = threadIdx.x;
-  double* S = c.scal;
+  const size_t off = (size_t)blockIdx.x * (size_t)K;
+  c.coeff += off; c.grad += off; c.m += off; c.rm += off; c.p += off; c.q += off; c.red += off;
+  double* S = c.scal + (size_t)blockIdx.x * CG_NSCAL;
+  if (c.running && S[CG_STOP] != 0.0) return;
   if (c.stage == CG_INIT) {
     for (int i = tid; i < K; i += kCgThreads) { const double rm = c.grad[i] / c.m[i]; c.rm[i] = rm; c.p[i] = rm; }
     return;
@@ -1352,7 +1358,8 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(const CgParams c) 
     }
     const double t1 = cg_block_sum(s1, sm), t2 = cg_block_sum(s2, sm);
     const double val_pr = -0.5 * t1 - t2;
-    const double val_lik = -0.5 * c.red[K] - c.nglobal * log(c.obssd);
+    const double ssq = c.ssq ? c.ssq[blockIdx.x] : c.red[K];
+    const double val_lik = -0.5 * ssq - c.nglobal * log(c.obssd);
     double val = c.lik_first ? (0.0 + val_lik) + val_pr : (0.0 + val_pr) + val_lik;
     if (c.domarg) val += c.val_margadj;
     const double valo = S[CG_VALO], alpha = S[CG_ALPHA], num = S[CG_NUM];
@@ -1388,12 +1395,71 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(const CgParams c) 
   if (tid == 0) {
     S[CG_NUM] = num; S[CG_STOP] = stop ? 1.0 : 0.0;
     if (!stop) { S[CG_DENOM] = denom; S[CG_ALPHA] = alpha; S[CG_VALO] = S[CG_VAL]; }
+    if (c.running) {
+      if (stop) S[CG_ITER] = c.iter;
+      else atomicAdd(c.running + (c.iter & 1), 1u);
+    }
   }
 }
 
-void launch_cg_stage(Ctx& c, const CgParams& p) {
-  cg_stage_kernel<<<1, kCgThreads, 0, c.stream>>>(p);
+void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol) {
+  cg_stage_kernel<<<(unsigned)ncol, kCgThreads, 0, c.stream>>>(p);
   check_launch(c, "cg_stage_kernel");
+}
+
+/* Residuals of C columns after mm_mat_dev, the PHI_UPDATE / PHI_HESS epilogue of phi_a_kernel column by column (same
+ * expressions, so a column's w equals the single-response kernel's bit for bit given the same yhat).  grid (nb, C);
+ * rows N .. ld-1 of w are written as zero (phi_tm_spec multiplies pad rows by Phi = 0, they must be finite).  update:
+ * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w. */
+constexpr int kResidThreads = 256;
+__global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double* yhat, const double* __restrict__ y, double* w, u64 N,
+                                                                   u64 ld, double sd, int update, double* __restrict__ partial) {
+  __shared__ double sm[kResidThreads];
+  const u64 col = blockIdx.y, base = col * ld;
+  double s = 0.0;
+  for (u64 i = (u64)blockIdx.x * kResidThreads + threadIdx.x; i < ld; i += (u64)gridDim.x * kResidThreads) {
+    double wv = 0.0;
+    if (i < N) {
+      const double yv = yhat[base + i];
+      if (update) {
+        const double rt = (yv - y[base + i]) / sd;
+        s += rt * rt;
+        wv = -1. * (rt / sd);
+      } else wv = (yv / sd) / sd;
+    }
+    w[base + i] = wv;
+  }
+  if (!update) return;
+  sm[threadIdx.x] = s;
+  __syncthreads();
+  for (int h = kResidThreads / 2; h > 0; h >>= 1) {
+    if (threadIdx.x < h) sm[threadIdx.x] += sm[threadIdx.x + h];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) partial[col * gridDim.x + blockIdx.x] = sm[0];
+}
+/* out[c] = sum of column c's nb partials, in index order */
+__global__ void resid_colsum_kernel(const double* __restrict__ partial, int nb, double* __restrict__ out) {
+  if (threadIdx.x != 0) return;
+  double s = 0.0;
+  for (int i = 0; i < nb; ++i) s += partial[(size_t)blockIdx.x * nb + i];
+  out[blockIdx.x] = s;
+}
+void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
+                        DevBuf<double>& partial, double* ssq_out) {
+  if (C == 0) return;
+  if (ld == 0) { /* a rank without rows still takes part in the sums over ranks */
+    if (update) OB_CUDA(cudaMemsetAsync(ssq_out, 0, C * sizeof(double), c.stream));
+    return;
+  }
+  const int nb = (int)std::max<u64>(1, std::min<u64>((ld + kResidThreads - 1) / kResidThreads, std::max<u64>(1, (u64)c.sms * 8 / C)));
+  if (update) partial.ensure((size_t)nb * C);
+  resid_multi_kernel<<<dim3((unsigned)nb, (unsigned)C), kResidThreads, 0, c.stream>>>(yhat, y, w, N, ld, sd, update ? 1 : 0,
+                                                                                      update ? partial.p : nullptr);
+  check_launch(c, "resid_multi_kernel");
+  if (!update) return;
+  resid_colsum_kernel<<<(unsigned)C, 32, 0, c.stream>>>(partial.p, nb, ssq_out);
+  check_launch(c, "resid_colsum_kernel");
 }
 
 void launch_sum_partials(Ctx& c, const double* partial, int n, double* out) {

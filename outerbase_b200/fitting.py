@@ -14,6 +14,7 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
   getsteps      R/fitting.R:188-195
   obfit         R/fitting.R:27-137        both stages: loglik_gda on a subsample, then loglik_gauss on all rows
   obfit_gauss   R/fitting.R:100-136       the stage-2 loop alone, started from the constructor defaults
+  obfit_multi                             obfit_gauss for C responses at the same inputs (no reference counterpart)
   obpred        R/fitting.R:149-155
 """
 from __future__ import annotations
@@ -310,8 +311,46 @@ def obfit(lib, x, y, numb=100, verbose=0, covnames=None, hyp=None, numberopts=2,
                 predobj=lib.predictor(loglik_faster), optinfo=optinfo, stage1=dict(logpdf=logpdf, loglik=loglik, rows=subset))
 
 
+def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verbose=0, knots=40):
+    """obfit_gauss for C responses observed at the same inputs (Y is N x C): each column standardised on its own, then
+    the same stage-2 loop on lpdfvec(logpr_gauss_multi, loglik_gauss_multi) with domarg -- one basis, one terms table,
+    shared hyper-parameters and para, one independent CG per column inside every objective evaluation."""
+    x = np.asfortranarray(np.asarray(x, dtype=float))
+    Y = np.asarray(Y, dtype=float)
+    if Y.ndim != 2:
+        raise ValueError("Y must be N x C")
+    if x.shape[0] != Y.shape[0]:
+        raise ValueError("x and Y dims do not align")
+    d = x.shape[1]
+    if numb < 2 * d:
+        raise ValueError("number of basis functions should be less than twice the dimension")
+    y_cent, y_sca = Y.mean(axis=0), Y.std(axis=0, ddof=1)
+    Ys = np.asfortranarray((Y - y_cent) / y_sca)
+    om = lib.outermod()
+    om.setcovfs(list(covnames) if covnames is not None else ["mat25pow"] * d)
+    if hyp is not None and len(hyp) == gethyp(om).size:
+        om.updatehyp(hyp)
+    om.setknot(genknotlist([knots] * d, x))
+    terms = om.selectterms(numb)
+    logpr = lib.logpr_gauss_multi(om, terms, Y.shape[1])
+    loglik = lib.loglik_gauss_multi(om, terms, Ys, x)
+    logpdf = lib.lpdfvec(logpr, loglik)  # prior first, as obfit_gauss
+    logpdf.domarg = True
+    optinfo = dict(B=None, lr=0.2)
+    for k in range(numberopts):
+        terms = om.selectterms(numb)
+        logpdf.updateterms(terms)
+        optinfo = BFGS_lpdf(om, logpdf, verbose=verbose, B=optinfo["B"], lr=optinfo["lr"] / 2)
+    return dict(y_cent=y_cent, y_sca=y_sca, om=om, terms=terms, logpdf=logpdf, loglik=loglik, logpr=logpr,
+                predobj=lib.predictor(loglik), optinfo=optinfo)
+
+
 def obpred(obmodel, x):
-    """R/fitting.R:149-155."""
+    """R/fitting.R:149-155.  A model of obfit_multi gives an N x C mean and an N x C variance: the shared variance
+    scaled by each column's y_sca^2."""
     obmodel["predobj"].update(np.asfortranarray(np.asarray(x, dtype=float)))
+    if np.ndim(obmodel["y_sca"]):
+        var = obmodel["predobj"].var()
+        return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(), var=np.outer(var, obmodel["y_sca"] ** 2))
     return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(),
                 var=obmodel["y_sca"] ** 2 * obmodel["predobj"].var())
