@@ -232,6 +232,12 @@ int ob_debug_terms_eval(const uint64_t* terms, uint64_t K, uint64_t d, const uin
                         int ngroups, int aug_dim, const double* bcols, const double* gcols0,
                         const double* a, double b, double* out_phi_a, double* out_phit,
                         uint64_t* stats /* W, Lcols, nodes, maxdepth, fast_ok, nslots, nwords_fwd, nwords_bwd */);
+/* Test hook: the layout the interpreter Phi a (transpose = 0) or Phi^T (transpose = 1) kernel runs with for this
+ * object's rows and a terms table (plain program, sq selects the squared operator).  out = {R rows per lane, tile
+ * buffers, program in shared memory (1) or global memory (0), shared-memory bytes}; R = 0: the brute-force kernels
+ * (a table the trie compiler refuses, or no layout fits in shared memory).  Specialised kernels are not reported. */
+int ob_outerbase_debug_phi_geometry(ob_outerbase* ob, const uint64_t* terms, uint64_t K, int transpose, int sq,
+                                    int* out /* 4 */);
 
 /* ------------------------------------------------------------------ stateless linalg.h seam
  * Exactly the eight free functions of src/linalg.h:9-58: same argument meaning, host

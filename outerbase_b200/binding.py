@@ -442,6 +442,14 @@ class outerbase(_Handle):
         self._lib.call("outerbase_spec_state", self._h, _p(t), _u(t.shape[0]), C.byref(st))
         return st.value
 
+    def debug_phi_geometry(self, terms, transpose=False, sq=0):
+        """Layout of the interpreter Phi a (Phi^T with transpose) kernel for this object's rows and a terms table:
+        R (rows per lane; 0 = brute-force kernels), nbuf (tile buffers), prog_in_smem, smem (bytes). Product only."""
+        t = _terms(terms)
+        out = (C.c_int * 4)()
+        self._lib.call("outerbase_debug_phi_geometry", self._h, _p(t), _u(t.shape[0]), C.c_int(1 if transpose else 0), C.c_int(sq), out)
+        return dict(zip(("R", "nbuf", "prog_in_smem", "smem"), map(int, out)))
+
     def _loopvals(self):
         nt, cs, ls, vp = C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_int()
         self._lib.call("outerbase_loopvals", self._h, C.byref(nt), C.byref(cs), C.byref(ls), C.byref(vp))

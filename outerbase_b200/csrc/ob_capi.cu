@@ -372,6 +372,14 @@ int ob_debug_terms_eval(const uint64_t* terms, uint64_t K, uint64_t d, const uin
   OB_CATCH
 }
 
+int ob_outerbase_debug_phi_geometry(ob_outerbase* ob, const uint64_t* terms, uint64_t K, int transpose, int sq, int* out) {
+  OB_TRY
+  need(ob, "ob"); need(terms, "terms"); need(out, "out");
+  obe::OuterBase& b = *ob->ob;
+  obd::phi_geometry_info(b.ctx, b.plan(b.program(terms, K, -1, transpose ? 1 : 0), sq ? 1 : 0, -1), transpose == 0, out);
+  OB_CATCH
+}
+
 /* ---- stateless linalg.h seam */
 #define SEAM_BASE(bmge, Mge, ge, hm, H) \
   need(ctx, "ctx");                     \

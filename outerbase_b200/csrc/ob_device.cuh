@@ -234,6 +234,9 @@ void launch_phi_a(Ctx& c, const PhiPlan& pl, const PhiAArgs& args, Workspace& ws
 /* Phi^T w -> out (K, device); result is the LOCAL (this rank's rows) sum */
 void launch_phi_t(Ctx& c, const PhiPlan& pl, const double* w, double* out, Workspace& ws);
 void launch_phi_t_reduce(Ctx& c, const double* partial, int nblocks, int nslots, const int32_t* slot_term, double* out);
+/* the layout launch_phi_a (is_a) / launch_phi_t picks for a plan: {rows per lane R, tile buffers, program in shared
+ * memory, shared-memory bytes}; R == 0 means the brute-force kernels */
+void phi_geometry_info(const Ctx& c, const PhiPlan& pl, bool is_a, int out[4]);
 /* ---- terms-specialised kernels (ob_spec.hpp generator, ob_spec_scaffold.inc frame, ob_spec_rt.cu run time) */
 struct SpecKernels;
 bool spec_compiler_available();

@@ -479,20 +479,77 @@ __global__ void phi_a_simple_kernel(const double* const* load_src, const int* co
   out[n] = __dmul_rn(acc, sc);
 }
 
-__global__ void phi_t_simple_kernel(const double* const* load_src, const int* col_op, const uint32_t* csr_ptr,
-                                    const uint32_t* csr_col, int K, const double* w, const double* scale, int sq,
-                                    unsigned long long N, double* out /* K, pre-zeroed */) {
-  const unsigned long long n = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-  double b = 0.0;
-  if (n < N) { double sc = scale[n]; if (sq) sc = __dmul_rn(sc, sc); b = __dmul_rn(sc, w[n]); }
-  for (int k = 0; k < K; ++k) {
-    double t = b;
-    if (n < N)
+/* partial[k * gridDim.x + blockIdx.x] = this CTA's share of (Phi^T w)_k: rows in grid-stride order per thread, then the
+ * warp butterfly, then the warps in index order.  blockIdx.y strides over the terms (few rows: more CTAs).  No atomics,
+ * so the result is the same bits on every run; the CTA partials are added in index order by colsum_partials_kernel. */
+constexpr int kSimpleTThreads = 512;
+__global__ void __launch_bounds__(kSimpleTThreads) phi_t_simple_kernel(const double* const* load_src, const int* col_op,
+                                                                       const uint32_t* csr_ptr, const uint32_t* csr_col, int K,
+                                                                       const double* w, const double* scale, int sq,
+                                                                       unsigned long long N, double* __restrict__ partial) {
+  constexpr int kWarps = kSimpleTThreads / 32;
+  __shared__ double warp_sum[2][kWarps]; /* double-buffered: one barrier per term */
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const unsigned long long stride = (unsigned long long)gridDim.x * kSimpleTThreads;
+  for (int k = blockIdx.y, it = 0; k < K; k += gridDim.y, it ^= 1) {
+    double s = 0.0;
+    for (unsigned long long n = (unsigned long long)blockIdx.x * kSimpleTThreads + threadIdx.x; n < N; n += stride) {
+      double sc = scale[n];
+      if (sq) sc = __dmul_rn(sc, sc);
+      double t = __dmul_rn(sc, w[n]);
       for (uint32_t j = csr_ptr[k]; j < csr_ptr[k + 1]; ++j) t = __dmul_rn(t, col_value(load_src, col_op, csr_col[j], n));
+      s += t;
+    }
 #pragma unroll
-    for (int m = 16; m > 0; m >>= 1) t += shfl_xor_d(t, m);
-    if ((threadIdx.x & 31) == 0) atomicAdd(&out[k], t);
+    for (int m = 16; m > 0; m >>= 1) s += shfl_xor_d(s, m);
+    if (lane == 0) warp_sum[it][warp] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double v = 0.0;
+      for (int i = 0; i < kWarps; ++i) v += warp_sum[it][i];
+      partial[(size_t)k * gridDim.x + blockIdx.x] = v;
+    }
   }
+}
+
+/* out[c] = sum of column c's nb partials (partial[c * nb + i]), in index order */
+__global__ void colsum_partials_kernel(const double* __restrict__ partial, int nb, double* __restrict__ out) {
+  if (threadIdx.x != 0) return;
+  double s = 0.0;
+  for (int i = 0; i < nb; ++i) s += partial[(size_t)blockIdx.x * nb + i];
+  out[blockIdx.x] = s;
+}
+
+/* Residuals of C columns after a plain product, the PHI_UPDATE / PHI_HESS epilogue of phi_a_kernel column by column
+ * (same expressions, so a column's w equals the trie kernel's bit for bit given the same yhat).  grid (nb, C);
+ * rows N .. ld-1 of w are written as zero (phi_tm_spec and phi_t_spec read pad rows, they must be finite).  update:
+ * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w. */
+constexpr int kResidThreads = 256;
+__global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double* yhat, const double* __restrict__ y, double* w, u64 N,
+                                                                   u64 ld, double sd, int update, double* __restrict__ partial) {
+  __shared__ double sm[kResidThreads];
+  const u64 col = blockIdx.y, base = col * ld;
+  double s = 0.0;
+  for (u64 i = (u64)blockIdx.x * kResidThreads + threadIdx.x; i < ld; i += (u64)gridDim.x * kResidThreads) {
+    double wv = 0.0;
+    if (i < N) {
+      const double yv = yhat[base + i];
+      if (update) {
+        const double rt = (yv - y[base + i]) / sd;
+        s += rt * rt;
+        wv = -1. * (rt / sd);
+      } else wv = (yv / sd) / sd;
+    }
+    w[base + i] = wv;
+  }
+  if (!update) return;
+  sm[threadIdx.x] = s;
+  __syncthreads();
+  for (int h = kResidThreads / 2; h > 0; h >>= 1) {
+    if (threadIdx.x < h) sm[threadIdx.x] += sm[threadIdx.x + h];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) partial[col * gridDim.x + blockIdx.x] = sm[0];
 }
 
 __global__ void getmat_kernel(const double* const* load_src, const int* col_op, const uint32_t* csr_ptr,
@@ -1208,6 +1265,15 @@ static PhiGeom phi_geometry(const Ctx& c, const DevProgram& pr, const ColTable& 
   PhiGeom none;
   return none;
 }
+/* the layout the interpreter kernel of a plan runs with; R == 0: the brute-force kernels */
+static PhiGeom plan_geometry(const Ctx& c, const PhiPlan& pl, bool is_a) {
+  if (!pl.prog->host.fast_ok) return PhiGeom();
+  return phi_geometry(c, *pl.prog, *pl.cols, is_a, pl.N);
+}
+void phi_geometry_info(const Ctx& c, const PhiPlan& pl, bool is_a, int out[4]) {
+  const PhiGeom g = plan_geometry(c, pl, is_a);
+  out[0] = g.R; out[1] = g.nbuf; out[2] = g.prog_in_smem; out[3] = (int)g.smem;
+}
 
 static void fill_params(PhiKParams& p, const PhiPlan& pl, const PhiGeom& g, bool is_a) {
   const DevProgram& pr = *pl.prog;
@@ -1233,15 +1299,25 @@ static void set_smem(Kern k, size_t bytes) {
 void launch_phi_a(Ctx& c, const PhiPlan& pl, const PhiAArgs& a, Workspace& ws, int* grid_out) {
   const DevProgram& pr = *pl.prog;
   if (pl.N == 0) { if (grid_out) *grid_out = 0; return; }
-  PhiGeom g;
-  if (pr.host.fast_ok) g = phi_geometry(c, pr, *pl.cols, true, pl.N);
-  if (g.R == 0) { /* brute-force form */
-    if (a.mode != PHI_PLAIN) throw std::logic_error("fused epilogues need the trie kernel");
+  const PhiGeom g = plan_geometry(c, pl, true);
+  if (g.R == 0) { /* brute-force form; UPDATE / HESS: the trie kernel's epilogue follows as resid_multi_kernel */
+    if (a.mode == PHI_DOT) throw std::logic_error("the dot epilogue needs the specialised kernel");
+    double* yv = a.mode == PHI_HESS ? a.w : a.out; /* HESS stores no yhat: w holds it until the epilogue rewrites it */
     const int bs = 128;
     phi_a_simple_kernel<<<(unsigned)((pl.N + bs - 1) / bs), bs, 0, c.stream>>>(
-        pl.cols->load_src.p, pl.cols->col_op.p, pr.csr_ptr.p, pr.csr_col.p, (int)pr.host.K, a.a, pl.scale, pl.sq, pl.N, a.out);
+        pl.cols->load_src.p, pl.cols->col_op.p, pr.csr_ptr.p, pr.csr_col.p, (int)pr.host.K, a.a, pl.scale, pl.sq, pl.N, yv);
     check_launch(c, "phi_a_simple_kernel");
-    if (grid_out) *grid_out = 0;
+    int nb = 0;
+    if (a.mode != PHI_PLAIN) {
+      /* at most one partial per SM, like the trie kernel's grid: ssq_partial buffers are sized for that */
+      const u64 ld = std::max(pl.ld, pl.N);
+      nb = (int)std::min<u64>((ld + kResidThreads - 1) / kResidThreads, (u64)c.sms);
+      const bool update = a.mode == PHI_UPDATE;
+      double* part = update ? (a.ssq_partial ? a.ssq_partial : ws.ssq.ensure(c.sms)) : nullptr;
+      resid_multi_kernel<<<dim3((unsigned)nb, 1), kResidThreads, 0, c.stream>>>(yv, a.y, a.w, pl.N, ld, a.sd, update ? 1 : 0, part);
+      check_launch(c, "resid_multi_kernel");
+    }
+    if (grid_out) *grid_out = a.mode == PHI_UPDATE ? nb : 0;
     return;
   }
   PhiKParams p{};
@@ -1265,14 +1341,17 @@ void launch_phi_t(Ctx& c, const PhiPlan& pl, const double* w, double* out, Works
   const int K = (int)pr.host.K;
   if (K == 0) return;
   if (pl.N == 0) { launch_fill(c, out, K, 0.0); return; }
-  PhiGeom g;
-  if (pr.host.fast_ok) g = phi_geometry(c, pr, *pl.cols, false, pl.N);
-  if (g.R == 0) {
-    launch_fill(c, out, K, 0.0);
-    const int bs = 128;
-    phi_t_simple_kernel<<<(unsigned)((pl.N + bs - 1) / bs), bs, 0, c.stream>>>(
-        pl.cols->load_src.p, pl.cols->col_op.p, pr.csr_ptr.p, pr.csr_col.p, K, w, pl.scale, pl.sq, pl.N, out);
+  const PhiGeom g = plan_geometry(c, pl, false);
+  if (g.R == 0) { /* brute-force form: per-CTA partials, added in a fixed order */
+    const u64 ctas = 2 * (u64)c.sms;
+    const int nb = (int)std::max<u64>(1, std::min<u64>((pl.N + kSimpleTThreads - 1) / kSimpleTThreads, ctas));
+    const unsigned nk = (unsigned)std::min<u64>({(u64)K, std::max<u64>(1, ctas / nb), 65535});
+    double* part = ws.partial.ensure((size_t)nb * K);
+    phi_t_simple_kernel<<<dim3((unsigned)nb, nk), kSimpleTThreads, 0, c.stream>>>(
+        pl.cols->load_src.p, pl.cols->col_op.p, pr.csr_ptr.p, pr.csr_col.p, K, w, pl.scale, pl.sq, pl.N, part);
     check_launch(c, "phi_t_simple_kernel");
+    colsum_partials_kernel<<<(unsigned)K, 32, 0, c.stream>>>(part, nb, out);
+    check_launch(c, "colsum_partials_kernel");
     return;
   }
   PhiKParams p{};
@@ -1407,44 +1486,6 @@ void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol) {
   check_launch(c, "cg_stage_kernel");
 }
 
-/* Residuals of C columns after mm_mat_dev, the PHI_UPDATE / PHI_HESS epilogue of phi_a_kernel column by column (same
- * expressions, so a column's w equals the single-response kernel's bit for bit given the same yhat).  grid (nb, C);
- * rows N .. ld-1 of w are written as zero (phi_tm_spec multiplies pad rows by Phi = 0, they must be finite).  update:
- * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w. */
-constexpr int kResidThreads = 256;
-__global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double* yhat, const double* __restrict__ y, double* w, u64 N,
-                                                                   u64 ld, double sd, int update, double* __restrict__ partial) {
-  __shared__ double sm[kResidThreads];
-  const u64 col = blockIdx.y, base = col * ld;
-  double s = 0.0;
-  for (u64 i = (u64)blockIdx.x * kResidThreads + threadIdx.x; i < ld; i += (u64)gridDim.x * kResidThreads) {
-    double wv = 0.0;
-    if (i < N) {
-      const double yv = yhat[base + i];
-      if (update) {
-        const double rt = (yv - y[base + i]) / sd;
-        s += rt * rt;
-        wv = -1. * (rt / sd);
-      } else wv = (yv / sd) / sd;
-    }
-    w[base + i] = wv;
-  }
-  if (!update) return;
-  sm[threadIdx.x] = s;
-  __syncthreads();
-  for (int h = kResidThreads / 2; h > 0; h >>= 1) {
-    if (threadIdx.x < h) sm[threadIdx.x] += sm[threadIdx.x + h];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) partial[col * gridDim.x + blockIdx.x] = sm[0];
-}
-/* out[c] = sum of column c's nb partials, in index order */
-__global__ void resid_colsum_kernel(const double* __restrict__ partial, int nb, double* __restrict__ out) {
-  if (threadIdx.x != 0) return;
-  double s = 0.0;
-  for (int i = 0; i < nb; ++i) s += partial[(size_t)blockIdx.x * nb + i];
-  out[blockIdx.x] = s;
-}
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
                         DevBuf<double>& partial, double* ssq_out) {
   if (C == 0) return;
@@ -1458,8 +1499,8 @@ void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, 
                                                                                       update ? partial.p : nullptr);
   check_launch(c, "resid_multi_kernel");
   if (!update) return;
-  resid_colsum_kernel<<<(unsigned)C, 32, 0, c.stream>>>(partial.p, nb, ssq_out);
-  check_launch(c, "resid_colsum_kernel");
+  colsum_partials_kernel<<<(unsigned)C, 32, 0, c.stream>>>(partial.p, nb, ssq_out);
+  check_launch(c, "colsum_partials_kernel");
 }
 
 void launch_sum_partials(Ctx& c, const double* partial, int n, double* out) {

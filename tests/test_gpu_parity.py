@@ -77,14 +77,17 @@ def test_seam_multi_rhs_and_getm(gpu, oracle):
 
 def test_bruteforce_path_is_bit_exact(gpu, oracle):
     """A terms table with a duplicated row is refused by the trie compiler and runs on the
-    brute-force kernel, which follows linalg.cpp:70-75 operation by operation."""
+    brute-force kernel, which follows linalg.cpp:70-75 operation by operation.  Its Phi^T sums per-CTA partials in a
+    fixed order: a second call gives the same bits."""
     o = oracle_basis(oracle, 10000, 100)
     terms = np.asfortranarray(np.vstack([o["terms"], o["terms"][5:6]]))
     a = o["rng"].normal(size=101)
     got = gpu.prodmm(terms, a, o["bm"], o["bs"], o["kp"])
     np.testing.assert_array_equal(got, o["ob"].matmul(terms, a))
     r = o["rng"].normal(size=10000)
-    assert relerr(gpu.tprodmm(terms, r, o["bm"], o["bs"], o["kp"]), o["ob"].tmatmul(terms, r)) < MATVEC_TOL
+    got = gpu.tprodmm(terms, r, o["bm"], o["bs"], o["kp"])
+    assert relerr(got, o["ob"].tmatmul(terms, r)) < MATVEC_TOL
+    np.testing.assert_array_equal(gpu.tprodmm(terms, r, o["bm"], o["bs"], o["kp"]), got)
 
 
 @pytest.mark.parametrize("covs", [None, ["mat25pow"] * 8, ["mat25ang", "mat25", "mat25pow", "mat25", "mat25", "mat25", "mat25", "mat25pow"]])
