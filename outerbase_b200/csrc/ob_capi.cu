@@ -27,7 +27,7 @@ struct ob_ctx { obd::Ctx c; explicit ob_ctx(int dev) : c(dev) {} };
 struct ob_outermod { obh::OuterMod om; };
 struct ob_outerbase { ob_ctx* ctx; std::unique_ptr<obe::OuterBase> ob; };
 struct ob_lpdf { ob_ctx* ctx; std::unique_ptr<obe::Lpdf> p; };
-struct ob_predictor { std::unique_ptr<obe::PredGauss> p; std::unique_ptr<obe::PredGda> pg; std::unique_ptr<obe::PredrStd> ps; };
+struct ob_predictor { std::unique_ptr<obe::Pred> p; };
 
 static void need(const void* p, const char* what) { if (!p) throw std::invalid_argument(std::string("null ") + what); }
 
@@ -569,18 +569,17 @@ int ob_predictor_create(ob_lpdf* loglik, ob_predictor** out) {
   OB_TRY
   auto* h = new ob_predictor();
   try {
-    if (auto* g3 = dynamic_cast<obe::LoglikStd*>(loglik->p.get())) h->ps.reset(new obe::PredrStd(*g3)); /* before its base class */
-    else if (auto* g = dynamic_cast<obe::LoglikGauss*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*g));
-    else if (auto* gm = dynamic_cast<obe::LoglikGaussMulti*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*gm));
-    else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(loglik->p.get())) h->pg.reset(new obe::PredGda(*g2));
+    if (auto* g3 = dynamic_cast<obe::LoglikStd*>(loglik->p.get())) h->p.reset(new obe::PredrStd(*g3)); /* before its base class */
+    else if (auto* g = dynamic_cast<obe::LoglikGaussBase*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*g));
+    else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(loglik->p.get())) h->p.reset(new obe::PredGda(*g2));
     else throw std::invalid_argument("cannot produce a predictor from this obj.");
   } catch (...) { delete h; throw; }
   *out = h;
   OB_CATCH
 }
 int ob_predictor_destroy(ob_predictor* p) { OB_TRY delete p; OB_CATCH }
-int ob_predictor_update(ob_predictor* p, const double* x, uint64_t N) { OB_TRY if (p->p) p->p->update(x, N); else if (p->pg) p->pg->update(x, N); else p->ps->update(x, N); OB_CATCH }
-int ob_predictor_mean(ob_predictor* p, double* out) { OB_TRY if (p->p) p->p->mean(out); else if (p->pg) p->pg->mean(out); else p->ps->mean(out); OB_CATCH }
-int ob_predictor_var(ob_predictor* p, double* out) { OB_TRY if (p->p) p->p->var(out); else if (p->pg) p->pg->var(out); else p->ps->var(out); OB_CATCH }
+int ob_predictor_update(ob_predictor* p, const double* x, uint64_t N) { OB_TRY p->p->update(x, N); OB_CATCH }
+int ob_predictor_mean(ob_predictor* p, double* out) { OB_TRY p->p->mean(out); OB_CATCH }
+int ob_predictor_var(ob_predictor* p, double* out) { OB_TRY p->p->var(out); OB_CATCH }
 
 } // extern "C"
