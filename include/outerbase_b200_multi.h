@@ -25,7 +25,9 @@
  * Refused on multi-response objects (OB_ERR_INVALID): the full Hessian (ob_lpdf_hess*, the full-Hessian branch of
  * lpdfvec), ob_lpdf_optnewton, and ob_lpdf_optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi).
  * ob_predictor_create on a loglik_gauss_multi: ob_predictor_mean writes N x C (Phi . coeff), ob_predictor_var writes
- * ONE N-vector shared by all columns (the total Hessian diagonal does not depend on the response).
+ * ONE N-vector shared by all columns (with shared para the total Hessian diagonal does not depend on the response).
+ * outerbase_b200_multi_percol.h declares the variants with one para entry per column (its own noise scale and
+ * coefficient scale for each response); when either child of the fit has them, ob_predictor_var writes N x C.
  */
 #ifndef OUTERBASE_B200_MULTI_H
 #define OUTERBASE_B200_MULTI_H

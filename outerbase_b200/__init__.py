@@ -20,6 +20,7 @@ LIBDIR = ROOT / "_lib"
 LIBPATH = LIBDIR / "libouterbase_b200.so"
 HEADER = REPO / "include" / "outerbase_b200.h"
 MULTI_HEADER = REPO / "include" / "outerbase_b200_multi.h"  # the multi-response extension
+PERCOL_HEADER = REPO / "include" / "outerbase_b200_multi_percol.h"  # its per-column para variants
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -33,7 +34,7 @@ def _stale() -> bool:
     if not LIBPATH.exists():
         return True
     t = LIBPATH.stat().st_mtime
-    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER]
+    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

@@ -217,11 +217,11 @@ class Library:
     def logpr_gauss(self, om, terms):
         return logpr_gauss(self, om, terms)
 
-    def loglik_gauss_multi(self, om, terms, Y, x):
-        return loglik_gauss_multi(self, om, terms, Y, x)
+    def loglik_gauss_multi(self, om, terms, Y, x, para_per_column=False):
+        return loglik_gauss_multi(self, om, terms, Y, x, para_per_column)
 
-    def logpr_gauss_multi(self, om, terms, ncol):
-        return logpr_gauss_multi(self, om, terms, ncol)
+    def logpr_gauss_multi(self, om, terms, ncol, para_per_column=False):
+        return logpr_gauss_multi(self, om, terms, ncol, para_per_column)
 
     def lpdfvec(self, a, b):
         if isinstance(a, _multi) or isinstance(b, _multi):
@@ -802,28 +802,39 @@ class _multi:
 
 
 class loglik_gauss_multi(_multi, lpdf):
-    """loglik_gauss on each column of Y (N x C), all columns on one basis (include/outerbase_b200.h)."""
+    """loglik_gauss on each column of Y (N x C), all columns on one basis (include/outerbase_b200_multi.h).
+    para_per_column: one noise log-sd per column (include/outerbase_b200_multi_percol.h) instead of one shared."""
 
-    def __init__(self, lib, om, terms, Y, x):
+    def __init__(self, lib, om, terms, Y, x, para_per_column=False):
         super().__init__(lib)
         self._om = om
+        self.para_per_column = bool(para_per_column)
         t, Y, x = _terms(terms), _f64(Y), _f64(x)
         if Y.ndim != 2:
             raise ValueError("Y must be N x C")
         if x.shape[0] != Y.shape[0]:
             raise ValueError("x and Y dims do not align")
-        lib.call("loglik_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _p(Y), _u(Y.shape[1]), _p(x), _u(Y.shape[0]),
-                 C.byref(self._h))
+        if self.para_per_column:
+            lib.call("loglik_gauss_multi_create_ex", lib.ctx, om._h, _p(t), _u(t.shape[0]), _p(Y), _u(Y.shape[1]), _p(x),
+                     _u(Y.shape[0]), C.c_int(1), C.byref(self._h))
+        else:
+            lib.call("loglik_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _p(Y), _u(Y.shape[1]), _p(x),
+                     _u(Y.shape[0]), C.byref(self._h))
 
 
 class logpr_gauss_multi(_multi, lpdf):
-    """An independent logpr_gauss on each of ncol coefficient columns, shared coeffscale."""
+    """An independent logpr_gauss on each of ncol coefficient columns, shared coeffscale (para_per_column: one
+    coeffscale per column)."""
 
-    def __init__(self, lib, om, terms, ncol):
+    def __init__(self, lib, om, terms, ncol, para_per_column=False):
         super().__init__(lib)
         self._om = om
+        self.para_per_column = bool(para_per_column)
         t = _terms(terms)
-        lib.call("logpr_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.byref(self._h))
+        if self.para_per_column:
+            lib.call("logpr_gauss_multi_create_ex", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.c_int(1), C.byref(self._h))
+        else:
+            lib.call("logpr_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.byref(self._h))
 
 
 class lpdfvec_multi(_multi, lpdfvec):
@@ -859,9 +870,21 @@ class predictor(_Handle):
 
 
 class predictor_multi(predictor):
-    """predictor(loglik_gauss_multi): mean N x C; var is one N-vector shared by all columns."""
+    """predictor(loglik_gauss_multi): mean N x C; var is one N-vector shared by all columns, or N x C when the
+    likelihood has a noise scale per column or was fitted under a prior with a coefficient scale per column."""
+
+    def __init__(self, lib, loglik):
+        super().__init__(lib, loglik)
+        self._var_ncol = int(loglik._get("predvar_ncol")[0])  # fixed when the predictor is made, as its variance
 
     def mean(self):
         out = np.empty((self._n, self._loglik.ncol), order="F")
         self._lib.call("predictor_mean", self._h, _p(out))
+        return out
+
+    def var(self):
+        if self._var_ncol == 1:
+            return super().var()
+        out = np.empty((self._n, self._loglik.ncol), order="F")
+        self._lib.call("predictor_var", self._h, _p(out))
         return out

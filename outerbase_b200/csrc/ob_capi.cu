@@ -5,6 +5,7 @@
  */
 #include "../../include/outerbase_b200.h"
 #include "../../include/outerbase_b200_multi.h"
+#include "../../include/outerbase_b200_multi_percol.h"
 
 #include "ob_engine.hpp"
 
@@ -464,25 +465,33 @@ int ob_logpr_gauss_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, u
   *out = h;
   OB_CATCH
 }
-int ob_loglik_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* Y, uint64_t C,
-                                 const double* x, uint64_t N, ob_lpdf** out) {
+int ob_loglik_gauss_multi_create_ex(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* Y, uint64_t C,
+                                    const double* x, uint64_t N, int para_per_column, ob_lpdf** out) {
   OB_TRY
   need(ctx, "ctx"); need(om, "om");
   if (C == 0) throw std::invalid_argument("ncol must be at least 1");
   auto* h = new ob_lpdf();
   h->ctx = ctx;
-  try { h->p.reset(new obe::LoglikGaussMulti(ctx->c, &om->om, terms, K, Y, C, x, N)); } catch (...) { delete h; throw; }
+  try { h->p.reset(new obe::LoglikGaussMulti(ctx->c, &om->om, terms, K, Y, C, x, N, para_per_column != 0)); } catch (...) { delete h; throw; }
   *out = h;
   OB_CATCH
 }
-int ob_logpr_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, uint64_t C, ob_lpdf** out) {
+int ob_loglik_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* Y, uint64_t C,
+                                 const double* x, uint64_t N, ob_lpdf** out) {
+  return ob_loglik_gauss_multi_create_ex(ctx, om, terms, K, Y, C, x, N, 0, out);
+}
+int ob_logpr_gauss_multi_create_ex(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, uint64_t C, int para_per_column,
+                                   ob_lpdf** out) {
   OB_TRY
   need(om, "om");
   auto* h = new ob_lpdf();
   h->ctx = ctx;
-  try { h->p.reset(new obe::LogprGaussMulti(&om->om, terms, K, C)); } catch (...) { delete h; throw; }
+  try { h->p.reset(new obe::LogprGaussMulti(&om->om, terms, K, C, para_per_column != 0)); } catch (...) { delete h; throw; }
   *out = h;
   OB_CATCH
+}
+int ob_logpr_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, uint64_t C, ob_lpdf** out) {
+  return ob_logpr_gauss_multi_create_ex(ctx, om, terms, K, C, 0, out);
 }
 int ob_lpdfvec_create(ob_lpdf* a, ob_lpdf* b, ob_lpdf** out) {
   OB_TRY
@@ -550,6 +559,11 @@ int ob_lpdf_get(ob_lpdf* l, const char* which, double* out, uint64_t* n) {
     if (mv && mv->multi()) v.assign(mv->cg_iters_cols.begin(), mv->cg_iters_cols.end());
     else v = {double(l->p->cg_iters)};
   } else if (w == "ncol") v = {double(l->p->ncol())};
+  else if (w == "predvar_ncol") {
+    auto* g = dynamic_cast<obe::LoglikGaussBase*>(l->p.get());
+    if (!g) throw std::invalid_argument("predvar_ncol is a field of loglik_gauss / loglik_gauss_multi");
+    v = {double(g->predvar_ncol())};
+  }
   else if (w == "yhat") {
     if (auto* g = dynamic_cast<obe::LoglikGauss*>(l->p.get())) v = g->get_yhat();
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(l->p.get())) v = g2->yhat;

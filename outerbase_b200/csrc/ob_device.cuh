@@ -288,7 +288,8 @@ enum CgStage : int {
 };
 /* Column-batched form (loglik_gauss_multi): the launch runs one CTA per column; coeff, grad, m, rm, p, q and red are K x C
  * column-major, scal holds CG_NSCAL scalars per column, sds is shared.  ncol = 1 with ssq = running = null is the
- * single-response launch. */
+ * single-response launch.  Per-column para: CTA c reads entry c of sca_col, obssd_col and vma_col instead of the
+ * scalar, for each of them that is set (uploaded once per optcg, not per iteration). */
 struct CgParams {
   int K, stage, lik_first, domarg;
   double* coeff; double* grad; const double* m; double* rm; double* p; double* q;
@@ -299,13 +300,17 @@ struct CgParams {
   const double* ssq = nullptr;  /* batched: per-column sums of squared residuals (red then holds K per column) */
   unsigned* running = nullptr;  /* batched: running[iter & 1] counts the columns that did not stop in CG_STEP of iteration iter */
   int iter = 0;
+  const double* sca_col = nullptr;    /* batched, per-column coefficient scale: C entries replacing sca */
+  const double* obssd_col = nullptr;  /* batched, per-column noise sd: C entries replacing obssd */
+  const double* vma_col = nullptr;    /* batched, per-column marginal adjustment: C entries replacing val_margadj */
 };
 enum { CG_NUM = 0, CG_DENOM, CG_ALPHA, CG_BETA, CG_VAL, CG_VALO, CG_VALDIFF, CG_STOP, CG_VAL_LIK, CG_VAL_PR, CG_ITER, CG_NSCAL = 16 };
 void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol = 1);
 /* after mm_mat_dev on C columns (leading dimension ld): update: w = -((yhat - y)/sd)/sd, ssq_out[c] = sum of
- * ((yhat - y)/sd)^2 over column c (fixed order); hessmult: w = (yhat/sd)/sd.  Pad rows of w are zero; yhat may alias w. */
+ * ((yhat - y)/sd)^2 over column c (fixed order); hessmult: w = (yhat/sd)/sd.  Pad rows of w are zero; yhat may alias w.
+ * sd_cols (device, C entries), when set, gives column c the sd sd_cols[c] instead of sd. */
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
-                        DevBuf<double>& partial, double* ssq_out);
+                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols = nullptr);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

@@ -726,6 +726,9 @@ struct Lpdf {
    * marginal adjustment, fit.cpp:259-263, only needs this contraction with c = 1 / diaghess) */
   virtual bool diaghessgradhyp_dot(const std::vector<double>&, std::vector<double>&) { return false; }
   virtual bool can_diaghessgradhyp_dot() const { return false; }
+  /* out[j] = sum_k diaghessgradpara[k, j] / dh[k] (lpdfvec's marginal adjustment, fit.cpp:264-266) without forming the
+   * nterms x npara matrix, when the object can; objects whose npara grows with the columns do */
+  virtual bool diaghessgradpara_dot(const std::vector<double>&, std::vector<double>&) { return false; }
   virtual void settotdiaghess(const std::vector<double>& dh) { totdiaghess = dh; didfulltothess = false; didnotothess = false; }
   /* full Hessian, fit.h:81-88: K x K, K x K x H, K x K x npara (column-major, slice after slice); empty when the
    * object has none (loglik_gauss, loglik_gda) */
@@ -739,6 +742,11 @@ struct Lpdf {
    * K x ncol column-major, nterms = K * ncol */
   virtual bool multi() const { return false; }
   virtual u64 ncol() const { return 1; }
+  /* multi-response objects with one para entry per column (for an lpdfvec: either child) */
+  virtual bool para_per_column() const { return false; }
+  /* set with totdiaghess by an lpdfvec with a per-column child: the total diagonal's K-long column blocks then differ,
+   * so a multi-response predictor gives one variance per column */
+  bool totdiaghess_percol = false;
 
   /* dense K x K algebra of the full-Hessian branch: host side, like every other K-sized object of the lpdf family */
   /* solve A X = B by elimination with partial pivoting (Armadillo solve(): LAPACK dgesv); B is n x m */
@@ -955,7 +963,10 @@ inline std::vector<double> tile_cols(const std::vector<double>& v, u64 K, u64 C)
  * order) of what the single-response object returns at that column, grad is K x C, and the Hessian diagonals, which do
  * not depend on the response, are computed once and repeated C times.  With C = 1 every formula is the reference's
  * own.  The subclasses are the two paths of the products: LoglikGauss (one vector, fused epilogues) and
- * LoglikGaussMulti (matrix products over the columns). */
+ * LoglikGaussMulti (matrix products over the columns).
+ * percol (para per column, multi-response only): npara = C, para[c] is column c's noise log-sd with loglik_gauss's
+ * default on that column; gradpara[c] is column c's own, and the Hessian diagonals are the one K-vector of squared
+ * column sums scaled by each column's exp(-2 para[c]) (diaghessgradpara: (K C) x C, block-diagonal). */
 struct LoglikGaussBase : Lpdf {
   Ctx& ctx;
   const OuterMod* om;
@@ -964,12 +975,16 @@ struct LoglikGaussBase : Lpdf {
   u64 N = 0, K = 0, C = 1;
   double Nglobal = 0;
   double obssd = 1;
+  bool percol = false;
+  std::vector<double> obssd_cols; /* C: column c's noise sd, exp(para[c]) (percol) or obssd */
   /* y, yhat, w: ld x C (pad rows zero) */
   DevBuf<double> y, yhat, w, kbuf, red, ones;
   std::vector<double> ssq_host; /* per-column sums of squared standardised residuals of the last update (all ranks) */
+  std::vector<double> sqcs;      /* the last sqcolsums(); empty after updateom / updateterms */
 
-  LoglikGaussBase(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
-      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_) {
+  LoglikGaussBase(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
+                  bool percol_ = false)
+      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_), percol(percol_) {
     if (C == 0) throw std::invalid_argument("ncol must be at least 1");
     d = om->d; npara = 1;
     terms.assign(t, t + K * d);
@@ -1001,12 +1016,26 @@ struct LoglikGaussBase : Lpdf {
       Nglobal = double(N);
       for (u64 j = 0; j < C; ++j) var[j] = arma_var(yh + j * N, N);
     }
-    double vs = 0;
-    for (double v : var) vs += v;
-    para0 = {std::log(0.01 * (vs / double(C)))};
-    paravar = {1};
+    if (percol) { /* column c: loglik_gauss's own default on Y[:,c] */
+      npara = C;
+      para0.resize(C);
+      for (u64 j = 0; j < C; ++j) para0[j] = std::log(0.01 * var[j]);
+      paravar.assign(C, 1.0);
+    } else {
+      double vs = 0;
+      for (double v : var) vs += v;
+      para0 = {std::log(0.01 * (vs / double(C)))};
+      paravar = {1};
+    }
     para = para0;
+    set_sds();
+  }
+  /* column c's entry of para */
+  double para_col(u64 c) const { return para[percol ? c : 0]; }
+  void set_sds() {
     obssd = std::exp(para[0]);
+    obssd_cols.resize(C);
+    for (u64 c = 0; c < C; ++c) obssd_cols[c] = percol ? std::exp(para[c]) : obssd;
   }
   void allreduce_host(double* v, u64 n) {
     red.upload(v, n, ctx.stream);
@@ -1027,14 +1056,24 @@ struct LoglikGaussBase : Lpdf {
   u64 nhyp() const override { return ob.H; }
   u64 nrow() const override { return N; }
   void setnthreads(int k) override { ob.nthreads = k; }
-  void updateom() override { ob.build(); }
-  void updatepara(const double* p, u64 n) override { para.assign(p, p + n); obssd = std::exp(para[0]); }
-  void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; }
-  double val_col(u64 c) const { return -0.5 * ssq_host[c] - Nglobal * std::log(obssd); }
+  void updateom() override { ob.build(); sqcs.clear(); }
+  bool para_per_column() const override { return percol; }
+  void updatepara(const double* p, u64 n) override {
+    if (percol && n != C) throw std::range_error("para must have one entry per column");
+    para.assign(p, p + n);
+    set_sds();
+  }
+  void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; sqcs.clear(); }
+  /* columns of the predictive variance of a predictor made from this likelihood now (PredGauss) */
+  u64 predvar_ncol() const { return multi() && (percol || totdiaghess_percol) ? C : 1; }
+  double val_col(u64 c) const { return -0.5 * ssq_host[c] - Nglobal * std::log(obssd_cols[c]); }
   /* val and gradpara of update() from ssq_host, loglik_gauss.cpp:121-129 */
   void set_val_gradpara() {
     if (compute_val) { val = 0; for (u64 c = 0; c < C; ++c) val += val_col(c); }
-    if (compute_grad && compute_gradpara) { gradpara = {0.0}; for (u64 c = 0; c < C; ++c) gradpara[0] += ssq_host[c] - Nglobal; }
+    if (compute_grad && compute_gradpara) {
+      if (percol) { gradpara.resize(C); for (u64 c = 0; c < C; ++c) gradpara[c] = ssq_host[c] - Nglobal; }
+      else { gradpara = {0.0}; for (u64 c = 0; c < C; ++c) gradpara[0] += ssq_host[c] - Nglobal; }
+    }
   }
 
   /* ---- device forms for the HBM-resident CG (LpdfVec::optcg_device), stream ordered: coefficients in, the likelihood
@@ -1055,19 +1094,47 @@ struct LoglikGaussBase : Lpdf {
     if (ones.cap < ob.ld) { ones.ensure(ob.ld); obd::launch_fill(ctx, ones.p, ob.ld, 1.0); }
     return ones.p;
   }
-  std::vector<double> diaghess() override { /* :154-157 */
+  /* the squared column sums Phi^2^T 1 (K), summed over ranks; kept in sqcs (they depend on the basis and the terms
+   * table only, not on para) */
+  std::vector<double> sqcolsums() {
     red.ensure(K);
     ob.tmm_dev(terms.data(), K, 1, ones_dev(), red.p);
-    std::vector<double> lh(K);
-    ob.d2h(lh.data(), red.p, K);
-    const double c = std::exp(-2 * para[0]);
-    for (double& v : lh) v = c * v;
-    return tile_cols(lh, K, C);
+    sqcs.resize(K);
+    ob.d2h(sqcs.data(), red.p, K);
+    return sqcs;
   }
+  /* (K C) x S from a K x S matrix: column block c scaled by exp(-2 para_c) (shared para: the same block repeated) */
+  std::vector<double> scale_cols(const std::vector<double>& v) const {
+    const u64 S = K ? v.size() / K : 0;
+    std::vector<double> o(K * C * S);
+    for (u64 c = 0; c < C; ++c) {
+      const double sc = std::exp(-2 * para_col(c));
+      for (u64 s = 0; s < S; ++s) for (u64 i = 0; i < K; ++i) o[(s * C + c) * K + i] = sc * v[s * K + i];
+    }
+    return o;
+  }
+  std::vector<double> diaghess() override { return scale_cols(sqcolsums()); } /* :154-157 */
   std::vector<double> diaghessgradpara() override { /* :176-179 */
     std::vector<double> lh = diaghess();
     for (double& v : lh) v = -2 * v;
-    return lh;
+    if (!percol) return lh;
+    std::vector<double> o(K * C * C, 0.0); /* block-diagonal: para c moves column c only */
+    for (u64 c = 0; c < C; ++c) std::copy(lh.begin() + c * K, lh.begin() + (c + 1) * K, o.begin() + c * K * C + c * K);
+    return o;
+  }
+  /* out[c] = sum_k diaghessgradpara[k, c] / dh[k] over column c's block, without the (K C) x C matrix; reuses the
+   * squared column sums of the diaghess() that formed dh (lpdfvec's buildhess) */
+  bool diaghessgradpara_dot(const std::vector<double>& dh, std::vector<double>& out) override {
+    if (!percol || dh.size() != K * C) return false;
+    const std::vector<double> lh = sqcs.size() == K ? sqcs : sqcolsums();
+    out.assign(C, 0.0);
+    std::vector<double> t(K);
+    for (u64 c = 0; c < C; ++c) {
+      const double sc = std::exp(-2 * para[c]);
+      for (u64 i = 0; i < K; ++i) t[i] = -2 * (sc * lh[i]) / dh[c * K + i];
+      out[c] = obh::sum2(t.data(), K);
+    }
+    return true;
   }
   std::vector<double> diaghessgradhyp() override { /* :165-168 */
     const u64 H = ob.H;
@@ -1075,14 +1142,12 @@ struct LoglikGaussBase : Lpdf {
     ob.tmm_ge_dev(terms.data(), K, 1, ones_dev(), red.p);
     std::vector<double> all(K * (1 + H));
     ob.d2h(all.data(), red.p, K * (1 + H));
-    std::vector<double> o(all.begin() + K, all.end());
-    const double c = std::exp(-2 * para[0]);
-    for (double& v : o) v = c * v;
-    return tile_cols(o, K, C);
+    return scale_cols(std::vector<double>(all.begin() + K, all.end()));
   }
   bool can_diaghessgradhyp_dot() const override { return ctx.dsweep; }
   /* sum_k c_k sum_n d(Phi^2)[n,k]/dhyp = sum_n d(Phi^2 c)[n]/dhyp: the hyper-gradient sweep on the squared operator.
-   * Linear in c: the columns' weights are summed first, then ONE sweep.  The swept / not-swept decision is COLLECTIVE:
+   * Linear in c: the columns' weights (each scaled by its exp(-2 para_c) when para is per column) are summed first, then
+   * ONE sweep.  The swept / not-swept decision is COLLECTIVE:
    * slot H of the reduction buffer counts the ranks whose sweep was unavailable (module build failure, table not
    * specialised, geometry), so every rank takes the same branch and the allreduce sequence stays aligned (the fallback
    * is a K*(1+H) allreduce in diaghessgradhyp()). */
@@ -1090,7 +1155,13 @@ struct LoglikGaussBase : Lpdf {
     const u64 H = ob.H;
     if (!ctx.dsweep || cv.size() != K * C || H == 0) return false;
     std::vector<double> s(K, 0.0);
-    for (u64 c = 0; c < C; ++c) for (u64 i = 0; i < K; ++i) s[i] += cv[c * K + i];
+    if (percol) /* each column's weights scaled by its own exp(-2 para_c); the result is then not scaled again */
+      for (u64 c = 0; c < C; ++c) {
+        const double sc = std::exp(-2 * para[c]);
+        for (u64 i = 0; i < K; ++i) s[i] += sc * cv[c * K + i];
+      }
+    else /* shared para: plain sums, scaled once after the sweep */
+      for (u64 c = 0; c < C; ++c) for (u64 i = 0; i < K; ++i) s[i] += cv[c * K + i];
     kbuf.upload(s, ctx.stream);
     red.ensure(H + 1);
     OB_CUDA(cudaMemsetAsync(red.p, 0, (H + 1) * sizeof(double), ctx.stream));
@@ -1105,6 +1176,7 @@ struct LoglikGaussBase : Lpdf {
     ob.d2h(r.data(), red.p, H + 1);
     if (r[H] != 0.0) return false; /* some rank could not sweep: all ranks fall back together */
     out.assign(r.begin(), r.begin() + H);
+    if (percol) return true;
     const double sc = std::exp(-2 * para[0]);
     for (double& v : out) v = sc * v;
     return true;
@@ -1370,25 +1442,55 @@ struct LoglikGda : Lpdf {
 
 /* ------------------------------------------------------------------ multi-response: C responses observed at the same rows
  * Every column is the single-response model on its own response, all columns share the basis, the terms table, the
- * hyper-parameters and both para entries.  val, gradhyp and gradpara are the sums over the columns (in column order) of
- * what the single-response object returns at that column, grad is K x C, the Hessian product is block-diagonal and the
- * Hessian diagonals are the single-response ones repeated C times.  The objective is meant for lpdfvec's diagonal
+ * hyper-parameters and both para entries (or, opted in per object, one para entry per column: its own noise scale or
+ * coefficient scale).  val, gradhyp and gradpara are the sums over the columns (in column order) of what the
+ * single-response object returns at that column, grad is K x C, the Hessian product is block-diagonal and the Hessian
+ * diagonals are the single-response ones repeated C times (per-column para: each column's own).  The objective is meant for lpdfvec's diagonal
  * branch and its column-batched CG (LpdfVec::optcg_device); the full Hessian, optnewton and the host optcg are refused. */
 
-struct LogprGaussMulti : Lpdf { /* an independent logpr_gauss on each column, shared coeffscale */
+/* an independent logpr_gauss on each column, shared coeffscale; percol: npara = C, para[c] is column c's coeffscale with
+ * logpr_gauss's para0 and paravar, gradpara[c] is column c's own and the Hessian diagonals are per column
+ * (diaghessgradpara: (K C) x C, block-diagonal) */
+struct LogprGaussMulti : Lpdf {
   LogprGauss one;
   u64 K, C;
+  bool percol;
   std::vector<double> val_cols;
-  LogprGaussMulti(const OuterMod* om_, const u64* t, u64 K_, u64 C_) : one(om_, t, K_), K(K_), C(C_) {
+  LogprGaussMulti(const OuterMod* om_, const u64* t, u64 K_, u64 C_, bool percol_ = false) : one(om_, t, K_), K(K_), C(C_), percol(percol_) {
     if (C == 0) throw std::invalid_argument("ncol must be at least 1");
     d = one.d; npara = one.npara; terms = one.terms; para0 = one.para0; paravar = one.paravar; para = one.para;
+    if (percol) {
+      npara = C;
+      para0.assign(C, one.para0[0]); paravar.assign(C, one.paravar[0]); para = para0;
+    }
     nterms = K * C;
+  }
+  /* point `one` at column c's para (shared para: it is always there) */
+  void at(u64 c) { if (percol) one.updatepara(&para[c], 1); }
+  double sca_col(u64 c) const { return percol ? std::exp(para[c]) : one.sca; }
+  /* (K C) x S: column c's K x S result, for every c (shared para: one result repeated) */
+  template <class F> std::vector<double> per_col(F f) {
+    if (!percol) return tile_cols(f(), K, C);
+    std::vector<double> o;
+    for (u64 c = 0; c < C; ++c) {
+      at(c);
+      const std::vector<double> v = f();
+      const u64 S = K ? v.size() / K : 0;
+      o.resize(K * C * S);
+      for (u64 s = 0; s < S; ++s) std::copy(v.begin() + s * K, v.begin() + (s + 1) * K, o.begin() + (s * C + c) * K);
+    }
+    return o;
   }
   bool multi() const override { return true; }
   u64 ncol() const override { return C; }
+  bool para_per_column() const override { return percol; }
   u64 nhyp() const override { return one.nhyp(); }
   void updateom() override { one.updateom(); }
-  void updatepara(const double* p, u64 n) override { one.updatepara(p, n); para = one.para; }
+  void updatepara(const double* p, u64 n) override {
+    if (!percol) { one.updatepara(p, n); para = one.para; return; }
+    if (n != C) throw std::range_error("para must have one entry per column");
+    para.assign(p, p + n);
+  }
   void updateterms(const u64* t, u64 K_) override { one.updateterms(t, K_); terms = one.terms; K = K_; nterms = K * C; }
   std::vector<double> column(const std::vector<double>& v, u64 c) const { return std::vector<double>(v.begin() + c * K, v.begin() + (c + 1) * K); }
   void update(const std::vector<double>& cf) override {
@@ -1398,30 +1500,53 @@ struct LogprGaussMulti : Lpdf { /* an independent logpr_gauss on each column, sh
     if (compute_val) { val = 0; val_cols.assign(C, 0.0); }
     if (compute_grad) grad.assign(K * C, 0.0);
     if (compute_gradhyp) gradhyp.assign(one.nhyp(), 0.0);
-    if (compute_gradpara) gradpara.assign(1, 0.0);
+    if (compute_gradpara) gradpara.assign(percol ? C : 1, 0.0);
     for (u64 c = 0; c < C; ++c) {
+      at(c);
       one.update(column(cf, c));
       if (compute_val) { val += one.val; val_cols[c] = one.val; }
       if (compute_grad) std::copy(one.grad.begin(), one.grad.end(), grad.begin() + c * K);
       if (compute_gradhyp) for (u64 h = 0; h < gradhyp.size(); ++h) gradhyp[h] += one.gradhyp[h];
-      if (compute_gradpara) gradpara[0] += one.gradpara[0];
+      if (compute_gradpara) gradpara[percol ? c : 0] += one.gradpara[0];
     }
   }
   std::vector<double> hessmult(const std::vector<double>& g) override {
     if (g.size() != K * C) throw std::range_error("g must have K x ncol entries");
     std::vector<double> o(K * C);
-    for (u64 c = 0; c < C; ++c) { const std::vector<double> h = one.hessmult(column(g, c)); std::copy(h.begin(), h.end(), o.begin() + c * K); }
+    for (u64 c = 0; c < C; ++c) { at(c); const std::vector<double> h = one.hessmult(column(g, c)); std::copy(h.begin(), h.end(), o.begin() + c * K); }
     return o;
   }
-  std::vector<double> diaghess() override { return tile_cols(one.diaghess(), K, C); }
-  std::vector<double> diaghessgradhyp() override { return tile_cols(one.diaghessgradhyp(), K, C); }
-  std::vector<double> diaghessgradpara() override { return tile_cols(one.diaghessgradpara(), K, C); }
+  std::vector<double> diaghess() override { return per_col([&] { return one.diaghess(); }); }
+  std::vector<double> diaghessgradhyp() override { return per_col([&] { return one.diaghessgradhyp(); }); }
+  std::vector<double> diaghessgradpara() override {
+    if (!percol) return tile_cols(one.diaghessgradpara(), K, C);
+    std::vector<double> o(K * C * C, 0.0); /* block-diagonal: para c moves column c only */
+    for (u64 c = 0; c < C; ++c) {
+      at(c);
+      const std::vector<double> v = one.diaghessgradpara();
+      std::copy(v.begin(), v.end(), o.begin() + c * K * C + c * K);
+    }
+    return o;
+  }
+  bool diaghessgradpara_dot(const std::vector<double>& dh, std::vector<double>& out) override {
+    if (!percol || dh.size() != K * C) return false;
+    out.assign(C, 0.0);
+    std::vector<double> t(K);
+    for (u64 c = 0; c < C; ++c) {
+      at(c);
+      const std::vector<double> v = one.diaghessgradpara();
+      for (u64 i = 0; i < K; ++i) t[i] = v[i] / dh[c * K + i];
+      out[c] = obh::sum2(t.data(), K);
+    }
+    return true;
+  }
   bool can_diaghessgradhyp_dot() const override { return true; }
   bool diaghessgradhyp_dot(const std::vector<double>& cv, std::vector<double>& out) override {
     if (cv.size() != K * C) return false;
     out.assign(one.nhyp(), 0.0);
     std::vector<double> o;
     for (u64 c = 0; c < C; ++c) {
+      at(c);
       one.diaghessgradhyp_dot(column(cv, c), o);
       for (u64 h = 0; h < out.size(); ++h) out[h] += o[h];
     }
@@ -1438,24 +1563,34 @@ struct LogprGaussMulti : Lpdf { /* an independent logpr_gauss on each column, sh
  * table, else column loops) with the residual pass resid_multi between them */
 struct LoglikGaussMulti : LoglikGaussBase {
   DevBuf<double> ssq, partial, gh;
+  DevBuf<double> sd_dev; /* percol: obssd_cols on the device, refreshed by updatepara */
 
-  LoglikGaussMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
-      : LoglikGaussBase(c, om_, t, K_, yh, C_, xh, N_) {
+  LoglikGaussMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
+                   bool percol_ = false)
+      : LoglikGaussBase(c, om_, t, K_, yh, C_, xh, N_, percol_) {
     ssq.ensure(C);
+    upload_sds();
   }
   bool multi() const override { return true; }
+  void upload_sds() {
+    if (!percol) return;
+    sd_dev.upload(obssd_cols, ctx.stream);
+    ctx.sync(); /* obssd_cols may change at the next updatepara */
+  }
+  void updatepara(const double* p, u64 n) override { LoglikGaussBase::updatepara(p, n); upload_sds(); }
+  const double* sd_cols_dev() const { return percol ? sd_dev.p : nullptr; }
 
   /* ssq[c]: column c's sum of squared standardised residuals, summed over ranks */
   void update_dev(const double* coeff_dev) override {
     ob.mm_mat_dev(terms.data(), K, 0, coeff_dev, C, yhat.p, ob.ld);
-    obd::launch_resid_multi(ctx, yhat.p, y.p, w.p, N, ob.ld, C, obssd, true, partial, ssq.p);
+    obd::launch_resid_multi(ctx, yhat.p, y.p, w.p, N, ob.ld, C, obssd, true, partial, ssq.p, sd_cols_dev());
     red.ensure(K * C);
     ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
     ctx.allreduce_sum(ssq.p, C);
   }
   void hessmult_dev(const double* g_dev) override { /* loglik_gauss.cpp:137-145 per column; w holds Phi g until the residual pass */
     ob.mm_mat_dev(terms.data(), K, 0, g_dev, C, w.p, ob.ld);
-    obd::launch_resid_multi(ctx, w.p, nullptr, w.p, N, ob.ld, C, obssd, false, partial, nullptr);
+    obd::launch_resid_multi(ctx, w.p, nullptr, w.p, N, ob.ld, C, obssd, false, partial, nullptr, sd_cols_dev());
     red.ensure(K * C);
     ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
   }
@@ -1499,6 +1634,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   std::vector<double> diaghessv, diaghessgradhypv, diaghessgradparav;
   std::vector<double> hessv, hessgradhypv, hessgradparav; /* full-Hessian branch, fit.h:121-123 */
   bool hyp_matrix_stale = false; /* buildhess took the contracted route: the K x H matrix is formed on demand */
+  bool para_matrix_stale = false; /* likewise for the nterms x npara matrix (per-column para) */
   bool redohess = true;
   Lpdf* kid[2];
   u64 parasrt[2], paraend[2];
@@ -1549,7 +1685,10 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     }
     return out;
   }
-  void settotdiaghess(const std::vector<double>& dh) override { totdiaghess = dh; for (Lpdf* l : kid) l->settotdiaghess(dh); }
+  void settotdiaghess(const std::vector<double>& dh) override {
+    totdiaghess = dh;
+    for (Lpdf* l : kid) { l->settotdiaghess(dh); l->totdiaghess_percol = para_per_column(); }
+  }
   void settothess(const std::vector<double>& h) override { tothess = h; for (Lpdf* l : kid) l->settothess(h); } /* :609-612 */
   std::vector<double> hess() override { return hessv; }
   std::vector<double> hessgradhyp() override { return hessgradhypv; }
@@ -1661,7 +1800,14 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
                            kid[1]->diaghessgradhyp_dot(cinv, dot1) && kid[0]->diaghessgradhyp_dot(cinv, dot0) && dot0.size() == dot1.size();
         if (swept) { diaghessgradhypv.clear(); hyp_matrix_stale = true; }
         else { diaghessgradhypv = diaghessgradhyp_(); hyp_matrix_stale = false; }
-        diaghessgradparav = diaghessgradpara_();
+        /* per-column children contract their para derivatives directly: with P growing with C, the dense
+         * nterms x P matrix is what would dominate (formed on demand, diaghessgradpara()) */
+        std::vector<double> pdot[2];
+        bool pdone[2];
+        for (int c = 0; c < 2; ++c) pdone[c] = kid[c]->diaghessgradpara_dot(diaghessv, pdot[c]);
+        para_matrix_stale = pdone[0] || pdone[1];
+        if (para_matrix_stale) diaghessgradparav.clear();
+        else diaghessgradparav = diaghessgradpara_();
         const u64 H = swept ? dot0.size() : diaghessgradhypv.size() / std::max<u64>(K, 1), P = para.size();
         std::vector<double> t(K);
         for (u64 i = 0; i < K; ++i) t[i] = std::log(diaghessv[i]);
@@ -1673,10 +1819,21 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
           gradhyp_margadj[h] = -0.5 * obh::sum2(t.data(), K);
         }
         gradpara_margadj.assign(P, 0.0);
-        for (u64 h = 0; h < P; ++h) {
-          for (u64 i = 0; i < K; ++i) t[i] = diaghessgradparav[i + h * K] / diaghessv[i];
-          gradpara_margadj[h] = -0.5 * obh::sum2(t.data(), K);
-        }
+        if (!para_matrix_stale)
+          for (u64 h = 0; h < P; ++h) {
+            for (u64 i = 0; i < K; ++i) t[i] = diaghessgradparav[i + h * K] / diaghessv[i];
+            gradpara_margadj[h] = -0.5 * obh::sum2(t.data(), K);
+          }
+        else
+          for (int c = 0; c < 2; ++c) {
+            const u64 nc = paraend[c] + 1 - parasrt[c];
+            if (pdone[c]) { for (u64 j = 0; j < nc; ++j) gradpara_margadj[parasrt[c] + j] = -0.5 * pdot[c][j]; continue; }
+            const std::vector<double> h = kid[c]->diaghessgradpara();
+            for (u64 j = 0; j < nc; ++j) {
+              for (u64 i = 0; i < K; ++i) t[i] = h[i + j * K] / diaghessv[i];
+              gradpara_margadj[parasrt[c] + j] = -0.5 * obh::sum2(t.data(), K);
+            }
+          }
       }
       if (fullhess) buildhess_full();
     }
@@ -1723,10 +1880,11 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
    * K C system, which would share alpha and beta over the columns.  cg_stage_kernel runs one CTA per column; a column
    * whose stop test passes is frozen as the reference `break`s, and the loop ends when no column runs (the value the
    * host reads is the count of running columns) or after maxepch.  The products of an iteration run over all C columns,
-   * frozen ones included.
+   * frozen ones included.  When either child has per-column para, the columns' diagonals differ: each column's
+   * marginal adjustment, coefficient scale and noise sd go to the kernel as C-entry device arrays, uploaded here once.
    * A single-response pairing returns false (the caller runs the host loop) without option device_cg, rows or a
    * specialised terms table, and for every other pairing; a multi-response object runs here or throws. */
-  DevBuf<double> cg_coeff, cg_grad, cg_m, cg_rm, cg_p, cg_q, cg_sds, cg_scal;
+  DevBuf<double> cg_coeff, cg_grad, cg_m, cg_rm, cg_p, cg_q, cg_sds, cg_scal, cg_sca, cg_vma;
   DevBuf<unsigned> cg_running;
   std::vector<u64> cg_iters_cols;
   bool optcg_device(double tol, u64 maxepch) {
@@ -1753,24 +1911,27 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     if (!all_finite(m) && !all_finite(grad)) { val = -std::numeric_limits<double>::infinity(); return true; }
     /* the starting value of each run: single response, the lpdfvec's own; multi-response, column c's value as the
      * single-response lpdfvec forms it (fit.cpp:352-380): children in order, then its own marginal adjustment -- the
-     * first K entries of the repeated diagonal are the single-response diagonal */
-    double vma = val_margadj;
-    if (mult) {
-      vma = 0;
-      if (domargadj) {
+     * diagonal's column block c is column c's single-response diagonal (with shared para, every block is block 0) */
+    const bool percol = mult && (lk->percol || prm->percol);
+    std::vector<double> vma_cols(percol ? C : 1, val_margadj);
+    if (mult)
+      for (u64 c = 0; c < vma_cols.size(); ++c) {
+        vma_cols[c] = 0;
+        if (!domargadj) continue;
         std::vector<double> t(K);
-        for (u64 i = 0; i < K; ++i) t[i] = std::log(diaghessv[i]);
-        vma = -0.5 * obh::sum2(t.data(), K);
+        for (u64 i = 0; i < K; ++i) t[i] = std::log(diaghessv[c * K + i]);
+        vma_cols[c] = -0.5 * obh::sum2(t.data(), K);
       }
-    }
-    std::vector<double> scal(C * NS, 0.0);
+    const double vma = vma_cols[0];
+    std::vector<double> scal(C * NS, 0.0), sca_cols;
     for (u64 c = 0; c < C; ++c) {
       double v = val;
       if (mult) {
         const double vl = lk->val_col(c), vp = prm->val_cols[c];
         v = lik_first ? (0.0 + vl) + vp : (0.0 + vp) + vl;
-        if (domargadj) v += vma;
+        if (domargadj) v += vma_cols[percol ? c : 0];
       }
+      if (percol) sca_cols.push_back(prm->sca_col(c));
       double* S = scal.data() + c * NS;
       S[obd::CG_VAL] = v; S[obd::CG_VALO] = v; S[obd::CG_VALDIFF] = 10; S[obd::CG_DENOM] = 1;
     }
@@ -1778,6 +1939,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     cg_sds.upload(pr->coeffsd, ctx.stream);
     cg_rm.ensure(K * C); cg_p.ensure(K * C); cg_q.ensure(K * C);
     cg_scal.upload(scal, ctx.stream);
+    if (percol) { cg_sca.upload(sca_cols, ctx.stream); cg_vma.upload(vma_cols, ctx.stream); }
     if (mult) cg_running.ensure(2);
     ctx.sync(); /* the host images above must outlive the uploads */
     obd::CgParams c{};
@@ -1785,6 +1947,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     c.coeff = cg_coeff.p; c.grad = cg_grad.p; c.m = cg_m.p; c.rm = cg_rm.p; c.p = cg_p.p; c.q = cg_q.p; c.sds = cg_sds.p;
     c.sca = pr->sca; c.obssd = lk->obssd; c.nglobal = lk->Nglobal; c.val_margadj = vma; c.tol = tol; c.scal = cg_scal.p;
     if (mult) { c.ssq = static_cast<LoglikGaussMulti*>(lk)->ssq.p; c.running = cg_running.p; }
+    if (percol) { c.sca_col = cg_sca.p; c.vma_col = cg_vma.p; c.obssd_col = static_cast<LoglikGaussMulti*>(lk)->sd_cols_dev(); }
     auto stage = [&](int st) { c.stage = st; c.red = lk->red.p; obd::launch_cg_stage(ctx, c, C); };
     stage(obd::CG_INIT);          /* rm = grad / m ; p = rm                       :58-60 */
     lk->hessmult_dev(cg_p.p);     /* q = hessmult(p), finished inside CG_STEP     :62 */
@@ -1826,12 +1989,16 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   }
   bool multi() const override { return kid[0]->multi(); }
   u64 ncol() const override { return kid[0]->ncol(); }
+  bool para_per_column() const override { return kid[0]->para_per_column() || kid[1]->para_per_column(); }
   std::vector<double> diaghess() override { return diaghessv; }
   std::vector<double> diaghessgradhyp() override {
     if (hyp_matrix_stale) { diaghessgradhypv = diaghessgradhyp_(); hyp_matrix_stale = false; }
     return diaghessgradhypv;
   }
-  std::vector<double> diaghessgradpara() override { return diaghessgradparav; }
+  std::vector<double> diaghessgradpara() override {
+    if (para_matrix_stale) { diaghessgradparav = diaghessgradpara_(); para_matrix_stale = false; }
+    return diaghessgradparav;
+  }
   double paralpdf(const double* p, u64 n) const override {
     if (n != para.size()) return -std::numeric_limits<double>::infinity();
     double out = 0;
@@ -1878,10 +2045,14 @@ struct Pred {
 
 struct PredGauss : Pred { /* loglik_gauss.cpp:196-227 */
   std::vector<double> coeffvar;
-  /* multi-response: the variance is one N-vector for all columns (the total Hessian diagonal is the same K-vector
-   * repeated over the columns) */
-  PredGauss(LoglikGaussBase& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.K, lk.C) {
-    if (!lk.multi()) coeffvar = inv_totdiaghess(lk);
+  bool percol, lik_percol;
+  /* multi-response, shared para everywhere: the variance is one N-vector for all columns (the total Hessian diagonal is
+   * the same K-vector repeated over the columns).  When the likelihood has per-column para, or its total diagonal came
+   * from an lpdfvec with a per-column prior, the columns' diagonals differ: N x C, column c = Phi^2 V[:,c] +
+   * exp(2 para_c) with V the K x C matrix of 1 / totdiaghess, as ONE squared multi-right-hand-side product. */
+  PredGauss(LoglikGaussBase& lk)
+      : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.K, lk.C), percol(lk.predvar_ncol() > 1), lik_percol(lk.percol) {
+    if (!lk.multi() || percol) coeffvar = inv_totdiaghess(lk);
     else {
       coeffvar.assign(K, 0.0);
       if (!lk.didnotothess && lk.totdiaghess.size() >= K)
@@ -1889,6 +2060,15 @@ struct PredGauss : Pred { /* loglik_gauss.cpp:196-227 */
     }
   }
   void var(double* out) override {
+    if (percol) {
+      if (coeffvar.size() != K * C) throw std::invalid_argument("predictor: the total Hessian diagonal must have K x ncol entries");
+      ob->mm_mat(1, terms.data(), K, coeffvar.data(), C, out);
+      for (u64 c = 0; c < C; ++c) {
+        const double v = std::exp(2 * para[lik_percol ? c : 0]);
+        for (u64 i = 0; i < ob->N; ++i) out[c * ob->N + i] += v;
+      }
+      return;
+    }
     ob->mm(1, terms.data(), K, coeffvar.data(), out);
     const double c = std::exp(2 * para[0]);
     for (u64 i = 0; i < ob->N; ++i) out[i] += c;

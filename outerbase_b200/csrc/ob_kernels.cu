@@ -521,14 +521,17 @@ __global__ void colsum_partials_kernel(const double* __restrict__ partial, int n
 }
 
 /* Residuals of C columns after a plain product, the PHI_UPDATE / PHI_HESS epilogue of phi_a_kernel column by column
- * (same expressions, so a column's w equals the trie kernel's bit for bit given the same yhat).  grid (nb, C);
+ * (same expressions, so a column's w equals the trie kernel's bit for bit given the same yhat and sd).  grid (nb, C);
  * rows N .. ld-1 of w are written as zero (phi_tm_spec and phi_t_spec read pad rows, they must be finite).  update:
- * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w. */
+ * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w.
+ * sds, when set, holds one sd per column (per-column noise) and replaces the scalar sd. */
 constexpr int kResidThreads = 256;
 __global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double* yhat, const double* __restrict__ y, double* w, u64 N,
-                                                                   u64 ld, double sd, int update, double* __restrict__ partial) {
+                                                                   u64 ld, double sd0, const double* __restrict__ sds, int update,
+                                                                   double* __restrict__ partial) {
   __shared__ double sm[kResidThreads];
   const u64 col = blockIdx.y, base = col * ld;
+  const double sd = sds ? sds[col] : sd0;
   double s = 0.0;
   for (u64 i = (u64)blockIdx.x * kResidThreads + threadIdx.x; i < ld; i += (u64)gridDim.x * kResidThreads) {
     double wv = 0.0;
@@ -1314,7 +1317,7 @@ void launch_phi_a(Ctx& c, const PhiPlan& pl, const PhiAArgs& a, Workspace& ws, i
       nb = (int)std::min<u64>((ld + kResidThreads - 1) / kResidThreads, (u64)c.sms);
       const bool update = a.mode == PHI_UPDATE;
       double* part = update ? (a.ssq_partial ? a.ssq_partial : ws.ssq.ensure(c.sms)) : nullptr;
-      resid_multi_kernel<<<dim3((unsigned)nb, 1), kResidThreads, 0, c.stream>>>(yv, a.y, a.w, pl.N, ld, a.sd, update ? 1 : 0, part);
+      resid_multi_kernel<<<dim3((unsigned)nb, 1), kResidThreads, 0, c.stream>>>(yv, a.y, a.w, pl.N, ld, a.sd, nullptr, update ? 1 : 0, part);
       check_launch(c, "resid_multi_kernel");
     }
     if (grid_out) *grid_out = a.mode == PHI_UPDATE ? nb : 0;
@@ -1419,6 +1422,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
   c.coeff += off; c.grad += off; c.m += off; c.rm += off; c.p += off; c.q += off; c.red += off;
   double* S = c.scal + (size_t)blockIdx.x * CG_NSCAL;
   if (c.running && S[CG_STOP] != 0.0) return;
+  const double sca = c.sca_col ? c.sca_col[blockIdx.x] : c.sca;
   if (c.stage == CG_INIT) {
     for (int i = tid; i < K; i += kCgThreads) { const double rm = c.grad[i] / c.m[i]; c.rm[i] = rm; c.p[i] = rm; }
     return;
@@ -1428,7 +1432,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
      * lpdfvec::update's sums over the children in their order (fit.cpp:352-361) */
     double s1 = 0.0, s2 = 0.0;
     for (int i = tid; i < K; i += kCgThreads) {
-      const double sd = c.sds[i] * c.sca;
+      const double sd = c.sds[i] * sca;
       const double st = c.coeff[i] / sd;
       s1 += st * st;
       s2 += log(sd);
@@ -1438,9 +1442,9 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
     const double t1 = cg_block_sum(s1, sm), t2 = cg_block_sum(s2, sm);
     const double val_pr = -0.5 * t1 - t2;
     const double ssq = c.ssq ? c.ssq[blockIdx.x] : c.red[K];
-    const double val_lik = -0.5 * ssq - c.nglobal * log(c.obssd);
+    const double val_lik = -0.5 * ssq - c.nglobal * log(c.obssd_col ? c.obssd_col[blockIdx.x] : c.obssd);
     double val = c.lik_first ? (0.0 + val_lik) + val_pr : (0.0 + val_pr) + val_lik;
-    if (c.domarg) val += c.val_margadj;
+    if (c.domarg) val += c.vma_col ? c.vma_col[blockIdx.x] : c.val_margadj;
     const double valo = S[CG_VALO], alpha = S[CG_ALPHA], num = S[CG_NUM];
     double s3 = 0.0;
     for (int i = tid; i < K; i += kCgThreads) {
@@ -1458,7 +1462,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
    * logpr_gauss::hessmult = p / (sd sca)^2 (logpr_gauss.cpp:112-114) */
   double sn = 0.0, sd_ = 0.0;
   for (int i = tid; i < K; i += kCgThreads) {
-    const double sd = c.sds[i] * c.sca;
+    const double sd = c.sds[i] * sca;
     const double hp = c.p[i] / (sd * sd), hl = c.red[i];
     const double q = c.lik_first ? hl + hp : hp + hl;
     c.q[i] = q;
@@ -1487,7 +1491,7 @@ void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol) {
 }
 
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
-                        DevBuf<double>& partial, double* ssq_out) {
+                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols) {
   if (C == 0) return;
   if (ld == 0) { /* a rank without rows still takes part in the sums over ranks */
     if (update) OB_CUDA(cudaMemsetAsync(ssq_out, 0, C * sizeof(double), c.stream));
@@ -1495,7 +1499,7 @@ void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, 
   }
   const int nb = (int)std::max<u64>(1, std::min<u64>((ld + kResidThreads - 1) / kResidThreads, std::max<u64>(1, (u64)c.sms * 8 / C)));
   if (update) partial.ensure((size_t)nb * C);
-  resid_multi_kernel<<<dim3((unsigned)nb, (unsigned)C), kResidThreads, 0, c.stream>>>(yhat, y, w, N, ld, sd, update ? 1 : 0,
+  resid_multi_kernel<<<dim3((unsigned)nb, (unsigned)C), kResidThreads, 0, c.stream>>>(yhat, y, w, N, ld, sd, sd_cols, update ? 1 : 0,
                                                                                       update ? partial.p : nullptr);
   check_launch(c, "resid_multi_kernel");
   if (!update) return;

@@ -311,10 +311,12 @@ def obfit(lib, x, y, numb=100, verbose=0, covnames=None, hyp=None, numberopts=2,
                 predobj=lib.predictor(loglik_faster), optinfo=optinfo, stage1=dict(logpdf=logpdf, loglik=loglik, rows=subset))
 
 
-def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verbose=0, knots=40):
+def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verbose=0, knots=40, para_per_column=False):
     """obfit_gauss for C responses observed at the same inputs (Y is N x C): each column standardised on its own, then
     the same stage-2 loop on lpdfvec(logpr_gauss_multi, loglik_gauss_multi) with domarg -- one basis, one terms table,
-    shared hyper-parameters and para, one independent CG per column inside every objective evaluation."""
+    shared hyper-parameters and para, one independent CG per column inside every objective evaluation.
+    para_per_column: each column gets its own noise scale and coefficient scale (para has 2 C entries), for outputs
+    whose signal-to-noise ratios differ; the hyper-parameters stay shared."""
     x = np.asfortranarray(np.asarray(x, dtype=float))
     Y = np.asarray(Y, dtype=float)
     if Y.ndim != 2:
@@ -332,8 +334,9 @@ def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verb
         om.updatehyp(hyp)
     om.setknot(genknotlist([knots] * d, x))
     terms = om.selectterms(numb)
-    logpr = lib.logpr_gauss_multi(om, terms, Y.shape[1])
-    loglik = lib.loglik_gauss_multi(om, terms, Ys, x)
+    percol = {"para_per_column": True} if para_per_column else {}
+    logpr = lib.logpr_gauss_multi(om, terms, Y.shape[1], **percol)
+    loglik = lib.loglik_gauss_multi(om, terms, Ys, x, **percol)
     logpdf = lib.lpdfvec(logpr, loglik)  # prior first, as obfit_gauss
     logpdf.domarg = True
     optinfo = dict(B=None, lr=0.2)
@@ -347,10 +350,11 @@ def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verb
 
 def obpred(obmodel, x):
     """R/fitting.R:149-155.  A model of obfit_multi gives an N x C mean and an N x C variance: the shared variance
-    scaled by each column's y_sca^2."""
+    (or, with para per column, each column's own) scaled by each column's y_sca^2."""
     obmodel["predobj"].update(np.asfortranarray(np.asarray(x, dtype=float)))
     if np.ndim(obmodel["y_sca"]):
         var = obmodel["predobj"].var()
-        return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(), var=np.outer(var, obmodel["y_sca"] ** 2))
+        var = var * obmodel["y_sca"] ** 2 if var.ndim == 2 else np.outer(var, obmodel["y_sca"] ** 2)
+        return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(), var=var)
     return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(),
                 var=obmodel["y_sca"] ** 2 * obmodel["predobj"].var())

@@ -8,7 +8,13 @@ Prints one JSON line per C in {8, 64}:
   bfgs_eval_ms                     one BFGS objective evaluation: updatehyp -> updateom -> optcg (fitting.lpdfwrapper)
   separate_*                       the C single-response fits one after another: total with object construction,
                                    and the optcg of each new object
-The GPU name and power limit are read in the same run."""
+The GPU name and power limit are read in the same run.
+
+--para-per-column compares the shared form with the per-column one (each column its own noise scale and coefficient
+scale) instead: for each C, both objects are built once and measured alternately, three rounds each, so that both see
+the same clocks; one JSON line per C with, per form, every round's ms_per_iter, launches_per_iter and bfgs_eval_ms (no
+separate fits)."""
+import argparse
 import json
 import subprocess
 import sys
@@ -53,13 +59,52 @@ def timed(lib, f):
     return (time.perf_counter() - t0) * 1e3, r
 
 
+def percol_main(lib, name, power, om, terms, x, N, K):
+    for C in (8, 64):
+        Y = responses(x, C)
+        vecs = {}
+        for form, pc in (("shared", False), ("per_column", True)):
+            vec = lib.lpdfvec(lib.logpr_gauss_multi(om, terms, C, para_per_column=pc),
+                              lib.loglik_gauss_multi(om, terms, Y, x, para_per_column=pc))
+            vec.domarg = True
+            vec.optcg(0.001, 100)  # warm: module compilation, programs, buffers
+            vecs[form] = (vec, vec.coeff.copy(), dict(hyp=np.array(om.gethyp()), para=np.array(vec.para)))
+        rounds = {f: dict(ms_per_iter=[], launches_per_iter=[], bfgs_eval_ms=[]) for f in vecs}
+        for _ in range(3):
+            for form, (vec, coeff, parlist) in vecs.items():
+                per = []
+                for ep in (2, 6):
+                    vec.set_coeff(np.zeros(K * C))
+                    n0 = lib.launch_count()
+                    ms, _ = timed(lib, lambda: vec.optcg(-1.0, ep))
+                    per.append((ms, lib.launch_count() - n0))
+                rounds[form]["ms_per_iter"].append(round((per[1][0] - per[0][0]) / 4, 3))
+                rounds[form]["launches_per_iter"].append((per[1][1] - per[0][1]) / 4)
+                vec.set_coeff(coeff)
+                ms, _ = timed(lib, lambda: fitting.lpdfwrapper(parlist, om, vec))
+                rounds[form]["bfgs_eval_ms"].append(round(ms, 2))
+        out = {"workload": f"multi-response optcg on the C3 model, N={N} K={K} C={C}, shared vs per-column para",
+               "gpu": name, "power_limit": power}
+        for form, r in rounds.items():
+            out[form] = dict(r, cg_iters_per_column=vecs[form][0].cg_iters_per_column.tolist(),
+                             ms_per_iter_median=float(np.median(r["ms_per_iter"])),
+                             bfgs_eval_ms_median=float(np.median(r["bfgs_eval_ms"])))
+        print(json.dumps(out), flush=True)
+        del vecs
+
+
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--para-per-column", action="store_true", help="shared against per-column para, alternately")
+    args = ap.parse_args()
     lib = obp.lib(0)
     lib.set_option("spec", 1)
     name, power = gpu_info()
     om, terms = bench.setup_model(lib)
     N, K = bench.N_TOTAL, terms.shape[0]
     x = bench.synth_rows(0, N, bench.D)
+    if args.para_per_column:
+        return percol_main(lib, name, power, om, terms, x, N, K)
     for C in (8, 64):
         Y = responses(x, C)
         lk = lib.loglik_gauss_multi(om, terms, Y, x)
