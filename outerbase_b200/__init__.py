@@ -21,6 +21,7 @@ LIBPATH = LIBDIR / "libouterbase_b200.so"
 HEADER = REPO / "include" / "outerbase_b200.h"
 MULTI_HEADER = REPO / "include" / "outerbase_b200_multi.h"  # the multi-response extension
 PERCOL_HEADER = REPO / "include" / "outerbase_b200_multi_percol.h"  # its per-column para variants
+MULTI_GDA_HEADER = REPO / "include" / "outerbase_b200_multi_gda.h"  # multi-response loglik_gda (two-stage fits)
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -34,7 +35,7 @@ def _stale() -> bool:
     if not LIBPATH.exists():
         return True
     t = LIBPATH.stat().st_mtime
-    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER]
+    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

@@ -223,13 +223,16 @@ class Library:
     def logpr_gauss_multi(self, om, terms, ncol, para_per_column=False):
         return logpr_gauss_multi(self, om, terms, ncol, para_per_column)
 
+    def loglik_gda_multi(self, om, terms, Y, x):
+        return loglik_gda_multi(self, om, terms, Y, x)
+
     def lpdfvec(self, a, b):
         if isinstance(a, _multi) or isinstance(b, _multi):
             return lpdfvec_multi(self, a, b)
         return lpdfvec(self, a, b)
 
     def predictor(self, loglik):
-        if isinstance(loglik, loglik_gauss_multi):
+        if isinstance(loglik, (loglik_gauss_multi, loglik_gda_multi)):
             return predictor_multi(self, loglik)
         return predictor(self, loglik)
 
@@ -837,6 +840,25 @@ class logpr_gauss_multi(_multi, lpdf):
             lib.call("logpr_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.byref(self._h))
 
 
+class loglik_gda_multi(_multi, lpdf):
+    """loglik_gda on each column of Y (N x C), all columns on one basis with one per-row noise scale
+    (include/outerbase_b200_multi_gda.h): the stage-1 likelihood of a two-stage multi-response fit."""
+
+    def __init__(self, lib, om, terms, Y, x):
+        super().__init__(lib)
+        self._om = om
+        t, Y, x = _terms(terms), _f64(Y), _f64(x)
+        if Y.ndim != 2:
+            raise ValueError("Y must be N x C")
+        if x.shape[0] != Y.shape[0]:
+            raise ValueError("x and Y dims do not align")
+        lib.call("loglik_gda_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _p(Y), _u(Y.shape[1]), _p(x),
+                 _u(Y.shape[0]), C.byref(self._h))
+
+    yhat = property(lambda s: s._get("yhat").reshape((-1, s.ncol), order="F"))
+    dodiag = property(fset=lambda s, v: s._flag("dodiag", v))
+
+
 class lpdfvec_multi(_multi, lpdfvec):
     """lpdfvec of two multi-response children; optcg runs one independent CG per column."""
     cg_iters_per_column = property(lambda s: s._get("cg_iters").astype(int))
@@ -870,8 +892,9 @@ class predictor(_Handle):
 
 
 class predictor_multi(predictor):
-    """predictor(loglik_gauss_multi): mean N x C; var is one N-vector shared by all columns, or N x C when the
-    likelihood has a noise scale per column or was fitted under a prior with a coefficient scale per column."""
+    """predictor(loglik_gauss_multi or loglik_gda_multi): mean N x C; var is one N-vector shared by all columns, or
+    N x C when the likelihood has a noise scale per column or was fitted under a prior with a coefficient scale per
+    column."""
 
     def __init__(self, lib, loglik):
         super().__init__(lib, loglik)

@@ -6,6 +6,7 @@
 #include "../../include/outerbase_b200.h"
 #include "../../include/outerbase_b200_multi.h"
 #include "../../include/outerbase_b200_multi_percol.h"
+#include "../../include/outerbase_b200_multi_gda.h"
 
 #include "ob_engine.hpp"
 
@@ -480,6 +481,17 @@ int ob_loglik_gauss_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* t
                                  const double* x, uint64_t N, ob_lpdf** out) {
   return ob_loglik_gauss_multi_create_ex(ctx, om, terms, K, Y, C, x, N, 0, out);
 }
+int ob_loglik_gda_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* Y, uint64_t C,
+                               const double* x, uint64_t N, ob_lpdf** out) {
+  OB_TRY
+  need(ctx, "ctx"); need(om, "om");
+  if (C == 0) throw std::invalid_argument("ncol must be at least 1");
+  auto* h = new ob_lpdf();
+  h->ctx = ctx;
+  try { h->p.reset(new obe::LoglikGdaMulti(ctx->c, &om->om, terms, K, Y, C, x, N)); } catch (...) { delete h; throw; }
+  *out = h;
+  OB_CATCH
+}
 int ob_logpr_gauss_multi_create_ex(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, uint64_t C, int para_per_column,
                                    ob_lpdf** out) {
   OB_TRY
@@ -533,9 +545,9 @@ int ob_lpdf_set_flag(ob_lpdf* l, const char* which, int value) {
     if (!v) throw std::invalid_argument("domarg is a field of lpdfvec");
     v->domargadj = value;
   } else if (w == "dodiag") { /* R field name of loglik_gda::doda, interfaceR.cpp:748 */
-    auto* v = dynamic_cast<obe::LoglikGda*>(l->p.get());
-    if (!v) throw std::invalid_argument("dodiag is a field of loglik_gda");
-    v->doda = value; v->redostd = true;
+    if (auto* v = dynamic_cast<obe::LoglikGda*>(l->p.get())) { v->doda = value; v->redostd = true; }
+    else if (auto* m = dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) { m->doda = value; m->redostd = true; }
+    else throw std::invalid_argument("dodiag is a field of loglik_gda / loglik_gda_multi");
   } else throw std::invalid_argument("unknown flag " + w);
   OB_CATCH
 }
@@ -560,14 +572,15 @@ int ob_lpdf_get(ob_lpdf* l, const char* which, double* out, uint64_t* n) {
     else v = {double(l->p->cg_iters)};
   } else if (w == "ncol") v = {double(l->p->ncol())};
   else if (w == "predvar_ncol") {
-    auto* g = dynamic_cast<obe::LoglikGaussBase*>(l->p.get());
-    if (!g) throw std::invalid_argument("predvar_ncol is a field of loglik_gauss / loglik_gauss_multi");
-    v = {double(g->predvar_ncol())};
+    if (auto* g = dynamic_cast<obe::LoglikGaussBase*>(l->p.get())) v = {double(g->predvar_ncol())};
+    else if (dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) v = {1.0};
+    else throw std::invalid_argument("predvar_ncol is a field of loglik_gauss / loglik_gauss_multi / loglik_gda_multi");
   }
   else if (w == "yhat") {
     if (auto* g = dynamic_cast<obe::LoglikGauss*>(l->p.get())) v = g->get_yhat();
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(l->p.get())) v = g2->yhat;
-    else throw std::invalid_argument("yhat is a field of loglik_gauss / loglik_gda");
+    else if (auto* g3 = dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) v = g3->get_yhat();
+    else throw std::invalid_argument("yhat is a field of loglik_gauss / loglik_gda / loglik_gda_multi");
   } else if (w == "coeffsd") {
     auto* g = dynamic_cast<obe::LogprGauss*>(l->p.get());
     if (!g) throw std::invalid_argument("coeffsd is a field of logpr_gauss");
@@ -586,6 +599,7 @@ int ob_predictor_create(ob_lpdf* loglik, ob_predictor** out) {
     if (auto* g3 = dynamic_cast<obe::LoglikStd*>(loglik->p.get())) h->p.reset(new obe::PredrStd(*g3)); /* before its base class */
     else if (auto* g = dynamic_cast<obe::LoglikGaussBase*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*g));
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(loglik->p.get())) h->p.reset(new obe::PredGda(*g2));
+    else if (auto* g4 = dynamic_cast<obe::LoglikGdaMulti*>(loglik->p.get())) h->p.reset(new obe::PredGda(*g4));
     else throw std::invalid_argument("cannot produce a predictor from this obj.");
   } catch (...) { delete h; throw; }
   *out = h;

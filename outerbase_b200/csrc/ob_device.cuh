@@ -303,14 +303,21 @@ struct CgParams {
   const double* sca_col = nullptr;    /* batched, per-column coefficient scale: C entries replacing sca */
   const double* obssd_col = nullptr;  /* batched, per-column noise sd: C entries replacing obssd */
   const double* vma_col = nullptr;    /* batched, per-column marginal adjustment: C entries replacing val_margadj */
+  /* loglik_gda_multi: the likelihood value is -0.5 ssq - sumlogsd (sumlogsd = sum_i log obssd_i, shared by the columns)
+   * instead of -0.5 ssq - nglobal log obssd */
+  int use_sumlogsd = 0;
+  double sumlogsd = 0;
 };
 enum { CG_NUM = 0, CG_DENOM, CG_ALPHA, CG_BETA, CG_VAL, CG_VALO, CG_VALDIFF, CG_STOP, CG_VAL_LIK, CG_VAL_PR, CG_ITER, CG_NSCAL = 16 };
 void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol = 1);
 /* after mm_mat_dev on C columns (leading dimension ld): update: w = -((yhat - y)/sd)/sd, ssq_out[c] = sum of
  * ((yhat - y)/sd)^2 over column c (fixed order); hessmult: w = (yhat/sd)/sd.  Pad rows of w are zero; yhat may alias w.
- * sd_cols (device, C entries), when set, gives column c the sd sd_cols[c] instead of sd. */
+ * sd_cols (device, C entries), when set, gives column c the sd sd_cols[c] instead of sd; sd_rows (device, ld entries),
+ * when set, gives row i of every column the sd sd_rows[i] (loglik_gda's per-row noise) instead of either. */
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
-                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols = nullptr);
+                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols = nullptr, const double* sd_rows = nullptr);
+/* loglik_gda's obssd on the device: obssd[i] = sqrt(v0 + v1 (1 - phi2varc[i])) (phi2varc null: sqrt(v0)), pad rows 1 */
+void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

@@ -9,6 +9,8 @@
  *   LoglikStd         loglik_std        src/lpdfs/loglik_std.cpp:41-203
  *   LoglikGda         loglik_gda        src/lpdfs/loglik_gda.cpp:47-239
  *   LogprGaussMulti   logpr_gauss on each of C columns
+ *   LoglikGdaMulti    loglik_gda on each of C columns (obfit_multi's stage 1)
+ *   DevLik            what the device CG needs of a likelihood: LoglikGaussBase and LoglikGdaMulti derive from it
  *   LpdfVec           lpdfvec           src/fit.cpp:174-267,310-428,557-607 (diagonal branch), 269-299 (full branch)
  *   Pred              the predictors PredGauss (pred_gauss, loglik_gauss.cpp:196-227), PredrStd, PredGda
  *
@@ -957,36 +959,24 @@ inline std::vector<double> tile_cols(const std::vector<double>& v, u64 K, u64 C)
   return o;
 }
 
-/* loglik_gauss (loglik_gauss.cpp:41-179) on C responses observed at the same rows (C = 1: loglik_gauss itself), all but
- * the products.  Every column is the single-response model on its own response; the columns share the basis, the terms
- * table, the hyper-parameters and the para entry.  val, gradhyp and gradpara are the sums over the columns (in column
- * order) of what the single-response object returns at that column, grad is K x C, and the Hessian diagonals, which do
- * not depend on the response, are computed once and repeated C times.  With C = 1 every formula is the reference's
- * own.  The subclasses are the two paths of the products: LoglikGauss (one vector, fused epilogues) and
- * LoglikGaussMulti (matrix products over the columns).
- * percol (para per column, multi-response only): npara = C, para[c] is column c's noise log-sd with loglik_gauss's
- * default on that column; gradpara[c] is column c's own, and the Hessian diagonals are the one K-vector of squared
- * column sums scaled by each column's exp(-2 para[c]) (diaghessgradpara: (K C) x C, block-diagonal). */
-struct LoglikGaussBase : Lpdf {
+/* A likelihood on C responses observed at the same rows that LpdfVec::optcg_device can drive: y, yhat and w are ld x C
+ * on the device (pad rows zero), the update and the Hessian product run on the device (update_dev / hessmult_dev:
+ * coefficients in, the likelihood part of grad or of the Hessian product in red[0 .. K C), nothing crosses to the host),
+ * val_col(c) is column c's value of the last host update, and cg_params fills the likelihood's fields of the CG stage
+ * kernel (its noise scale, and the device array of per-column sums of squared residuals for C columns). */
+struct DevLik : Lpdf {
   Ctx& ctx;
   const OuterMod* om;
   OuterBase ob;
   std::vector<double> x_host; /* kept for predictor(loglik), loglik_gauss.cpp:198 */
   u64 N = 0, K = 0, C = 1;
-  double Nglobal = 0;
-  double obssd = 1;
-  bool percol = false;
-  std::vector<double> obssd_cols; /* C: column c's noise sd, exp(para[c]) (percol) or obssd */
-  /* y, yhat, w: ld x C (pad rows zero) */
-  DevBuf<double> y, yhat, w, kbuf, red, ones;
+  DevBuf<double> y, yhat, w, kbuf, red;
   std::vector<double> ssq_host; /* per-column sums of squared standardised residuals of the last update (all ranks) */
-  std::vector<double> sqcs;      /* the last sqcolsums(); empty after updateom / updateterms */
 
-  LoglikGaussBase(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
-                  bool percol_ = false)
-      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_), percol(percol_) {
+  DevLik(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
+      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_) {
     if (C == 0) throw std::invalid_argument("ncol must be at least 1");
-    d = om->d; npara = 1;
+    d = om->d;
     terms.assign(t, t + K * d);
     nterms = K * C;
     x_host.assign(xh, xh + N * d);
@@ -997,6 +987,48 @@ struct LoglikGaussBase : Lpdf {
       if (N) OB_CUDA(cudaMemcpyAsync(y.p + j * ld, yh + j * N, N * sizeof(double), cudaMemcpyHostToDevice, ctx.stream));
     yhat.ensure(ld * C); w.ensure(ld * C);
     ctx.sync();
+  }
+  static double arma_var(const double* x, u64 n) {
+    if (n < 2) return 0.0;
+    const double mean = obh::sum2(x, n) / double(n);
+    double a2 = 0, a3 = 0;
+    u64 i, j;
+    for (i = 0, j = 1; j < n; i += 2, j += 2) { const double ti = mean - x[i], tj = mean - x[j]; a2 += ti * ti + tj * tj; a3 += ti + tj; }
+    if (i < n) { const double ti = mean - x[i]; a2 += ti * ti; a3 += ti; }
+    return (a2 - a3 * a3 / double(n)) / double(n - 1);
+  }
+  u64 ncol() const override { return C; }
+  u64 nhyp() const override { return ob.H; }
+  u64 nrow() const override { return N; }
+  void setnthreads(int k) override { ob.nthreads = k; }
+  virtual void update_dev(const double* coeff_dev) = 0;
+  virtual void hessmult_dev(const double* g_dev) = 0;
+  virtual double val_col(u64 c) const = 0;
+  virtual void cg_params(obd::CgParams& c) const = 0;
+};
+
+/* loglik_gauss (loglik_gauss.cpp:41-179) on C responses observed at the same rows (C = 1: loglik_gauss itself), all but
+ * the products.  Every column is the single-response model on its own response; the columns share the basis, the terms
+ * table, the hyper-parameters and the para entry.  val, gradhyp and gradpara are the sums over the columns (in column
+ * order) of what the single-response object returns at that column, grad is K x C, and the Hessian diagonals, which do
+ * not depend on the response, are computed once and repeated C times.  With C = 1 every formula is the reference's
+ * own.  The subclasses are the two paths of the products: LoglikGauss (one vector, fused epilogues) and
+ * LoglikGaussMulti (matrix products over the columns).
+ * percol (para per column, multi-response only): npara = C, para[c] is column c's noise log-sd with loglik_gauss's
+ * default on that column; gradpara[c] is column c's own, and the Hessian diagonals are the one K-vector of squared
+ * column sums scaled by each column's exp(-2 para[c]) (diaghessgradpara: (K C) x C, block-diagonal). */
+struct LoglikGaussBase : DevLik {
+  double Nglobal = 0;
+  double obssd = 1;
+  bool percol = false;
+  std::vector<double> obssd_cols; /* C: column c's noise sd, exp(para[c]) (percol) or obssd */
+  DevBuf<double> ones;
+  std::vector<double> sqcs;      /* the last sqcolsums(); empty after updateom / updateterms */
+
+  LoglikGaussBase(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
+                  bool percol_ = false)
+      : DevLik(c, om_, t, K_, yh, C_, xh, N_), percol(percol_) {
+    npara = 1;
     /* para0 = log(0.01 * mean over the columns of var(y[:,c])), loglik_gauss.cpp:48 (Armadillo two-pass var); over ALL
      * ranks' rows */
     std::vector<double> var(C);
@@ -1043,19 +1075,6 @@ struct LoglikGaussBase : Lpdf {
     OB_CUDA(cudaMemcpyAsync(v, red.p, n * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
     ctx.sync();
   }
-  static double arma_var(const double* x, u64 n) {
-    if (n < 2) return 0.0;
-    const double mean = obh::sum2(x, n) / double(n);
-    double a2 = 0, a3 = 0;
-    u64 i, j;
-    for (i = 0, j = 1; j < n; i += 2, j += 2) { const double ti = mean - x[i], tj = mean - x[j]; a2 += ti * ti + tj * tj; a3 += ti + tj; }
-    if (i < n) { const double ti = mean - x[i]; a2 += ti * ti; a3 += ti; }
-    return (a2 - a3 * a3 / double(n)) / double(n - 1);
-  }
-  u64 ncol() const override { return C; }
-  u64 nhyp() const override { return ob.H; }
-  u64 nrow() const override { return N; }
-  void setnthreads(int k) override { ob.nthreads = k; }
   void updateom() override { ob.build(); sqcs.clear(); }
   bool para_per_column() const override { return percol; }
   void updatepara(const double* p, u64 n) override {
@@ -1066,7 +1085,8 @@ struct LoglikGaussBase : Lpdf {
   void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; sqcs.clear(); }
   /* columns of the predictive variance of a predictor made from this likelihood now (PredGauss) */
   u64 predvar_ncol() const { return multi() && (percol || totdiaghess_percol) ? C : 1; }
-  double val_col(u64 c) const { return -0.5 * ssq_host[c] - Nglobal * std::log(obssd_cols[c]); }
+  double val_col(u64 c) const override { return -0.5 * ssq_host[c] - Nglobal * std::log(obssd_cols[c]); }
+  void cg_params(obd::CgParams& c) const override { c.obssd = obssd; c.nglobal = Nglobal; }
   /* val and gradpara of update() from ssq_host, loglik_gauss.cpp:121-129 */
   void set_val_gradpara() {
     if (compute_val) { val = 0; for (u64 c = 0; c < C; ++c) val += val_col(c); }
@@ -1076,11 +1096,8 @@ struct LoglikGaussBase : Lpdf {
     }
   }
 
-  /* ---- device forms for the HBM-resident CG (LpdfVec::optcg_device), stream ordered: coefficients in, the likelihood
-   * part of grad (update_dev) or of the Hessian product (hessmult_dev) in red[0 .. K C), summed over ranks; nothing
-   * crosses to the host.  update_dev also leaves each column's sum of squared standardised residuals on the device. */
-  virtual void update_dev(const double* coeff_dev) = 0;
-  virtual void hessmult_dev(const double* g_dev) = 0;
+  /* device forms (DevLik), stream ordered, summed over ranks; update_dev also leaves each column's sum of squared
+   * standardised residuals on the device */
   std::vector<double> hessmult(const std::vector<double>& g) override { /* :137-145 */
     if (g.size() != K * C) throw std::range_error("g must have K x ncol entries");
     kbuf.upload(g, ctx.stream);
@@ -1302,14 +1319,74 @@ struct LoglikStd : LoglikGauss {
   }
 };
 
-struct LoglikGda : Lpdf {
+/* loglik_gda's per-row noise sd and the host work that depends on it only, not on the response (shared by LoglikGda and
+ * LoglikGdaMulti): the sd's derivatives (loglik_gda.cpp:226-235) and the Hessian diagonals (:172-211), all K- or
+ * N-sized on the host around the GPU products, in the reference's operation order */
+struct GdaSd {
+  std::vector<double> obssd, obssd_gradhyp, obssd_gradpara;
+  /* from obssd and rterms = residvar (read only with doda) */
+  void sd_grads(OuterBase& ob, const u64* terms, u64 K, const std::vector<double>& para, bool doda, const std::vector<double>& rterms) {
+    const u64 N = obssd.size(), H = ob.H;
+    if (doda) {
+      obssd_gradhyp.resize(N * H);
+      ob.residvar_gradhyp(terms, K, obssd_gradhyp.data());
+      for (u64 h = 0; h < H; ++h)
+        for (u64 i = 0; i < N; ++i) obssd_gradhyp[i + h * N] *= (std::exp(2 * para[1]) * 0.5) / obssd[i];
+    }
+    obssd_gradpara.assign(N * 2, 0.0);
+    for (u64 i = 0; i < N; ++i) {
+      obssd_gradpara[i] = std::exp(2 * para[0]) / obssd[i];
+      obssd_gradpara[i + N] = doda ? std::exp(2 * para[1]) * rterms[i] / obssd[i] : 0.0;
+    }
+  }
+  std::vector<double> gda_diaghess(OuterBase& ob, const u64* terms, u64 K) const { /* :172-175 */
+    const u64 N = obssd.size();
+    std::vector<double> t(N), o(K);
+    for (u64 i = 0; i < N; ++i) t[i] = 1 / (obssd[i] * obssd[i]);
+    ob.tmm(1, terms, K, t.data(), o.data());
+    return o;
+  }
+  std::vector<double> gda_diaghessgradhyp(OuterBase& ob, const u64* terms, u64 K, bool doda) const { /* :182-196 */
+    const u64 N = obssd.size(), H = ob.H;
+    std::vector<double> temp(N), lh(K * H);
+    for (u64 i = 0; i < N; ++i) temp[i] = 1 / (obssd[i] * obssd[i]);
+    ob.tmm_gradhyp(1, terms, K, temp.data(), nullptr, lh.data());
+    for (u64 i = 0; i < N; ++i) temp[i] *= -2 / obssd[i];
+    if (doda) {
+      std::vector<double> t2(obssd_gradhyp), add(K * H);
+      for (u64 h = 0; h < H; ++h)
+        for (u64 i = 0; i < N; ++i) t2[i + h * N] *= temp[i];
+      ob.tmm_mat(1, terms, K, t2.data(), H, add.data());
+      for (u64 i = 0; i < K * H; ++i) lh[i] += add[i];
+    }
+    return lh;
+  }
+  std::vector<double> gda_diaghessgradpara(OuterBase& ob, const u64* terms, u64 K) const { /* :203-211 */
+    const u64 N = obssd.size();
+    std::vector<double> t2(obssd_gradpara), o(K * 2);
+    for (u64 q = 0; q < 2; ++q)
+      for (u64 i = 0; i < N; ++i) t2[i + q * N] *= (1 / (obssd[i] * obssd[i])) * (-2 / obssd[i]);
+    ob.tmm_mat(1, terms, K, t2.data(), 2, o.data());
+    return o;
+  }
+  /* Armadillo's two-accumulator dot */
+  static double dot2(const double* a, const double* b, u64 n) {
+    double s1 = 0, s2 = 0;
+    u64 j;
+    for (j = 1; j < n; j += 2) { s1 += a[j - 1] * b[j - 1]; s2 += a[j] * b[j]; }
+    if ((j - 1) < n) s1 += a[j - 1] * b[j - 1];
+    return s1 + s2;
+  }
+};
+
+struct LoglikGda : Lpdf, GdaSd {
   Ctx& ctx;
   const OuterMod* om;
   OuterBase ob;
   std::vector<double> x_host, y;
   u64 N = 0;
   bool doda = true, redostd = true;
-  std::vector<double> yhat, obssd, yhatge, obssd_gradhyp, obssd_gradpara, residtemp, residtemp2;
+  std::vector<double> yhat, yhatge, residtemp, residtemp2;
 
   LoglikGda(Ctx& c, const OuterMod* om_, const u64* t, u64 K, const double* yh, const double* xh, u64 N_)
       : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K), N(N_) {
@@ -1319,7 +1396,7 @@ struct LoglikGda : Lpdf {
     nterms = K;
     x_host.assign(xh, xh + N * d);
     y.assign(yh, yh + N);
-    para0 = {0.5 * std::log(0.01 * LoglikGauss::arma_var(yh, N)), 0.0};
+    para0 = {0.5 * std::log(0.01 * DevLik::arma_var(yh, N)), 0.0};
     paravar = {4, 4};
     para = para0;
     buildstd();
@@ -1328,16 +1405,9 @@ struct LoglikGda : Lpdf {
   void updateom() override { ob.build(); if (doda) redostd = true; }
   void updatepara(const double* p, u64 n) override { para.assign(p, p + n); redostd = true; }
   void updateterms(const u64* t, u64 K) override { terms.assign(t, t + K * d); nterms = K; if (doda) redostd = true; }
-  static double dot2(const double* a, const double* b, u64 n) { /* Armadillo's two-accumulator dot */
-    double s1 = 0, s2 = 0;
-    u64 j;
-    for (j = 1; j < n; j += 2) { s1 += a[j - 1] * b[j - 1]; s2 += a[j] * b[j]; }
-    if ((j - 1) < n) s1 += a[j - 1] * b[j - 1];
-    return s1 + s2;
-  }
   void buildstd() { /* :217-236 */
     if (redostd) {
-      const u64 H = ob.H, K = nterms;
+      const u64 K = nterms;
       std::vector<double> rterms(N);
       ob.residvar(terms.data(), K, rterms.data());
       obssd.resize(N);
@@ -1346,17 +1416,7 @@ struct LoglikGda : Lpdf {
         if (doda) v += std::exp(2 * para[1]) * rterms[i];
         obssd[i] = std::sqrt(v);
       }
-      if (doda) {
-        obssd_gradhyp.resize(N * H);
-        ob.residvar_gradhyp(terms.data(), K, obssd_gradhyp.data());
-        for (u64 h = 0; h < H; ++h)
-          for (u64 i = 0; i < N; ++i) obssd_gradhyp[i + h * N] *= (std::exp(2 * para[1]) * 0.5) / obssd[i];
-      }
-      obssd_gradpara.assign(N * 2, 0.0);
-      for (u64 i = 0; i < N; ++i) {
-        obssd_gradpara[i] = std::exp(2 * para[0]) / obssd[i];
-        obssd_gradpara[i + N] = doda ? std::exp(2 * para[1]) * rterms[i] / obssd[i] : 0.0;
-      }
+      sd_grads(ob, terms.data(), K, para, doda, rterms);
     }
     redostd = false;
   }
@@ -1407,35 +1467,9 @@ struct LoglikGda : Lpdf {
     ob.tmm(0, terms.data(), K, yt.data(), o.data());
     return o;
   }
-  std::vector<double> diaghess() override { /* :172-175 */
-    std::vector<double> t(N), o(nterms);
-    for (u64 i = 0; i < N; ++i) t[i] = 1 / (obssd[i] * obssd[i]);
-    ob.tmm(1, terms.data(), nterms, t.data(), o.data());
-    return o;
-  }
-  std::vector<double> diaghessgradhyp() override { /* :182-196 */
-    const u64 K = nterms, H = ob.H;
-    std::vector<double> temp(N), lh(K * H);
-    for (u64 i = 0; i < N; ++i) temp[i] = 1 / (obssd[i] * obssd[i]);
-    ob.tmm_gradhyp(1, terms.data(), K, temp.data(), nullptr, lh.data());
-    for (u64 i = 0; i < N; ++i) temp[i] *= -2 / obssd[i];
-    if (doda) {
-      std::vector<double> t2(obssd_gradhyp), add(K * H);
-      for (u64 h = 0; h < H; ++h)
-        for (u64 i = 0; i < N; ++i) t2[i + h * N] *= temp[i];
-      ob.tmm_mat(1, terms.data(), K, t2.data(), H, add.data());
-      for (u64 i = 0; i < K * H; ++i) lh[i] += add[i];
-    }
-    return lh;
-  }
-  std::vector<double> diaghessgradpara() override { /* :203-211 */
-    const u64 K = nterms;
-    std::vector<double> t2(obssd_gradpara), o(K * 2);
-    for (u64 q = 0; q < 2; ++q)
-      for (u64 i = 0; i < N; ++i) t2[i + q * N] *= (1 / (obssd[i] * obssd[i])) * (-2 / obssd[i]);
-    ob.tmm_mat(1, terms.data(), K, t2.data(), 2, o.data());
-    return o;
-  }
+  std::vector<double> diaghess() override { return gda_diaghess(ob, terms.data(), nterms); }
+  std::vector<double> diaghessgradhyp() override { return gda_diaghessgradhyp(ob, terms.data(), nterms, doda); }
+  std::vector<double> diaghessgradpara() override { return gda_diaghessgradpara(ob, terms.data(), nterms); }
   u64 nhyp() const override { return ob.H; }
   u64 nrow() const override { return N; }
 };
@@ -1571,6 +1605,7 @@ struct LoglikGaussMulti : LoglikGaussBase {
     ssq.ensure(C);
     upload_sds();
   }
+  void cg_params(obd::CgParams& c) const override { LoglikGaussBase::cg_params(c); c.ssq = ssq.p; c.obssd_col = sd_cols_dev(); }
   bool multi() const override { return true; }
   void upload_sds() {
     if (!percol) return;
@@ -1627,6 +1662,154 @@ struct LoglikGaussMulti : LoglikGaussBase {
   void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi)"); }
 };
 
+/* loglik_gda (loglik_gda.cpp:47-239) on C responses observed at the same rows: column c is loglik_gda on Y[:,c].  The
+ * columns share the basis, the terms table, the hyper-parameters, dodiag and both para entries, so the per-row noise
+ * sd obssd is one N-vector; it is formed on the device (gda_obssd_kernel) from the squared product residvar runs, and
+ * rebuilt where LoglikGda sets redostd.  val, gradhyp and gradpara are the sums over the columns (in column order) of
+ * loglik_gda's, grad is K x C, hessmult is block-diagonal, and the Hessian diagonals, which do not depend on the
+ * response, are loglik_gda's computed once and repeated C times.  The products are the matrix path of LoglikGaussMulti:
+ * mm_mat_dev | resid_multi with the per-row sd | tmm_mat_dev; the sd's hyper-gradient bookkeeping stays on the host as in
+ * LoglikGda and runs once per update with gradients.  Para is never per column; one rank only (obfit's stage-1
+ * subsample). */
+struct LoglikGdaMulti : DevLik, GdaSd {
+  bool doda = true, redostd = true;
+  double sumlogsd = 0; /* sum_i log obssd_i in obh::sum2 order: the likelihood's constant, the same for every column */
+  std::vector<double> y_host;
+  DevBuf<double> sd, phi2, ssq, partial, gh;
+
+  LoglikGdaMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
+      : DevLik(c, om_, t, K_, yh, C_, xh, N_) {
+    if (ctx.nranks > 1) throw std::logic_error("loglik_gda_multi is the single-rank subsample model of obfit stage 1");
+    npara = 2;
+    y_host.assign(yh, yh + N * C);
+    double vs = 0; /* para0[0] = 0.5 log(0.01 mean_c var(Y[:,c])), loglik_gda.cpp:59 on the mean variance */
+    for (u64 j = 0; j < C; ++j) vs += arma_var(yh + j * N, N);
+    para0 = {0.5 * std::log(0.01 * (vs / double(C))), 0.0};
+    paravar = {4, 4};
+    para = para0;
+    ssq.ensure(C);
+    buildstd();
+  }
+  bool multi() const override { return true; }
+  void updateom() override { ob.build(); if (doda) redostd = true; }
+  void updatepara(const double* p, u64 n) override {
+    if (n != 2) throw std::range_error("para must have two entries");
+    para.assign(p, p + n);
+    redostd = true;
+  }
+  void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; if (doda) redostd = true; }
+  void buildstd() { /* loglik_gda.cpp:217-236 */
+    if (!redostd) return;
+    const u64 ld = ob.ld;
+    std::vector<double> rterms;
+    sd.ensure(std::max<u64>(ld, 1));
+    if (doda) { /* residvar = 1 - Phi^2 varc */
+      std::vector<double> varc(K);
+      om->getvar(terms.data(), K, varc.data());
+      kbuf.upload(varc, ctx.stream);
+      phi2.ensure(std::max<u64>(ld, 1));
+      ob.mm_dev(terms.data(), K, 1, kbuf.p, phi2.p);
+      rterms.resize(N);
+      ob.d2h(rterms.data(), phi2.p, N);
+      for (u64 i = 0; i < N; ++i) rterms[i] = 1 - rterms[i];
+    }
+    obd::launch_gda_obssd(ctx, doda ? phi2.p : nullptr, N, ld, std::exp(2 * para[0]), std::exp(2 * para[1]), sd.p);
+    obssd.resize(N);
+    ob.d2h(obssd.data(), sd.p, N);
+    sd_grads(ob, terms.data(), K, para, doda, rterms);
+    std::vector<double> t(N);
+    for (u64 i = 0; i < N; ++i) t[i] = std::log(obssd[i]);
+    sumlogsd = obh::sum2(t.data(), N);
+    redostd = false;
+  }
+  double val_col(u64 c) const override { return -0.5 * ssq_host[c] - sumlogsd; }
+  void cg_params(obd::CgParams& c) const override { c.ssq = ssq.p; c.use_sumlogsd = 1; c.sumlogsd = sumlogsd; }
+  /* ssq[c]: column c's sum of squared standardised residuals */
+  void update_dev(const double* coeff_dev) override {
+    ob.mm_mat_dev(terms.data(), K, 0, coeff_dev, C, yhat.p, ob.ld);
+    obd::launch_resid_multi(ctx, yhat.p, y.p, w.p, N, ob.ld, C, 1.0, true, partial, ssq.p, nullptr, sd.p);
+    red.ensure(K * C);
+    ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
+  }
+  void hessmult_dev(const double* g_dev) override { /* loglik_gda.cpp:156-164 per column; w holds Phi g until the residual pass */
+    ob.mm_mat_dev(terms.data(), K, 0, g_dev, C, w.p, ob.ld);
+    obd::launch_resid_multi(ctx, w.p, nullptr, w.p, N, ob.ld, C, 1.0, false, partial, nullptr, nullptr, sd.p);
+    red.ensure(K * C);
+    ob.tmm_mat_dev(terms.data(), K, 0, w.p, ob.ld, C, red.p);
+  }
+  void update(const std::vector<double>& cf) override { /* loglik_gda.cpp:116-149 per column */
+    if (cf.size() != K * C) throw std::range_error("coeff must have K x ncol entries");
+    coeff = cf;
+    buildstd();
+    const u64 H = ob.H, ld = ob.ld;
+    kbuf.upload(coeff, ctx.stream);
+    update_dev(kbuf.p);
+    ssq_host.resize(C);
+    ob.d2h(ssq_host.data(), ssq.p, C);
+    if (compute_val) { val = 0; for (u64 c = 0; c < C; ++c) val += val_col(c); }
+    if (!compute_grad) return;
+    grad.resize(K * C);
+    ob.d2h(grad.data(), red.p, K * C);
+    if (!compute_gradhyp && !compute_gradpara) return;
+    std::vector<double> ghr(H * C, 0.0);
+    if (compute_gradhyp && H > 0) { /* the residual term, one hyper-gradient pass per column (:136) */
+      gh.ensure(H * C);
+      OB_CUDA(cudaMemsetAsync(gh.p, 0, H * C * sizeof(double), ctx.stream));
+      for (u64 c = 0; c < C; ++c) {
+        const std::vector<double> a(coeff.begin() + c * K, coeff.begin() + (c + 1) * K);
+        ob.gradhyp_dots(terms.data(), K, a, kbuf.p + c * K, w.p + c * ld, yhat.p + c * ld, gh.p + c * H);
+      }
+      ob.d2h(ghr.data(), gh.p, H * C);
+    }
+    /* the sd's terms (:137-147): the 1 / obssd dots do not depend on the response */
+    std::vector<double> yh(N), inv(N), rt2(N), invh(H, 0.0), invp(2);
+    for (u64 i = 0; i < N; ++i) inv[i] = 1 / obssd[i];
+    if (doda) for (u64 h = 0; h < H; ++h) invh[h] = dot2(inv.data(), obssd_gradhyp.data() + h * N, N);
+    for (u64 q = 0; q < 2; ++q) invp[q] = dot2(inv.data(), obssd_gradpara.data() + q * N, N);
+    if (compute_gradhyp) gradhyp.assign(H, 0.0);
+    if (compute_gradpara) gradpara.assign(2, 0.0);
+    for (u64 c = 0; c < C; ++c) {
+      ob.d2h(yh.data(), yhat.p + c * ld, N);
+      const double* yc = y_host.data() + c * N;
+      for (u64 i = 0; i < N; ++i) { const double r = (yh[i] - yc[i]) / obssd[i]; rt2[i] = r * r; rt2[i] /= obssd[i]; }
+      if (compute_gradhyp)
+        for (u64 h = 0; h < H; ++h) {
+          double g = ghr[c * H + h];
+          if (doda) { g += dot2(rt2.data(), obssd_gradhyp.data() + h * N, N); g -= invh[h]; }
+          gradhyp[h] += g;
+        }
+      if (compute_gradpara)
+        for (u64 q = 0; q < 2; ++q) {
+          double g = dot2(rt2.data(), obssd_gradpara.data() + q * N, N);
+          g -= invp[q];
+          gradpara[q] += g;
+        }
+    }
+  }
+  std::vector<double> hessmult(const std::vector<double>& g) override {
+    if (g.size() != K * C) throw std::range_error("g must have K x ncol entries");
+    kbuf.upload(g, ctx.stream);
+    hessmult_dev(kbuf.p);
+    std::vector<double> o(K * C);
+    ob.d2h(o.data(), red.p, K * C);
+    return o;
+  }
+  /* N x C, the last update's */
+  std::vector<double> get_yhat() {
+    std::vector<double> o(N * C);
+    for (u64 c = 0; c < C; ++c) ob.d2h(o.data() + c * N, yhat.p + c * ob.ld, N);
+    return o;
+  }
+  std::vector<double> diaghess() override { return tile_cols(gda_diaghess(ob, terms.data(), K), K, C); }
+  std::vector<double> diaghessgradhyp() override { return tile_cols(gda_diaghessgradhyp(ob, terms.data(), K, doda), K, C); }
+  std::vector<double> diaghessgradpara() override { return tile_cols(gda_diaghessgradpara(ob, terms.data(), K), K, C); }
+  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
+  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
+  void optnewton() override { refuse_multi("optnewton"); }
+  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gda_multi)"); }
+};
+
 struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   double val_margadj = 0;
   std::vector<double> gradhyp_margadj, gradpara_margadj;
@@ -1641,6 +1824,8 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   LpdfVec(Lpdf* a, Lpdf* b) {
     if (a->multi() != b->multi() || a->ncol() != b->ncol())
       throw std::invalid_argument("lpdfvec: children must both be single-response, or multi-response with the same number of columns");
+    if ((dynamic_cast<LoglikGdaMulti*>(a) && b->para_per_column()) || (dynamic_cast<LoglikGdaMulti*>(b) && a->para_per_column()))
+      throw std::invalid_argument("lpdfvec: loglik_gda_multi pairs with a shared-para logpr_gauss_multi only");
     kid[0] = a; kid[1] = b;
     terms = a->terms; d = a->d;
     nterms = a->nterms;
@@ -1870,7 +2055,8 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     return out;
   }
   /* lpdf::optcg (fit.cpp:37-96) with every K-vector and scalar of the loop in HBM, for lpdfvec(logpr_gauss,
-   * loglik_gauss) and lpdfvec(logpr_gauss_multi, loglik_gauss_multi) in either order.  The reference's sequence is kept
+   * loglik_gauss), lpdfvec(logpr_gauss_multi, loglik_gauss_multi) and lpdfvec(logpr_gauss_multi, loglik_gda_multi) in
+   * either order (the likelihood is a DevLik).  The reference's sequence is kept
    * operation by operation -- first update() and diaghess() through the host path (they build the cached Hessian
    * diagonal and the marginal adjustment, fit.cpp:252-267), then per iteration: CG_STEP | stop test | update |
    * CG_POST_UPDATE | hessmult, each a few launches on the library stream; the host reads one value per iteration; the
@@ -1889,14 +2075,14 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   std::vector<u64> cg_iters_cols;
   bool optcg_device(double tol, u64 maxepch) {
     const bool mult = multi();
-    auto* lk = dynamic_cast<LoglikGaussBase*>(kid[0]);
+    auto* lk = dynamic_cast<DevLik*>(kid[0]);
     const bool lik_first = lk != nullptr;
-    if (!lik_first) lk = dynamic_cast<LoglikGaussBase*>(kid[1]);
+    if (!lik_first) lk = dynamic_cast<DevLik*>(kid[1]);
     Lpdf* prior = kid[lik_first ? 1 : 0];
     auto* prm = dynamic_cast<LogprGaussMulti*>(prior);
     const LogprGauss* pr = prm ? &prm->one : dynamic_cast<LogprGauss*>(prior);
     if (!lk || !pr) {
-      if (mult) throw std::invalid_argument("optcg on multi-response objects needs lpdfvec(logpr_gauss_multi, loglik_gauss_multi)");
+      if (mult) throw std::invalid_argument("optcg on multi-response objects needs lpdfvec(logpr_gauss_multi, loglik_gauss_multi or loglik_gda_multi)");
       return false;
     }
     Ctx& ctx = lk->ctx;
@@ -1912,7 +2098,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     /* the starting value of each run: single response, the lpdfvec's own; multi-response, column c's value as the
      * single-response lpdfvec forms it (fit.cpp:352-380): children in order, then its own marginal adjustment -- the
      * diagonal's column block c is column c's single-response diagonal (with shared para, every block is block 0) */
-    const bool percol = mult && (lk->percol || prm->percol);
+    const bool percol = mult && (lk->para_per_column() || prm->percol);
     std::vector<double> vma_cols(percol ? C : 1, val_margadj);
     if (mult)
       for (u64 c = 0; c < vma_cols.size(); ++c) {
@@ -1945,9 +2131,10 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     obd::CgParams c{};
     c.K = (int)K; c.lik_first = lik_first ? 1 : 0; c.domarg = domargadj ? 1 : 0;
     c.coeff = cg_coeff.p; c.grad = cg_grad.p; c.m = cg_m.p; c.rm = cg_rm.p; c.p = cg_p.p; c.q = cg_q.p; c.sds = cg_sds.p;
-    c.sca = pr->sca; c.obssd = lk->obssd; c.nglobal = lk->Nglobal; c.val_margadj = vma; c.tol = tol; c.scal = cg_scal.p;
-    if (mult) { c.ssq = static_cast<LoglikGaussMulti*>(lk)->ssq.p; c.running = cg_running.p; }
-    if (percol) { c.sca_col = cg_sca.p; c.vma_col = cg_vma.p; c.obssd_col = static_cast<LoglikGaussMulti*>(lk)->sd_cols_dev(); }
+    c.sca = pr->sca; c.val_margadj = vma; c.tol = tol; c.scal = cg_scal.p;
+    lk->cg_params(c);
+    if (mult) c.running = cg_running.p;
+    if (percol) { c.sca_col = cg_sca.p; c.vma_col = cg_vma.p; }
     auto stage = [&](int st) { c.stage = st; c.red = lk->red.p; obd::launch_cg_stage(ctx, c, C); };
     stage(obd::CG_INIT);          /* rm = grad / m ; p = rm                       :58-60 */
     lk->hessmult_dev(cg_p.p);     /* q = hessmult(p), finished inside CG_STEP     :62 */
@@ -2098,10 +2285,13 @@ struct PredrStd : Pred { /* loglik_std.cpp:219-257 */
   }
 };
 
+/* multi-response (LoglikGdaMulti): the mean is N x C, the variance one N-vector for all columns from the first K entries
+ * of 1 / totdiaghess (its column blocks are equal) */
 struct PredGda : Pred { /* loglik_gda.cpp:249-283 */
   std::vector<double> coeffvar;
   bool doda;
   PredGda(LoglikGda& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.nterms), coeffvar(inv_totdiaghess(lk)), doda(lk.doda) {}
+  PredGda(LoglikGdaMulti& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.K, lk.C), coeffvar(inv_totdiaghess(lk)), doda(lk.doda) {}
   void var(double* out) override {
     ob->mm(1, terms.data(), K, coeffvar.data(), out);
     std::vector<double> rv(ob->N);

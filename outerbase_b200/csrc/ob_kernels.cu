@@ -524,18 +524,21 @@ __global__ void colsum_partials_kernel(const double* __restrict__ partial, int n
  * (same expressions, so a column's w equals the trie kernel's bit for bit given the same yhat and sd).  grid (nb, C);
  * rows N .. ld-1 of w are written as zero (phi_tm_spec and phi_t_spec read pad rows, they must be finite).  update:
  * partial[c * nb + b] = this CTA's sum of ((yhat - y) / sd)^2 over its rows of column c, fixed tree.  yhat may alias w.
- * sds, when set, holds one sd per column (per-column noise) and replaces the scalar sd. */
+ * sds, when set, holds one sd per column (per-column noise) and replaces the scalar sd.  rowsd, when set, holds one sd
+ * per row shared by the columns (loglik_gda's obssd) and replaces both: the same expressions as LoglikGda::update /
+ * hessmult with that row's sd. */
 constexpr int kResidThreads = 256;
 __global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double* yhat, const double* __restrict__ y, double* w, u64 N,
                                                                    u64 ld, double sd0, const double* __restrict__ sds, int update,
-                                                                   double* __restrict__ partial) {
+                                                                   double* __restrict__ partial, const double* __restrict__ rowsd = nullptr) {
   __shared__ double sm[kResidThreads];
   const u64 col = blockIdx.y, base = col * ld;
-  const double sd = sds ? sds[col] : sd0;
+  const double sdc = sds ? sds[col] : sd0;
   double s = 0.0;
   for (u64 i = (u64)blockIdx.x * kResidThreads + threadIdx.x; i < ld; i += (u64)gridDim.x * kResidThreads) {
     double wv = 0.0;
     if (i < N) {
+      const double sd = rowsd ? rowsd[i] : sdc;
       const double yv = yhat[base + i];
       if (update) {
         const double rt = (yv - y[base + i]) / sd;
@@ -553,6 +556,19 @@ __global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double
     __syncthreads();
   }
   if (threadIdx.x == 0) partial[col * gridDim.x + blockIdx.x] = sm[0];
+}
+
+/* loglik_gda's per-row noise sd (LoglikGda::buildstd): v = v0, plus v1 (1 - phi2varc[i]) when phi2varc is set (dodiag;
+ * phi2varc = Phi^2 varc, so that 1 - phi2varc is OuterBase::residvar), obssd = sqrt(v); rows N .. ld-1 are 1 */
+__global__ void gda_obssd_kernel(const double* __restrict__ phi2varc, u64 N, u64 ld, double v0, double v1, double* __restrict__ obssd) {
+  const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= ld) return;
+  double v = 1.0;
+  if (i < N) {
+    v = v0;
+    if (phi2varc) v += v1 * (1 - phi2varc[i]);
+  }
+  obssd[i] = sqrt(v);
 }
 
 __global__ void getmat_kernel(const double* const* load_src, const int* col_op, const uint32_t* csr_ptr,
@@ -1442,7 +1458,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
     const double t1 = cg_block_sum(s1, sm), t2 = cg_block_sum(s2, sm);
     const double val_pr = -0.5 * t1 - t2;
     const double ssq = c.ssq ? c.ssq[blockIdx.x] : c.red[K];
-    const double val_lik = -0.5 * ssq - c.nglobal * log(c.obssd_col ? c.obssd_col[blockIdx.x] : c.obssd);
+    const double val_lik = c.use_sumlogsd ? -0.5 * ssq - c.sumlogsd : -0.5 * ssq - c.nglobal * log(c.obssd_col ? c.obssd_col[blockIdx.x] : c.obssd);
     double val = c.lik_first ? (0.0 + val_lik) + val_pr : (0.0 + val_pr) + val_lik;
     if (c.domarg) val += c.vma_col ? c.vma_col[blockIdx.x] : c.val_margadj;
     const double valo = S[CG_VALO], alpha = S[CG_ALPHA], num = S[CG_NUM];
@@ -1491,7 +1507,7 @@ void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol) {
 }
 
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
-                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols) {
+                        DevBuf<double>& partial, double* ssq_out, const double* sd_cols, const double* sd_rows) {
   if (C == 0) return;
   if (ld == 0) { /* a rank without rows still takes part in the sums over ranks */
     if (update) OB_CUDA(cudaMemsetAsync(ssq_out, 0, C * sizeof(double), c.stream));
@@ -1500,7 +1516,7 @@ void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, 
   const int nb = (int)std::max<u64>(1, std::min<u64>((ld + kResidThreads - 1) / kResidThreads, std::max<u64>(1, (u64)c.sms * 8 / C)));
   if (update) partial.ensure((size_t)nb * C);
   resid_multi_kernel<<<dim3((unsigned)nb, (unsigned)C), kResidThreads, 0, c.stream>>>(yhat, y, w, N, ld, sd, sd_cols, update ? 1 : 0,
-                                                                                      update ? partial.p : nullptr);
+                                                                                      update ? partial.p : nullptr, sd_rows);
   check_launch(c, "resid_multi_kernel");
   if (!update) return;
   colsum_partials_kernel<<<(unsigned)C, 32, 0, c.stream>>>(partial.p, nb, ssq_out);
@@ -1588,6 +1604,12 @@ void launch_rowdot(Ctx& c, const double* A, const double* B, u64 N, u64 K, u64 l
   if (N == 0) return;
   rowdot_kernel<<<(unsigned)((N + 255) / 256), 256, 0, c.stream>>>(A, B, N, K, ld, add, out);
   check_launch(c, "rowdot_kernel");
+}
+
+void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd) {
+  if (ld == 0) return;
+  gda_obssd_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, c.stream>>>(phi2varc, N, ld, v0, v1, obssd);
+  check_launch(c, "gda_obssd_kernel");
 }
 
 void launch_fill(Ctx& c, double* p, u64 n, double v) {

@@ -14,7 +14,9 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
   getsteps      R/fitting.R:188-195
   obfit         R/fitting.R:27-137        both stages: loglik_gda on a subsample, then loglik_gauss on all rows
   obfit_gauss   R/fitting.R:100-136       the stage-2 loop alone, started from the constructor defaults
-  obfit_multi                             obfit_gauss for C responses at the same inputs (no reference counterpart)
+  obfit_multi                             obfit_gauss for C responses at the same inputs (no reference counterpart);
+                                          stage1=True: obfit's two stages, stage 1 on loglik_gda_multi over one row
+                                          subsample shared by the columns
   obpred        R/fitting.R:149-155
 """
 from __future__ import annotations
@@ -311,41 +313,103 @@ def obfit(lib, x, y, numb=100, verbose=0, covnames=None, hyp=None, numberopts=2,
                 predobj=lib.predictor(loglik_faster), optinfo=optinfo, stage1=dict(logpdf=logpdf, loglik=loglik, rows=subset))
 
 
-def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verbose=0, knots=40, para_per_column=False):
+def obfit_multi(lib, x, Y, numb=100, covnames=None, hyp=None, numberopts=2, verbose=0, knots=40, para_per_column=False,
+                stage1=False, seed=0):
     """obfit_gauss for C responses observed at the same inputs (Y is N x C): each column standardised on its own, then
     the same stage-2 loop on lpdfvec(logpr_gauss_multi, loglik_gauss_multi) with domarg -- one basis, one terms table,
     shared hyper-parameters and para, one independent CG per column inside every objective evaluation.
     para_per_column: each column gets its own noise scale and coefficient scale (para has 2 C entries), for outputs
-    whose signal-to-noise ratios differ; the hyper-parameters stay shared."""
+    whose signal-to-noise ratios differ; the hyper-parameters stay shared.
+    stage1: obfit's two stages (R/fitting.R:27-137) instead of stage 2 alone.  Stage 1 fits the hyper-parameters on
+    lpdfvec(logpr_gauss_multi, loglik_gda_multi) over ONE seeded subsample of at most 3 numbr rows shared by all columns
+    (`knots` is then unused: 40 knots, as obfit); stage 2 starts from its hyper-parameters, its two shared para entries
+    (each repeated C times with para_per_column) and its BFGS metric scaled by ssr / n (none with para_per_column: the
+    stage-1 metric has no per-column para block).  With C = 1 this is obfit itself."""
     x = np.asfortranarray(np.asarray(x, dtype=float))
     Y = np.asarray(Y, dtype=float)
     if Y.ndim != 2:
         raise ValueError("Y must be N x C")
     if x.shape[0] != Y.shape[0]:
         raise ValueError("x and Y dims do not align")
-    d = x.shape[1]
+    n, d = x.shape
+    C = Y.shape[1]
+    if stage1:  # obfit's checks, R/fitting.R:30-68
+        if n < d:
+            raise ValueError("dimension larger than sample size has not been tested")
+        if d == 1:
+            raise ValueError("dimension must be larger than 1")
+        if d == 2:
+            raise ValueError("dimension 2 has not been tested")
     if numb < 2 * d:
         raise ValueError("number of basis functions should be less than twice the dimension")
+    if stage1 and numb > 100000:
+        raise ValueError("number of basis functions is beyond testing")
     y_cent, y_sca = Y.mean(axis=0), Y.std(axis=0, ddof=1)
     Ys = np.asfortranarray((Y - y_cent) / y_sca)
+    covnames = list(covnames) if covnames is not None else ["mat25pow"] * d
+    if stage1:
+        if len(covnames) != d:
+            raise ValueError("cov names must be same size as columns in x")
+        for k in range(d):
+            checkcov(covnames[k], x[:, k])
     om = lib.outermod()
-    om.setcovfs(list(covnames) if covnames is not None else ["mat25pow"] * d)
+    om.setcovfs(covnames)
     if hyp is not None and len(hyp) == gethyp(om).size:
         om.updatehyp(hyp)
-    om.setknot(genknotlist([knots] * d, x))
-    terms = om.selectterms(numb)
     percol = {"para_per_column": True} if para_per_column else {}
-    logpr = lib.logpr_gauss_multi(om, terms, Y.shape[1], **percol)
-    loglik = lib.loglik_gauss_multi(om, terms, Ys, x, **percol)
-    logpdf = lib.lpdfvec(logpr, loglik)  # prior first, as obfit_gauss
-    logpdf.domarg = True
-    optinfo = dict(B=None, lr=0.2)
-    for k in range(numberopts):
+    if not stage1:
+        om.setknot(genknotlist([knots] * d, x))
         terms = om.selectterms(numb)
-        logpdf.updateterms(terms)
-        optinfo = BFGS_lpdf(om, logpdf, verbose=verbose, B=optinfo["B"], lr=optinfo["lr"] / 2)
-    return dict(y_cent=y_cent, y_sca=y_sca, om=om, terms=terms, logpdf=logpdf, loglik=loglik, logpr=logpr,
-                predobj=lib.predictor(loglik), optinfo=optinfo)
+        logpr = lib.logpr_gauss_multi(om, terms, C, **percol)
+        loglik = lib.loglik_gauss_multi(om, terms, Ys, x, **percol)
+        logpdf = lib.lpdfvec(logpr, loglik)  # prior first, as obfit_gauss
+        logpdf.domarg = True
+        optinfo = dict(B=None, lr=0.2)
+        for k in range(numberopts):
+            terms = om.selectterms(numb)
+            logpdf.updateterms(terms)
+            optinfo = BFGS_lpdf(om, logpdf, verbose=verbose, B=optinfo["B"], lr=optinfo["lr"] / 2)
+        return dict(y_cent=y_cent, y_sca=y_sca, om=om, terms=terms, logpdf=logpdf, loglik=loglik, logpr=logpr,
+                    predobj=lib.predictor(loglik), optinfo=optinfo)
+    om.setknot(genknotlist([40] * d, x))
+    # ---- stage 1: few terms, one row subsample for every column, loglik_gda_multi (R/fitting.R:76-98)
+    numbr = min(n // 2, numb, 80 * d)
+    terms = om.selectterms(numbr)
+    ssr = min(n, 3 * numbr)
+    logpr = lib.logpr_gauss_multi(om, terms, C)
+    subset = np.sort(np.random.default_rng(seed).choice(n, size=ssr, replace=False))
+    loglik = lib.loglik_gda_multi(om, terms, np.asfortranarray(Ys[subset]), np.asfortranarray(x[subset]))
+    loglik.dodiag = True
+    logpdf = lib.lpdfvec(logpr, loglik)
+    if verbose > 0:
+        print("doing partial optimization")
+    optinfo = BFGS_lpdf(om, logpdf, verbose=verbose, cgsteps=100)
+    # ---- stage 2: all rows, loglik_gauss_multi (R/fitting.R:100-136)
+    terms = om.selectterms(numb)
+    bassize = np.ceil(np.maximum(16, np.minimum(70, 2 * np.asarray(terms).max(axis=0)))).astype(int)
+    om.setknot(genknotlist(bassize, x))
+    if para_per_column:
+        logpr = lib.logpr_gauss_multi(om, terms, C, **percol)
+    loglik_faster = lib.loglik_gauss_multi(om, terms, Ys, x, **percol)
+    logpdf_faster = lib.lpdfvec(logpr, loglik_faster)
+    logpdf_faster.domarg = True
+    para = np.asarray(getpara(logpdf))[:2]
+    if para_per_column:
+        B, para = None, np.repeat(para, C)
+    else:
+        B = np.asarray(optinfo["B"])[:-1, :-1]      # one fewer para, so we strip that one off
+        B = ssr / n * B                              # decrease scale
+    logpdf_faster.updatepara(para)
+    lr = optinfo["lr"]
+    for k in range(numberopts):
+        if verbose > 0:
+            print("doing optimization", k + 1)
+        terms = om.selectterms(numb)
+        logpdf_faster.updateterms(terms)
+        optinfo = BFGS_lpdf(om, logpdf_faster, verbose=verbose, B=B, lr=lr / 2)
+        B, lr = optinfo["B"], optinfo["lr"]
+    return dict(y_cent=y_cent, y_sca=y_sca, om=om, terms=terms, logpdf=logpdf_faster, loglik=loglik_faster, logpr=logpr,
+                predobj=lib.predictor(loglik_faster), optinfo=optinfo, stage1=dict(logpdf=logpdf, loglik=loglik, rows=subset))
 
 
 def obpred(obmodel, x):
