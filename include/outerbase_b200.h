@@ -156,7 +156,16 @@ int ob_outerbase_residvar(ob_outerbase* ob, const uint64_t* terms, uint64_t K, d
 int ob_outerbase_residvar_gradhyp(ob_outerbase* ob, const uint64_t* terms, uint64_t K, double* out /* N x H */);
 /* Device-pointer forms of mm / tmm / mm_mat for callers that keep vectors in HBM
  * (the CG loop, bench.py's `value`).  All *_dev pointers are device memory on
- * ctx's GPU; work is enqueued on ctx's stream and NOT synchronised. */
+ * ctx's GPU; work is enqueued on ctx's stream and NOT synchronised.
+ * set_terms installs the terms table (K x d) they multiply with and must come first:
+ * before it every *_dev call and terms_stats return OB_ERR_STATE and enqueue nothing.
+ * Buffer lengths, with N the rows of the outerbase and K the terms installed:
+ *   mm_dev      a_dev K,       out_dev N   (entries from N on are not written)
+ *   tmm_dev     a_dev N,       out_dev K   (whatever follows a_dev's N entries, NaN included, never contributes)
+ *   mm_mat_dev  A_dev K x C,   out_dev N x C, column-major, leading dimension N
+ *   tmm_mat_dev A_dev N x C,   out_dev K x C, column-major, leading dimensions N and K
+ * Any 8-byte-aligned device pointer is accepted: the library itself pads or realigns an
+ * input that its kernels stage in whole row tiles. */
 int ob_outerbase_set_terms(ob_outerbase* ob, const uint64_t* terms, uint64_t K);
 int ob_outerbase_mm_dev(ob_outerbase* ob, int sq, const double* a_dev, double* out_dev);
 int ob_outerbase_tmm_dev(ob_outerbase* ob, int sq, const double* a_dev, double* out_dev);

@@ -494,6 +494,8 @@ class outerbase(_Handle):
     def _mm(self, sq, terms, a, out=None):
         t, a = _terms(terms), _f64(a)
         if a.ndim == 2:
+            if a.shape[0] != t.shape[0]:
+                raise ValueError("a must have one row per term")
             out = np.empty((self.n_row, a.shape[1]), order="F")
             self._lib.call("outerbase_mm_mat", self._h, C.c_int(sq), _p(t), _u(t.shape[0]), _p(a), _u(a.shape[1]), _p(out))
             return out

@@ -221,28 +221,36 @@ int ob_outerbase_residvar_gradhyp(ob_outerbase* ob, const uint64_t* terms, uint6
 }
 int ob_outerbase_set_terms(ob_outerbase* ob, const uint64_t* terms, uint64_t K) {
   OB_TRY
+  need(ob, "ob"); if (K) need(terms, "terms");
   obe::OuterBase& b = *ob->ob;
   b.cur_terms.assign(terms, terms + K * b.d);
   b.cur_K = K;
   b.coltable(b.program(b.cur_terms.data(), K, -1, 0), 0, -1);
   b.coltable(b.program(b.cur_terms.data(), K, -1, 1), 0, -1);
+  b.terms_set = true;
   OB_CATCH
 }
+/* the object behind a *_dev call: a forgotten set_terms would otherwise run a zero-term program silently */
+static obe::OuterBase& installed(ob_outerbase* ob) {
+  need(ob, "ob");
+  if (!ob->ob->terms_set) throw std::logic_error("set_terms has not been called on this outerbase");
+  return *ob->ob;
+}
 int ob_outerbase_mm_dev(ob_outerbase* ob, int sq, const double* a_dev, double* out_dev) {
-  OB_TRY obe::OuterBase& b = *ob->ob; b.mm_dev(b.cur_terms.data(), b.cur_K, sq, a_dev, out_dev); OB_CATCH
+  OB_TRY obe::OuterBase& b = installed(ob); b.mm_dev(b.cur_terms.data(), b.cur_K, sq, a_dev, out_dev); OB_CATCH
 }
 int ob_outerbase_tmm_dev(ob_outerbase* ob, int sq, const double* a_dev, double* out_dev) {
-  OB_TRY obe::OuterBase& b = *ob->ob; b.tmm_dev(b.cur_terms.data(), b.cur_K, sq, a_dev, out_dev, true, b.N); OB_CATCH
+  OB_TRY obe::OuterBase& b = installed(ob); b.tmm_dev(b.cur_terms.data(), b.cur_K, sq, a_dev, out_dev, true, b.N); OB_CATCH
 }
 int ob_outerbase_mm_mat_dev(ob_outerbase* ob, int sq, const double* A_dev, uint64_t C, double* out_dev) {
-  OB_TRY obe::OuterBase& b = *ob->ob; b.mm_mat_dev(b.cur_terms.data(), b.cur_K, sq, A_dev, C, out_dev, b.N); OB_CATCH
+  OB_TRY obe::OuterBase& b = installed(ob); b.mm_mat_dev(b.cur_terms.data(), b.cur_K, sq, A_dev, C, out_dev, b.N); OB_CATCH
 }
 int ob_outerbase_tmm_mat_dev(ob_outerbase* ob, int sq, const double* A_dev, uint64_t C, double* out_dev) {
-  OB_TRY obe::OuterBase& b = *ob->ob; b.tmm_mat_dev(b.cur_terms.data(), b.cur_K, sq, A_dev, b.N, C, out_dev); OB_CATCH
+  OB_TRY obe::OuterBase& b = installed(ob); b.tmm_mat_dev(b.cur_terms.data(), b.cur_K, sq, A_dev, b.N, C, out_dev); OB_CATCH
 }
 int ob_outerbase_terms_stats(ob_outerbase* ob, uint64_t* W, uint64_t* Lcols, uint64_t* nodes, uint64_t* maxdepth) {
   OB_TRY
-  obe::OuterBase& b = *ob->ob;
+  obe::OuterBase& b = installed(ob);
   const obt::Program& P = b.program(b.cur_terms.data(), b.cur_K, -1)->host;
   *W = P.W; *Lcols = P.Lcols; *nodes = P.nodes; *maxdepth = P.maxdepth;
   OB_CATCH

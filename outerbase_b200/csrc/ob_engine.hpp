@@ -105,9 +105,10 @@ struct OuterBase {
   DevBuf<double> tmpC, tmpKd, tmpHp, tmpNg, tmpK2, tmpGe;
   DevBuf<unsigned char> tmpMask;
   std::list<SpecEntry> specs;
-  /* terms installed by set_terms for the *_dev entry points */
+  /* terms installed by set_terms for the *_dev entry points; they refuse to run before it */
   std::vector<u64> cur_terms;
   u64 cur_K = 0;
+  bool terms_set = false;
 
   /* hint_terms (K x d): the table the owner is going to multiply with -- the basis is built for its levels only */
   OuterBase(Ctx& c, const OuterMod* om_, const double* xh, u64 N_, bool dograd_, const u64* hint_terms = nullptr, u64 hint_K = 0)
