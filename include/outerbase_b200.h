@@ -247,6 +247,12 @@ int ob_debug_terms_eval(const uint64_t* terms, uint64_t K, uint64_t d, const uin
  * (a table the trie compiler refuses, or no layout fits in shared memory).  Specialised kernels are not reported. */
 int ob_outerbase_debug_phi_geometry(ob_outerbase* ob, const uint64_t* terms, uint64_t K, int transpose, int sq,
                                     int* out /* 4 */);
+/* Test hook: the kernel each dimension's last basis build ran on.  out holds 4 values per dimension, dimension l at
+ * out[4 l .. 4 l + 3] = {family: 1 the tensor-core (DMMA) kernel, 0 the FMA kernel; its tile: column tiles of 8 (DMMA)
+ * or rows per CTA (FMA); columns built (levels 0 .. mo-1); dynamic shared-memory bytes}.  The lpdf form reports the
+ * basis a likelihood holds. */
+int ob_outerbase_debug_build_geometry(ob_outerbase* ob, int* out /* 4 d */);
+int ob_lpdf_debug_build_geometry(ob_lpdf* l, int* out /* 4 d */);
 
 /* ------------------------------------------------------------------ stateless linalg.h seam
  * Exactly the eight free functions of src/linalg.h:9-58: same argument meaning, host

@@ -128,6 +128,8 @@ int ref_spec_compile_check(const char*, uint64_t*, double*) { g_err = "the refer
 int ref_debug_terms_eval(const uint64_t*, uint64_t, uint64_t, const uint64_t*, int, int, const double*, const double*, const double*, double,
                          double*, double*, uint64_t*) { g_err = "the reference has no terms compiler"; return REF_ERR_STATE; }
 int ref_outerbase_debug_phi_geometry(ref_outerbase*, const uint64_t*, uint64_t, int, int, int*) { g_err = "the reference has no kernels"; return REF_ERR_STATE; }
+int ref_outerbase_debug_build_geometry(ref_outerbase*, int*) { g_err = "the reference has no kernels"; return REF_ERR_STATE; }
+int ref_lpdf_debug_build_geometry(ref_lpdf*, int*) { g_err = "the reference has no kernels"; return REF_ERR_STATE; }
 
 static covf* make_covf(const std::string& n) { /* interfaceR.cpp:60-68 */
   if (n == "mat25") return new covf_mat25();

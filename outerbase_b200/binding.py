@@ -316,6 +316,12 @@ class _Handle:
             pass
 
 
+def _build_geometry(lib, name, h, d):
+    out = (C.c_int * (4 * d))()
+    lib.call(name, h, out)
+    return [("dmma" if out[4 * l] else "fma", out[4 * l + 1], out[4 * l + 2], out[4 * l + 3]) for l in range(d)]
+
+
 class outermod(_Handle):
     """new(outermod) -- src/modandbase.h:9-54."""
     _destroy = "outermod_destroy"
@@ -452,6 +458,11 @@ class outerbase(_Handle):
         out = (C.c_int * 4)()
         self._lib.call("outerbase_debug_phi_geometry", self._h, _p(t), _u(t.shape[0]), C.c_int(1 if transpose else 0), C.c_int(sq), out)
         return dict(zip(("R", "nbuf", "prog_in_smem", "smem"), map(int, out)))
+
+    def debug_build_geometry(self):
+        """The kernel each dimension's last basis build ran on: one (family, tile, mo, smem) per dimension, family
+        "dmma" (tile = column tiles of 8) or "fma" (tile = rows per CTA). Product only."""
+        return _build_geometry(self._lib, "outerbase_debug_build_geometry", self._h, self.d)
 
     def _loopvals(self):
         nt, cs, ls, vp = C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_int()
@@ -645,6 +656,10 @@ class lpdf(_Handle):
     compute_grad = property(fset=lambda s, v: s._flag("compute_grad", v))
     compute_gradhyp = property(fset=lambda s, v: s._flag("compute_gradhyp", v))
     compute_gradpara = property(fset=lambda s, v: s._flag("compute_gradpara", v))
+
+    def debug_build_geometry(self):
+        """outerbase.debug_build_geometry for the basis a likelihood holds. Product only."""
+        return _build_geometry(self._lib, "lpdf_debug_build_geometry", self._h, self._om.d)
 
     def setnthreads(self, k):
         self._lib.call("lpdf_setnthreads", self._h, C.c_int(int(k)))

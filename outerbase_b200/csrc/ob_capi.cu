@@ -390,6 +390,25 @@ int ob_outerbase_debug_phi_geometry(ob_outerbase* ob, const uint64_t* terms, uin
   OB_CATCH
 }
 
+static void build_geometry(const obe::OuterBase& b, int* out) {
+  if (b.build_geom.size() != b.d) throw std::logic_error("this object has not built a basis");
+  for (size_t l = 0; l < b.build_geom.size(); ++l) {
+    const obd::BuildGeom& g = b.build_geom[l];
+    out[4 * l] = g.mma; out[4 * l + 1] = g.tile; out[4 * l + 2] = g.mo; out[4 * l + 3] = g.smem;
+  }
+}
+int ob_outerbase_debug_build_geometry(ob_outerbase* ob, int* out) {
+  OB_TRY need(ob, "ob"); need(out, "out"); build_geometry(*ob->ob, out); OB_CATCH
+}
+int ob_lpdf_debug_build_geometry(ob_lpdf* l, int* out) {
+  OB_TRY
+  need(l, "l"); need(out, "out");
+  if (auto* lik = dynamic_cast<obe::DevLik*>(l->p.get())) build_geometry(lik->ob, out);
+  else if (auto* gda = dynamic_cast<obe::LoglikGda*>(l->p.get())) build_geometry(gda->ob, out);
+  else throw std::invalid_argument("only a likelihood holds a basis");
+  OB_CATCH
+}
+
 /* ---- stateless linalg.h seam */
 #define SEAM_BASE(bmge, Mge, ge, hm, H) \
   need(ctx, "ctx");                     \

@@ -330,9 +330,15 @@ struct BuildDims {
   u64 rot_off;   /* column offset of the dim's block in rotmat */
   u64 rotg_off[2];
 };
+/* the kernel one dimension was built with: mma = 1 the DMMA kernel (tile = NT column tiles of 8), 0 the FMA kernel
+ * (tile = ROWS rows per CTA); mo columns built; smem dynamic shared-memory bytes */
+struct BuildGeom { int mma, tile, mo, smem; };
+/* geom receives one entry per dimension.  Every dimension's kernel is chosen before any is launched: a dimension with
+ * more knots than any kernel holds throws std::range_error and nothing is written. */
 void launch_basis_build(Ctx& c, const std::vector<BuildDims>& dims, const double* x_dev, u64 N, u64 ld,
                         const double* knots_dev, const double* rot_dev, u64 rot_ld, const double* rotg_dev,
-                        double* basemat, double* basematge, double* scalemat, double* scale, bool dograd);
+                        double* basemat, double* basematge, double* scalemat, double* scale, bool dograd,
+                        std::vector<BuildGeom>& geom);
 void launch_getbase(Ctx& c, const double* basemat, const double* scalemat_col, u64 N, u64 ld, u64 col0, u64 m, double* out);
 void launch_cov(Ctx& c, int kind, const double* hyp, const double* x1, u64 n1, const double* x2, u64 n2,
                 double* out, double* outg /* may be null */);

@@ -62,6 +62,7 @@ struct OuterBase {
    * the lpdf classes know their terms and start pruned. */
   std::vector<u64> mo, cst, cge;
   u64 Mc = 0, Mgec = 0;
+  std::vector<obd::BuildGeom> build_geom; /* the kernel each dimension's last build ran on (a test hook reports it) */
   DevBuf<double> x, basemat, basematge, scalemat, scale;
   /* basematsq (modandbase.cpp:527-531), materialised at the first squared operator after a build: squaring the staged
    * tile inside the Phi kernels instead made every squared product 3x slower than the plain one, and a BFGS
@@ -221,7 +222,7 @@ struct OuterBase {
       for (int h = 0; h < D.nh; ++h) { D.ge_off[h] = cge[hypst[l] + h]; D.rotg_off[h] = gest[hypst[l] + h]; }
     }
     obd::launch_basis_build(ctx, dims, x.p, N, ld, knots_dev.p, rot_dev.p, om->rotmat.nr, rotg_dev.p, basemat.p,
-                            dograd ? basematge.p : nullptr, scalemat.p, scale.p, dograd);
+                            dograd ? basematge.p : nullptr, scalemat.p, scale.p, dograd, build_geom);
     ctx.sync(); /* host vectors above must outlive the async uploads */
     coltables.clear(); /* buffers may have moved */
     sq_valid = false;

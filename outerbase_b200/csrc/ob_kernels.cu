@@ -1634,10 +1634,48 @@ void launch_cov(Ctx& c, int kind, const double* hyp, const double* x1, u64 n1, c
 
 void launch_basis_build(Ctx& c, const std::vector<BuildDims>& dims, const double* x_dev, u64 N, u64 ld, const double* knots_dev,
                         const double* rot_dev, u64 rot_ld, const double* rotg_dev, double* basemat, double* basematge,
-                        double* scalemat, double* scale, bool dograd) {
+                        double* scalemat, double* scale, bool dograd, std::vector<BuildGeom>& geom) {
   if (ld == 0) return;
+  static const bool use_mma = !(getenv("OB_BUILD") && std::string(getenv("OB_BUILD")) == "fma");
+  /* shared memory of the FMA kernel (ROWS rows per CTA) and of the DMMA kernel (NT column tiles) for m knots */
+  auto need = [](int m, int nh, int rows) {
+    const size_t mp = ((m + 3) / 4) * 4 + 4;
+    return ((size_t)(1 + nh) * m * mp + (size_t)(1 + nh) * m * rows + 2 * m + 2 * rows) * sizeof(double);
+  };
+  auto need_mma = [](int m, int nh, int nt) {
+    const size_t mk = (m + 3) & ~3;
+    return ((size_t)(1 + nh) * mk * (nt * 8 + 4) + (size_t)(1 + nh) * mk * 72 + 2 * m + 2 * 64) * sizeof(double);
+  };
+  const size_t optin = c.smem_optin;
+  std::vector<BuildGeom> plan(dims.size());
   for (size_t l = 0; l < dims.size(); ++l) {
     const BuildDims& D = dims[l];
+    const int nh = dograd ? D.nh : 0;
+    const int mo = D.mo > 0 && D.mo < D.m ? D.mo : D.m;
+    /* column tiles of 8: the smallest instantiation that covers the columns to build (the accumulators of a tile
+     * live in registers, so the count is a template argument) */
+    const int nt = (mo + 7) / 8;
+    BuildGeom& G = plan[l];
+    G = BuildGeom{-1, 0, mo, 0};
+    if (use_mma && D.m <= 72)
+      for (const int t : {1, 2, 3, 5, 9})
+        if (nt <= t && need_mma(D.m, nh, t) <= optin) { G = BuildGeom{1, t, mo, (int)need_mma(D.m, nh, t)}; break; }
+    if (G.mma < 0) {
+      if (need(D.m, nh, 64) <= optin) G = BuildGeom{0, 64, mo, (int)need(D.m, nh, 64)};
+      else if (need(D.m, nh, 32) <= optin) G = BuildGeom{0, 32, mo, (int)need(D.m, nh, 32)};
+      else {
+        int cap = D.m;
+        while (cap > 2 && need(cap, nh, 32) > optin) --cap;
+        throw std::range_error("basis build: dimension " + std::to_string(l + 1) + " has " + std::to_string(D.m) +
+                               " knots, more than the " + std::to_string(cap) + " the basis-build kernel holds in a dimension with " +
+                               std::to_string(nh) + " hyper-parameter gradient" + (nh == 1 ? "" : "s"));
+      }
+    }
+  }
+  geom = plan;
+  for (size_t l = 0; l < dims.size(); ++l) {
+    const BuildDims& D = dims[l];
+    const BuildGeom& G = plan[l];
     BuildKParams p{};
     p.kind = D.kind; p.m = D.m; p.nh = D.nh; p.mp = ((D.m + 3) / 4) * 4 + 4;
     p.h0 = D.hyp[0]; p.h1 = D.hyp[1];
@@ -1652,37 +1690,31 @@ void launch_basis_build(Ctx& c, const std::vector<BuildDims>& dims, const double
     p.bg1 = dograd && D.nh > 1 ? basematge + D.ge_off[1] * ld : nullptr;
     p.scalecol = scalemat + l * ld;
     p.N = N; p.ld = ld; p.dograd = dograd ? 1 : 0;
-    p.mo = D.mo > 0 && D.mo < D.m ? D.mo : D.m;
-    const int nh = dograd ? D.nh : 0;
-    auto need = [&](int rows) {
-      return ((size_t)(1 + nh) * D.m * p.mp + (size_t)(1 + nh) * D.m * rows + 2 * D.m + 2 * rows) * sizeof(double);
-    };
-    const int mk = (D.m + 3) & ~3;
-    auto need_mma = [&](int nt) {
-      return ((size_t)(1 + nh) * mk * (nt * 8 + 4) + (size_t)(1 + nh) * mk * 72 + 2 * D.m + 2 * 64) * sizeof(double);
-    };
-    static const bool use_mma = !(getenv("OB_BUILD") && std::string(getenv("OB_BUILD")) == "fma");
-    /* column tiles of 8: the smallest instantiation that covers the columns to build (the accumulators of a tile
-     * live in registers, so the count is a template argument); 2 CTAs per SM up to 5 tiles */
+    p.mo = G.mo;
+    const size_t smem = (size_t)G.smem;
+    /* 2 CTAs per SM up to 5 column tiles */
 #define OB_BUILD_MMA(NT_, PER_SM)                                                                                   \
     {                                                                                                               \
-      set_smem(basis_build_mma_kernel<NT_>, need_mma(NT_));                                                         \
-      basis_build_mma_kernel<NT_><<<(unsigned)std::min<u64>((ld + 63) / 64, (u64)c.sms * PER_SM), 256, need_mma(NT_), c.stream>>>(p); \
+      set_smem(basis_build_mma_kernel<NT_>, smem);                                                                  \
+      basis_build_mma_kernel<NT_><<<(unsigned)std::min<u64>((ld + 63) / 64, (u64)c.sms * PER_SM), 256, smem, c.stream>>>(p); \
     }
-    const int nt = (p.mo + 7) / 8;
-    if (use_mma && D.m <= 72 && nt <= 1 && need_mma(1) <= c.smem_optin) OB_BUILD_MMA(1, 2)
-    else if (use_mma && D.m <= 72 && nt <= 2 && need_mma(2) <= c.smem_optin) OB_BUILD_MMA(2, 2)
-    else if (use_mma && D.m <= 72 && nt <= 3 && need_mma(3) <= c.smem_optin) OB_BUILD_MMA(3, 2)
-    else if (use_mma && D.m <= 72 && nt <= 5 && need_mma(5) <= c.smem_optin) OB_BUILD_MMA(5, 2)
-    else if (use_mma && D.m <= 72 && need_mma(9) <= c.smem_optin) OB_BUILD_MMA(9, 1)
+    if (G.mma) {
+      switch (G.tile) {
+        case 1: OB_BUILD_MMA(1, 2) break;
+        case 2: OB_BUILD_MMA(2, 2) break;
+        case 3: OB_BUILD_MMA(3, 2) break;
+        case 5: OB_BUILD_MMA(5, 2) break;
+        default: OB_BUILD_MMA(9, 1) break;
+      }
+    }
 #undef OB_BUILD_MMA
-    else if (need(64) <= c.smem_optin) {
-      set_smem(basis_build_kernel<64>, need(64));
-      basis_build_kernel<64><<<(unsigned)((ld + 63) / 64), 256, need(64), c.stream>>>(p);
-    } else if (need(32) <= c.smem_optin) {
-      set_smem(basis_build_kernel<32>, need(32));
-      basis_build_kernel<32><<<(unsigned)((ld + 31) / 32), 256, need(32), c.stream>>>(p);
-    } else throw std::range_error("too many knots in one dimension for the basis-build kernel");
+    else if (G.tile == 64) {
+      set_smem(basis_build_kernel<64>, smem);
+      basis_build_kernel<64><<<(unsigned)((ld + 63) / 64), 256, smem, c.stream>>>(p);
+    } else {
+      set_smem(basis_build_kernel<32>, smem);
+      basis_build_kernel<32><<<(unsigned)((ld + 31) / 32), 256, smem, c.stream>>>(p);
+    }
     check_launch(c, "basis_build_kernel");
   }
   basescale_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, c.stream>>>(scalemat, ld, (int)dims.size(), N, scale);
