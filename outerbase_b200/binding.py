@@ -136,6 +136,13 @@ class Library:
         self.call("spec_compile_check", source.encode(), C.byref(nb), C.byref(sec))
         return nb.value, sec.value
 
+    def debug_normals(self, seed, stream, column, first, n):
+        """n standard normals of the posterior draws' generator (seed, stream, column) from index `first` on, computed
+        on the host (include/outerbase_b200_draws.h); no GPU needed."""
+        out = np.empty(int(n))
+        self.call("debug_normals", _u(seed), C.c_uint32(int(stream)), _u(column), _u(first), _u(n), _p(out))
+        return out
+
     def fp64_peak(self) -> float:
         v = C.c_double()
         self.call("ctx_fp64_peak", self.ctx, C.byref(v))
@@ -856,6 +863,11 @@ class logpr_gauss_multi(_multi, lpdf):
         else:
             lib.call("logpr_gauss_multi_create", lib.ctx, om._h, _p(t), _u(t.shape[0]), _u(ncol), C.byref(self._h))
 
+    def set_mean(self, mean=None):
+        """Centre column c's prior at mean[:, c] (K x ncol); None: every prior centred at 0."""
+        m = _f64(mean) if mean is not None else None
+        self._lib.call("logpr_gauss_multi_set_mean", self._h, _p(m), _u(0 if m is None else m.size))
+
 
 class loglik_gda_multi(_multi, lpdf):
     """loglik_gda on each column of Y (N x C), all columns on one basis with one per-row noise scale
@@ -880,6 +892,42 @@ class lpdfvec_multi(_multi, lpdfvec):
     """lpdfvec of two multi-response children; optcg runs one independent CG per column."""
     cg_iters_per_column = property(lambda s: s._get("cg_iters").astype(int))
     cg_iters = property(lambda s: int(s._get("cg_iters").max()))
+
+
+class posterior_draws(_Handle):
+    """S joint draws from the posterior of a fitted lpdfvec(logpr_gauss, loglik_gauss), by perturb-and-MAP
+    (include/outerbase_b200_draws.h): the object copies the fit when it is made; `solve` runs the S perturbed fits,
+    `coeff` is K x S, `predict(x)` the N x S draws of the latent function at new inputs."""
+    _destroy = "draws_destroy"
+
+    def __init__(self, lib, logpdf, S, seed=0):
+        super().__init__(lib)
+        self.S = int(S)
+        lib.call("draws_create", logpdf._h, _u(S), _u(seed), C.byref(self._h))
+
+    def _get(self, which, nrow=None):
+        n = C.c_uint64()
+        self._lib.call("draws_get", self._h, which.encode(), C.c_void_p(0), C.byref(n))
+        out = np.empty(n.value)
+        self._lib.call("draws_get", self._h, which.encode(), _p(out), C.byref(n))
+        return out if nrow is None else out.reshape((-1, self.S), order="F")
+
+    def solve(self, tol=0.001, maxepch=100):
+        self._lib.call("draws_solve", self._h, C.c_double(tol), _u(maxepch))
+        return self
+
+    coeff = property(lambda s: s._get("coeff", True))
+    cg_iters = property(lambda s: s._get("cg_iters").astype(int))
+    y = property(lambda s: s._get("y", True))  # the perturbed responses, N x S
+    prior_mean = property(lambda s: s._get("prior_mean", True))  # the prior centres delta_s, K x S
+
+    def predict(self, x):
+        x = _f64(x)
+        if x.ndim != 2:
+            raise ValueError("x must be N x d")
+        out = np.empty((x.shape[0], self.S), order="F")
+        self._lib.call("draws_predict", self._h, _p(x), _u(x.shape[0]), _p(out))
+        return out
 
 
 class predictor(_Handle):

@@ -7,6 +7,7 @@
 #include "../../include/outerbase_b200_multi.h"
 #include "../../include/outerbase_b200_multi_percol.h"
 #include "../../include/outerbase_b200_multi_gda.h"
+#include "../../include/outerbase_b200_draws.h"
 
 #include "ob_engine.hpp"
 
@@ -30,6 +31,7 @@ struct ob_outermod { obh::OuterMod om; };
 struct ob_outerbase { ob_ctx* ctx; std::unique_ptr<obe::OuterBase> ob; };
 struct ob_lpdf { ob_ctx* ctx; std::unique_ptr<obe::Lpdf> p; };
 struct ob_predictor { std::unique_ptr<obe::Pred> p; };
+struct ob_draws { std::unique_ptr<obe::Draws> d; };
 
 static void need(const void* p, const char* what) { if (!p) throw std::invalid_argument(std::string("null ") + what); }
 
@@ -636,5 +638,56 @@ int ob_predictor_destroy(ob_predictor* p) { OB_TRY delete p; OB_CATCH }
 int ob_predictor_update(ob_predictor* p, const double* x, uint64_t N) { OB_TRY p->p->update(x, N); OB_CATCH }
 int ob_predictor_mean(ob_predictor* p, double* out) { OB_TRY p->p->mean(out); OB_CATCH }
 int ob_predictor_var(ob_predictor* p, double* out) { OB_TRY p->p->var(out); OB_CATCH }
+
+/* ---- posterior draws (include/outerbase_b200_draws.h) */
+int ob_draws_create(ob_lpdf* logpdf, uint64_t S, uint64_t seed, ob_draws** out) {
+  OB_TRY
+  need(logpdf, "logpdf"); need(out, "out");
+  auto* h = new ob_draws();
+  try { h->d.reset(new obe::Draws(logpdf->p.get(), S, seed)); } catch (...) { delete h; throw; }
+  *out = h;
+  OB_CATCH
+}
+int ob_draws_destroy(ob_draws* d) { OB_TRY delete d; OB_CATCH }
+int ob_draws_solve(ob_draws* d, double tol, uint64_t maxepch) { OB_TRY need(d, "d"); d->d->solve(tol, maxepch); OB_CATCH }
+int ob_draws_get(ob_draws* d, const char* which, double* out, uint64_t* n) {
+  OB_TRY
+  need(d, "d"); need(which, "which"); need(n, "n");
+  obe::Draws& D = *d->d;
+  const std::string w = which;
+  std::vector<double> v;
+  if (w == "coeff") v = D.coeff();
+  else if (w == "cg_iters") { D.coeff(); v.assign(D.vec->cg_iters_cols.begin(), D.vec->cg_iters_cols.end()); }
+  else if (w == "y") v = D.y();
+  else if (w == "prior_mean") v = D.pr->mean;
+  else throw std::invalid_argument("unknown field " + w);
+  *n = v.size();
+  if (out) std::copy(v.begin(), v.end(), out);
+  OB_CATCH
+}
+int ob_draws_predict(ob_draws* d, const double* x, uint64_t N, double* out) {
+  OB_TRY need(d, "d"); if (N) { need(x, "x"); need(out, "out"); } d->d->predict(x, N, out); OB_CATCH
+}
+int ob_debug_normals(uint64_t seed, uint32_t stream, uint64_t column, uint64_t first, uint64_t n, double* out) {
+  OB_TRY
+  if (n) need(out, "out");
+  if (column > 0xFFFFFFFFull || (n && (first + n - 1) >> 1 > 0xFFFFFFFFull))
+    throw std::range_error("the generator's column and index are 32-bit words");
+  for (u64 i = first; i < first + n; ++i) {
+    double z[2];
+    obd::draw_normal_pair(seed, stream, (uint32_t)column, (uint32_t)(i >> 1), z);
+    out[i - first] = z[i & 1];
+  }
+  OB_CATCH
+}
+int ob_logpr_gauss_multi_set_mean(ob_lpdf* logpr, const double* mean, uint64_t n) {
+  OB_TRY
+  need(logpr, "logpr");
+  auto* m = dynamic_cast<obe::LogprGaussMulti*>(logpr->p.get());
+  if (!m) throw std::invalid_argument("set_mean is a method of logpr_gauss_multi");
+  if (n) need(mean, "mean");
+  m->set_mean(mean, n);
+  OB_CATCH
+}
 
 } // extern "C"

@@ -307,6 +307,9 @@ struct CgParams {
    * instead of -0.5 ssq - nglobal log obssd */
   int use_sumlogsd = 0;
   double sumlogsd = 0;
+  /* posterior draws (DESIGN §3.9): K x C prior means; CG_POST_UPDATE takes (coeff - prior_mean) / sd for the prior's
+   * value and gradient.  Null: every prior is centred at 0 (every other launch) */
+  const double* prior_mean = nullptr;
 };
 enum { CG_NUM = 0, CG_DENOM, CG_ALPHA, CG_BETA, CG_VAL, CG_VALO, CG_VALDIFF, CG_STOP, CG_VAL_LIK, CG_VAL_PR, CG_ITER, CG_NSCAL = 16 };
 void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol = 1);
@@ -318,6 +321,45 @@ void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, 
                         DevBuf<double>& partial, double* ssq_out, const double* sd_cols = nullptr, const double* sd_rows = nullptr);
 /* loglik_gda's obssd on the device: obssd[i] = sqrt(v0 + v1 (1 - phi2varc[i])) (phi2varc null: sqrt(v0)), pad rows 1 */
 void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd);
+
+/* ---- standard normals of the posterior draws (DESIGN §3.9), the same on the host and the device.
+ * Philox4x32-10 (Salmon, Moraes, Dror, Shaw, SC'11; the constants of Random123) with key (seed low 32, seed high 32) and
+ * counter (index, stream, column, 0).  One output gives two uniforms in (0, 1], u = ((x >> 11) + 1) 2^-53 with x the
+ * 64-bit words (v1 v0) and (v3 v2), and two normals by Box-Muller: r cos(2 pi u2), r sin(2 pi u2), r = sqrt(-2 log u1).
+ * Normal i of (seed, stream, column) is component i & 1 of index i >> 1, so a value depends on nothing but these four. */
+enum DrawStream : uint32_t { DRAW_ROWS = 0 /* row noise eps */, DRAW_PRIOR = 1 /* prior noise xi */ };
+__host__ __device__ inline uint32_t philox_mulhilo(uint32_t a, uint32_t b, uint32_t* lo) {
+  *lo = a * b;
+#ifdef __CUDA_ARCH__
+  return __umulhi(a, b);
+#else
+  return (uint32_t)(((uint64_t)a * b) >> 32);
+#endif
+}
+__host__ __device__ inline void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+  for (int r = 0; r < 10; ++r) {
+    if (r) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+    uint32_t lo0, lo1;
+    const uint32_t hi0 = philox_mulhilo(0xD2511F53u, c[0], &lo0), hi1 = philox_mulhilo(0xCD9E8D57u, c[2], &lo1);
+    const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
+    c[0] = n0; c[1] = lo1; c[2] = n2; c[3] = lo0;
+  }
+}
+/* normals 2 index and 2 index + 1 of (seed, stream, column) */
+__host__ __device__ inline void draw_normal_pair(uint64_t seed, uint32_t stream, uint32_t column, uint32_t index, double z[2]) {
+  uint32_t c[4] = {index, stream, column, 0u};
+  philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  const double u1 = (double)((((uint64_t)c[1] << 32 | c[0]) >> 11) + 1) * 0x1p-53;
+  const double u2 = (double)((((uint64_t)c[3] << 32 | c[2]) >> 11) + 1) * 0x1p-53;
+  const double r = sqrt(-2.0 * log(u1)), th = 6.283185307179586 * u2;
+  z[0] = r * cos(th);
+  z[1] = r * sin(th);
+}
+/* the perturbations of S posterior draws, one launch: y[i, s] = y0[i] + sigma eps_s[i] for the N rows (pad rows of the
+ * ld x S y written 0) and delta[k, s] = (sds[k] sca) xi_s[k] (K x S), eps and xi the normals of streams DRAW_ROWS and
+ * DRAW_PRIOR in column s */
+void launch_draws_perturb(Ctx& c, const double* y0, u64 N, u64 ld, double sigma, const double* sds, double sca, u64 K, u64 S,
+                          uint64_t seed, double* y, double* delta);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

@@ -975,8 +975,11 @@ struct DevLik : Lpdf {
   DevBuf<double> y, yhat, w, kbuf, red;
   std::vector<double> ssq_host; /* per-column sums of squared standardised residuals of the last update (all ranks) */
 
-  DevLik(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
-      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K_), N(N_), K(K_), C(C_) {
+  /* ybcast: yh is ONE response (N) that every column starts from (the posterior draws perturb the columns on the
+   * device); dograd: build the basis with its hyper-parameter gradient columns */
+  DevLik(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
+         bool ybcast = false, bool dograd = true)
+      : ctx(c), om(om_), ob(c, om_, xh, N_, dograd, t, K_), N(N_), K(K_), C(C_) {
     if (C == 0) throw std::invalid_argument("ncol must be at least 1");
     d = om->d;
     terms.assign(t, t + K * d);
@@ -986,7 +989,8 @@ struct DevLik : Lpdf {
     y.ensure(ld * C);
     OB_CUDA(cudaMemsetAsync(y.p, 0, ld * C * sizeof(double), ctx.stream));
     for (u64 j = 0; j < C; ++j)
-      if (N) OB_CUDA(cudaMemcpyAsync(y.p + j * ld, yh + j * N, N * sizeof(double), cudaMemcpyHostToDevice, ctx.stream));
+      if (N && ybcast && j > 0) OB_CUDA(cudaMemcpyAsync(y.p + j * ld, y.p, N * sizeof(double), cudaMemcpyDeviceToDevice, ctx.stream));
+      else if (N) OB_CUDA(cudaMemcpyAsync(y.p + j * ld, yh + j * N, N * sizeof(double), cudaMemcpyHostToDevice, ctx.stream));
     yhat.ensure(ld * C); w.ensure(ld * C);
     ctx.sync();
   }
@@ -1028,27 +1032,28 @@ struct LoglikGaussBase : DevLik {
   std::vector<double> sqcs;      /* the last sqcolsums(); empty after updateom / updateterms */
 
   LoglikGaussBase(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
-                  bool percol_ = false)
-      : DevLik(c, om_, t, K_, yh, C_, xh, N_), percol(percol_) {
+                  bool percol_ = false, bool ybcast = false, bool dograd = true)
+      : DevLik(c, om_, t, K_, yh, C_, xh, N_, ybcast, dograd), percol(percol_) {
     npara = 1;
     /* para0 = log(0.01 * mean over the columns of var(y[:,c])), loglik_gauss.cpp:48 (Armadillo two-pass var); over ALL
      * ranks' rows */
+    const u64 cs = ybcast ? 0 : N; /* column stride of yh */
     std::vector<double> var(C);
     if (ctx.nranks > 1) {
       std::vector<double> st(C + 1, 0.0), ss(C, 0.0);
       st[0] = double(N);
-      for (u64 j = 0; j < C; ++j) for (u64 i = 0; i < N; ++i) st[1 + j] += yh[i + j * N];
+      for (u64 j = 0; j < C; ++j) for (u64 i = 0; i < N; ++i) st[1 + j] += yh[i + j * cs];
       allreduce_host(st.data(), C + 1);
       Nglobal = st[0];
       for (u64 j = 0; j < C; ++j) {
         const double mean = st[1 + j] / st[0];
-        for (u64 i = 0; i < N; ++i) ss[j] += (yh[i + j * N] - mean) * (yh[i + j * N] - mean);
+        for (u64 i = 0; i < N; ++i) ss[j] += (yh[i + j * cs] - mean) * (yh[i + j * cs] - mean);
       }
       allreduce_host(ss.data(), C);
       for (u64 j = 0; j < C; ++j) var[j] = ss[j] / (Nglobal - 1);
     } else {
       Nglobal = double(N);
-      for (u64 j = 0; j < C; ++j) var[j] = arma_var(yh + j * N, N);
+      for (u64 j = 0; j < C; ++j) var[j] = arma_var(yh + j * cs, N);
     }
     if (percol) { /* column c: loglik_gauss's own default on Y[:,c] */
       npara = C;
@@ -1492,6 +1497,13 @@ struct LogprGaussMulti : Lpdf {
   u64 K, C;
   bool percol;
   std::vector<double> val_cols;
+  /* K x C prior means (posterior draws, DESIGN §3.9): column c's prior is centred at mean[:, c], i.e. update evaluates
+   * logpr_gauss at coeff[:, c] - mean[:, c].  Empty: every prior is centred at 0.  The Hessian does not depend on it. */
+  std::vector<double> mean;
+  void set_mean(const double* m, u64 n) {
+    if (n && n != K * C) throw std::range_error("the prior mean must have K x ncol entries");
+    mean.assign(m, m + n);
+  }
   LogprGaussMulti(const OuterMod* om_, const u64* t, u64 K_, u64 C_, bool percol_ = false) : one(om_, t, K_), K(K_), C(C_), percol(percol_) {
     if (C == 0) throw std::invalid_argument("ncol must be at least 1");
     d = one.d; npara = one.npara; terms = one.terms; para0 = one.para0; paravar = one.paravar; para = one.para;
@@ -1527,7 +1539,7 @@ struct LogprGaussMulti : Lpdf {
     if (n != C) throw std::range_error("para must have one entry per column");
     para.assign(p, p + n);
   }
-  void updateterms(const u64* t, u64 K_) override { one.updateterms(t, K_); terms = one.terms; K = K_; nterms = K * C; }
+  void updateterms(const u64* t, u64 K_) override { one.updateterms(t, K_); terms = one.terms; K = K_; nterms = K * C; mean.clear(); }
   std::vector<double> column(const std::vector<double>& v, u64 c) const { return std::vector<double>(v.begin() + c * K, v.begin() + (c + 1) * K); }
   void update(const std::vector<double>& cf) override {
     if (cf.size() != K * C) throw std::range_error("coeff must have K x ncol entries");
@@ -1539,7 +1551,9 @@ struct LogprGaussMulti : Lpdf {
     if (compute_gradpara) gradpara.assign(percol ? C : 1, 0.0);
     for (u64 c = 0; c < C; ++c) {
       at(c);
-      one.update(column(cf, c));
+      std::vector<double> cc = column(cf, c);
+      if (!mean.empty()) for (u64 i = 0; i < K; ++i) cc[i] -= mean[c * K + i];
+      one.update(cc);
       if (compute_val) { val += one.val; val_cols[c] = one.val; }
       if (compute_grad) std::copy(one.grad.begin(), one.grad.end(), grad.begin() + c * K);
       if (compute_gradhyp) for (u64 h = 0; h < gradhyp.size(); ++h) gradhyp[h] += one.gradhyp[h];
@@ -1602,8 +1616,8 @@ struct LoglikGaussMulti : LoglikGaussBase {
   DevBuf<double> sd_dev; /* percol: obssd_cols on the device, refreshed by updatepara */
 
   LoglikGaussMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_,
-                   bool percol_ = false)
-      : LoglikGaussBase(c, om_, t, K_, yh, C_, xh, N_, percol_) {
+                   bool percol_ = false, bool ybcast = false, bool dograd = true)
+      : LoglikGaussBase(c, om_, t, K_, yh, C_, xh, N_, percol_, ybcast, dograd) {
     ssq.ensure(C);
     upload_sds();
   }
@@ -2072,10 +2086,11 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
    * marginal adjustment, coefficient scale and noise sd go to the kernel as C-entry device arrays, uploaded here once.
    * A single-response pairing returns false (the caller runs the host loop) without option device_cg, rows or a
    * specialised terms table, and for every other pairing; a multi-response object runs here or throws. */
-  DevBuf<double> cg_coeff, cg_grad, cg_m, cg_rm, cg_p, cg_q, cg_sds, cg_scal, cg_sca, cg_vma;
+  /* final_update = false skips the closing update with gradients: the posterior draws (Draws) use the coefficients only */
+  DevBuf<double> cg_coeff, cg_grad, cg_m, cg_rm, cg_p, cg_q, cg_sds, cg_scal, cg_sca, cg_vma, cg_mean;
   DevBuf<unsigned> cg_running;
   std::vector<u64> cg_iters_cols;
-  bool optcg_device(double tol, u64 maxepch) {
+  bool optcg_device(double tol, u64 maxepch, bool final_update = true) {
     const bool mult = multi();
     auto* lk = dynamic_cast<DevLik*>(kid[0]);
     const bool lik_first = lk != nullptr;
@@ -2128,6 +2143,8 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     cg_rm.ensure(K * C); cg_p.ensure(K * C); cg_q.ensure(K * C);
     cg_scal.upload(scal, ctx.stream);
     if (percol) { cg_sca.upload(sca_cols, ctx.stream); cg_vma.upload(vma_cols, ctx.stream); }
+    const bool centred = prm && !prm->mean.empty();
+    if (centred) cg_mean.upload(prm->mean, ctx.stream);
     if (mult) cg_running.ensure(2);
     ctx.sync(); /* the host images above must outlive the uploads */
     obd::CgParams c{};
@@ -2137,6 +2154,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     lk->cg_params(c);
     if (mult) c.running = cg_running.p;
     if (percol) { c.sca_col = cg_sca.p; c.vma_col = cg_vma.p; }
+    if (centred) c.prior_mean = cg_mean.p;
     auto stage = [&](int st) { c.stage = st; c.red = lk->red.p; obd::launch_cg_stage(ctx, c, C); };
     stage(obd::CG_INIT);          /* rm = grad / m ; p = rm                       :58-60 */
     lk->hessmult_dev(cg_p.p);     /* q = hessmult(p), finished inside CG_STEP     :62 */
@@ -2163,6 +2181,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     ctx.sync();
     if (mult)
       for (u64 j = 0; j < C; ++j) cg_iters_cols[j] = scal[j * NS + obd::CG_STOP] != 0.0 ? (u64)scal[j * NS + obd::CG_ITER] : k;
+    if (!final_update) return true;
     compute_gradhyp = true; compute_gradpara = true;
     update(std::vector<double>(coeff));
     compute_gradhyp = false; compute_gradpara = false;
@@ -2299,6 +2318,94 @@ struct PredGda : Pred { /* loglik_gda.cpp:249-283 */
     std::vector<double> rv(ob->N);
     if (doda) ob->residvar(terms.data(), K, rv.data());
     for (u64 i = 0; i < ob->N; ++i) { out[i] += std::exp(2 * para[0]); if (doda) out[i] += std::exp(2 * para[1]) * rv[i]; }
+  }
+};
+
+/* ------------------------------------------------------------------ posterior draws (DESIGN §3.9)
+ * S joint draws of the coefficients of a fitted lpdfvec(logpr_gauss, loglik_gauss), conditional on its hyper-parameters,
+ * terms and para, by perturb-and-MAP: draw s solves
+ *   theta_s = argmax -|y + sigma eps_s - Phi theta|^2 / (2 sigma^2) - (theta - delta_s)^T D^-1 (theta - delta_s) / 2,
+ * eps_s ~ N(0, I_N), delta_s = coeffsd sca xi_s ~ N(0, D), so theta_s ~ N(mu, H^-1), H = Phi^T Phi / sigma^2 + D^-1, when
+ * solved exactly.  The S solves are the columns of lpdfvec(logpr_gauss_multi(S) centred at delta, loglik_gauss_multi(S) on
+ * the perturbed responses) without the marginal adjustment (it does not depend on theta), run by the column-batched
+ * device CG from the fitted coefficients.  The object copies the om and everything else it needs at creation. */
+struct Draws {
+  /* the fit's likelihood; refuses every other model */
+  static LoglikGauss& fitted_lik(Lpdf* fit) {
+    auto* v = dynamic_cast<LpdfVec*>(fit);
+    if (!v) throw std::invalid_argument("posterior draws need a fitted lpdfvec(logpr_gauss, loglik_gauss)");
+    if (v->multi() || v->para_per_column())
+      throw std::invalid_argument("posterior draws: multi-response and per-column-para fits are not supported");
+    for (Lpdf* k : v->kid) {
+      if (dynamic_cast<LoglikStd*>(k)) throw std::invalid_argument("posterior draws: loglik_std fits are not supported, only loglik_gauss");
+      if (dynamic_cast<LoglikGda*>(k)) throw std::invalid_argument("posterior draws: loglik_gda fits are not supported, only loglik_gauss");
+    }
+    auto* lik = dynamic_cast<LoglikGauss*>(v->kid[0]);
+    if (!lik) lik = dynamic_cast<LoglikGauss*>(v->kid[1]);
+    if (!lik || !dynamic_cast<LogprGauss*>(v->kid[lik == v->kid[0] ? 1 : 0]))
+      throw std::invalid_argument("posterior draws need a fitted lpdfvec(logpr_gauss, loglik_gauss)");
+    if (lik->ctx.nranks > 1) throw std::invalid_argument("posterior draws run on one rank only (the generator's row index is rank-local)");
+    return *lik;
+  }
+
+  Ctx& ctx;
+  OuterMod om; /* the fit's om at creation */
+  std::vector<u64> terms;
+  u64 N = 0, K = 0, S = 0, seed = 0;
+  std::vector<double> mu; /* the fit's coefficients, every column's start */
+  std::unique_ptr<LogprGaussMulti> pr;
+  std::unique_ptr<LoglikGaussMulti> lk;
+  std::unique_ptr<LpdfVec> vec; /* declared last: destroyed before the children it points to */
+  DevBuf<double> y0, sds, delta;
+  bool solved = false;
+
+  Draws(Lpdf* fit, u64 S_, u64 seed_) : ctx(fitted_lik(fit).ctx), om(*fitted_lik(fit).om), S(S_), seed(seed_) {
+    if (S == 0) throw std::invalid_argument("posterior draws: S must be at least 1");
+    LoglikGauss& fl = fitted_lik(fit);
+    auto* fv = static_cast<LpdfVec*>(fit);
+    const bool lik_first = fv->kid[0] == &fl;
+    const LogprGauss& fp = *static_cast<LogprGauss*>(fv->kid[lik_first ? 1 : 0]);
+    terms = fl.terms; N = fl.N; K = fl.K;
+    mu = fv->coeff.size() == K ? fv->coeff : std::vector<double>(K, 0.0);
+    std::vector<double> yh(N);
+    fl.ob.d2h(yh.data(), fl.y.p, N);
+    pr.reset(new LogprGaussMulti(&om, terms.data(), K, S));
+    pr->updatepara(fp.para.data(), fp.para.size());
+    lk.reset(new LoglikGaussMulti(ctx, &om, terms.data(), K, yh.data(), S, fl.x_host.data(), N, false, /*ybcast=*/true, /*dograd=*/false));
+    lk->updatepara(fl.para.data(), fl.para.size());
+    vec.reset(lik_first ? new LpdfVec(lk.get(), pr.get()) : new LpdfVec(pr.get(), lk.get()));
+    vec->domargadj = false;
+    const u64 ld = lk->ob.ld;
+    y0.ensure(ld);
+    OB_CUDA(cudaMemcpyAsync(y0.p, fl.y.p, ld * sizeof(double), cudaMemcpyDeviceToDevice, ctx.stream));
+    sds.upload(pr->one.coeffsd, ctx.stream);
+    delta.ensure(K * S);
+    obd::launch_draws_perturb(ctx, y0.p, N, ld, lk->obssd, sds.p, pr->one.sca, K, S, seed, lk->y.p, delta.p);
+    pr->mean.resize(K * S);
+    lk->ob.d2h(pr->mean.data(), delta.p, K * S);
+  }
+  void solve(double tol, u64 maxepch) {
+    vec->coeff.resize(K * S);
+    for (u64 s = 0; s < S; ++s) std::copy(mu.begin(), mu.end(), vec->coeff.begin() + s * K);
+    vec->fullhess = false;
+    vec->optcg_device(tol, maxepch, /*final_update=*/false);
+    solved = true;
+  }
+  const std::vector<double>& coeff() const {
+    if (!solved) throw std::logic_error("posterior draws: solve has not run");
+    return vec->coeff;
+  }
+  /* N x S perturbed responses */
+  std::vector<double> y() {
+    std::vector<double> o(N * S);
+    for (u64 s = 0; s < S; ++s) lk->ob.d2h(o.data() + s * N, lk->y.p + s * lk->ob.ld, N);
+    return o;
+  }
+  /* the draws of the latent function at new inputs (Nx x S): Phi(x) coeff, one product with S columns */
+  void predict(const double* x, u64 Nx, double* out) {
+    const std::vector<double>& a = coeff();
+    OuterBase ob(ctx, &om, x, Nx, false, terms.data(), K);
+    ob.mm_mat(0, terms.data(), K, a.data(), S, out);
   }
 };
 

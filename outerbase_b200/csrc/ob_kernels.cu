@@ -1436,6 +1436,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
   const int K = c.K, tid = threadIdx.x;
   const size_t off = (size_t)blockIdx.x * (size_t)K;
   c.coeff += off; c.grad += off; c.m += off; c.rm += off; c.p += off; c.q += off; c.red += off;
+  if (c.prior_mean) c.prior_mean += off;
   double* S = c.scal + (size_t)blockIdx.x * CG_NSCAL;
   if (c.running && S[CG_STOP] != 0.0) return;
   const double sca = c.sca_col ? c.sca_col[blockIdx.x] : c.sca;
@@ -1449,7 +1450,7 @@ __global__ void __launch_bounds__(kCgThreads) cg_stage_kernel(CgParams c) {
     double s1 = 0.0, s2 = 0.0;
     for (int i = tid; i < K; i += kCgThreads) {
       const double sd = c.sds[i] * sca;
-      const double st = c.coeff[i] / sd;
+      const double st = (c.prior_mean ? c.coeff[i] - c.prior_mean[i] : c.coeff[i]) / sd;
       s1 += st * st;
       s2 += log(sd);
       const double gpr = -1. * st / sd, glik = c.red[i];
@@ -1604,6 +1605,43 @@ void launch_rowdot(Ctx& c, const double* A, const double* B, u64 N, u64 K, u64 l
   if (N == 0) return;
   rowdot_kernel<<<(unsigned)((N + 255) / 256), 256, 0, c.stream>>>(A, B, N, K, ld, add, out);
   check_launch(c, "rowdot_kernel");
+}
+
+/* one thread per pair of rows (2t, 2t + 1) of column s, then one per pair of prior entries; the products are rounded
+ * before the add (no FMA), so y[i, s] - y0[i] is sigma eps as the host forms it */
+__global__ void draws_perturb_kernel(const double* __restrict__ y0, unsigned long long N, unsigned long long ld, double sigma,
+                                     const double* __restrict__ sds, double sca, unsigned long long K, unsigned s0,
+                                     unsigned long long seed, double* __restrict__ y, double* __restrict__ delta) {
+  const unsigned s = s0 + blockIdx.y;
+  const unsigned long long t = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x, rp = ld / 2;
+  double z[2];
+  if (t < rp) {
+    draw_normal_pair(seed, DRAW_ROWS, s, (uint32_t)t, z);
+    for (int j = 0; j < 2; ++j) {
+      const unsigned long long i = 2 * t + j;
+      y[i + s * ld] = i < N ? y0[i] + __dmul_rn(sigma, z[j]) : 0.0;
+    }
+  } else if (t < rp + (K + 1) / 2) {
+    const unsigned long long q = t - rp;
+    draw_normal_pair(seed, DRAW_PRIOR, s, (uint32_t)q, z);
+    for (int j = 0; j < 2; ++j) {
+      const unsigned long long k = 2 * q + j;
+      if (k < K) delta[k + s * K] = __dmul_rn(sds[k] * sca, z[j]);
+    }
+  }
+}
+void launch_draws_perturb(Ctx& c, const double* y0, u64 N, u64 ld, double sigma, const double* sds, double sca, u64 K, u64 S,
+                          uint64_t seed, double* y, double* delta) {
+  if (ld % 2 || ld / 2 > 0xFFFFFFFFull || (K + 1) / 2 > 0xFFFFFFFFull || S > 0xFFFFFFFFull)
+    throw std::range_error("posterior draws: the generator's index and column are 32-bit words");
+  const u64 n = ld / 2 + (K + 1) / 2;
+  if (n == 0) return;
+  for (u64 s0 = 0; s0 < S; s0 += 65535) {
+    const unsigned cols = (unsigned)std::min<u64>(65535, S - s0);
+    draws_perturb_kernel<<<dim3((unsigned)((n + 255) / 256), cols), 256, 0, c.stream>>>(y0, N, ld, sigma, sds, sca, K, (unsigned)s0,
+                                                                                       seed, y, delta);
+    check_launch(c, "draws_perturb_kernel");
+  }
 }
 
 void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd) {

@@ -18,6 +18,8 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
                                           stage1=True: obfit's two stages, stage 1 on loglik_gda_multi over one row
                                           subsample shared by the columns
   obpred        R/fitting.R:149-155
+  obdraws                                 S joint posterior draws of a fitted model at new inputs (no reference
+                                          counterpart)
 """
 from __future__ import annotations
 
@@ -25,7 +27,7 @@ import math
 
 import numpy as np
 
-from .binding import gethyp, getpara
+from .binding import gethyp, getpara, posterior_draws
 
 
 def _flatten(parlist):
@@ -422,3 +424,11 @@ def obpred(obmodel, x):
         return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(), var=var)
     return dict(mean=obmodel["y_cent"] + obmodel["y_sca"] * obmodel["predobj"].mean(),
                 var=obmodel["y_sca"] ** 2 * obmodel["predobj"].var())
+
+
+def obdraws(obmodel, x, S=64, seed=0, tol=0.001, maxepch=100):
+    """S joint posterior draws of the latent function at the rows of x (N x S, in y's units: y_cent + y_sca f) for a model
+    of obfit / obfit_gauss, conditional on its hyper-parameters, terms and para (posterior_draws: perturb-and-MAP, exact
+    at CG convergence; tol is the CG tolerance of the S solves).  Observation noise at x is not included."""
+    draws = posterior_draws(obmodel["logpdf"]._lib, obmodel["logpdf"], S, seed).solve(tol, maxepch)
+    return obmodel["y_cent"] + obmodel["y_sca"] * draws.predict(np.asfortranarray(np.asarray(x, dtype=float)))
