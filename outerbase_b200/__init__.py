@@ -23,6 +23,7 @@ MULTI_HEADER = REPO / "include" / "outerbase_b200_multi.h"  # the multi-response
 PERCOL_HEADER = REPO / "include" / "outerbase_b200_multi_percol.h"  # its per-column para variants
 MULTI_GDA_HEADER = REPO / "include" / "outerbase_b200_multi_gda.h"  # multi-response loglik_gda (two-stage fits)
 DRAWS_HEADER = REPO / "include" / "outerbase_b200_draws.h"  # posterior draws of a fitted model
+SOBOL_HEADER = REPO / "include" / "outerbase_b200_sobol.h"  # Sobol sensitivity indices of a fitted model
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -36,7 +37,7 @@ def _stale() -> bool:
     if not LIBPATH.exists():
         return True
     t = LIBPATH.stat().st_mtime
-    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER, DRAWS_HEADER]
+    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER, DRAWS_HEADER, SOBOL_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

@@ -930,6 +930,34 @@ class posterior_draws(_Handle):
         return out
 
 
+def sobol(lib, om, terms, coeff, x):
+    """Mean, variance, first-order and total-effect variances of f_b = sum_k coeff[k, b] Phi_k under the product of the
+    empirical marginals of x's columns (include/outerbase_b200_sobol.h).  coeff is a K-vector (mean and var are floats,
+    first and total have d entries) or K x B (mean and var have B entries, first and total are d x B).  The indices are
+    first / var and total / var."""
+    t = _terms(terms)
+    K, d = t.shape
+    if d != om.d:
+        raise ValueError(f"terms has {d} columns, the outermod {om.d} dimensions")
+    x = _f64(x)
+    if x.ndim != 2 or x.shape[1] != d:
+        raise ValueError("x must be nq x d")
+    c = _f64(coeff)
+    vec = c.ndim == 1
+    if vec:
+        c = c.reshape((-1, 1), order="F")
+    if c.ndim != 2 or c.shape[0] != K:
+        raise ValueError("coeff must have one row per term")
+    B = c.shape[1]
+    mean, var = np.empty(B), np.empty(B)
+    first, total = np.empty((d, B), order="F"), np.empty((d, B), order="F")
+    lib.call("sobol", lib.ctx, om._h, _p(t), _u(K), _p(c), _u(B), _p(x), _u(x.shape[0]), _p(mean), _p(var), _p(first),
+             _p(total))
+    if vec:
+        return dict(mean=float(mean[0]), var=float(var[0]), first=first[:, 0].copy(), total=total[:, 0].copy())
+    return dict(mean=mean, var=var, first=first, total=total)
+
+
 class predictor(_Handle):
     """new(predictor, loglik) -- src/fit.h:352-361."""
     _destroy = "predictor_destroy"

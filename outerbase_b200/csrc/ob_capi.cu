@@ -8,6 +8,7 @@
 #include "../../include/outerbase_b200_multi_percol.h"
 #include "../../include/outerbase_b200_multi_gda.h"
 #include "../../include/outerbase_b200_draws.h"
+#include "../../include/outerbase_b200_sobol.h"
 
 #include "ob_engine.hpp"
 
@@ -687,6 +688,18 @@ int ob_logpr_gauss_multi_set_mean(ob_lpdf* logpr, const double* mean, uint64_t n
   if (!m) throw std::invalid_argument("set_mean is a method of logpr_gauss_multi");
   if (n) need(mean, "mean");
   m->set_mean(mean, n);
+  OB_CATCH
+}
+
+/* ---- Sobol indices (include/outerbase_b200_sobol.h) */
+int ob_sobol(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* coeff, uint64_t B,
+             const double* xq, uint64_t nq, double* mean, double* var, double* first, double* total) {
+  OB_TRY
+  need(ctx, "ctx"); need(om, "om");
+  if (K) { need(terms, "terms"); if (B) need(coeff, "coeff"); }
+  if (nq) need(xq, "xq");
+  if (B) { need(mean, "mean"); need(var, "var"); need(first, "first"); need(total, "total"); }
+  obe::sobol(ctx->c, &om->om, terms, K, coeff, B, xq, nq, mean, var, first, total);
   OB_CATCH
 }
 

@@ -361,6 +361,27 @@ __host__ __device__ inline void draw_normal_pair(uint64_t seed, uint32_t stream,
 void launch_draws_perturb(Ctx& c, const double* y0, u64 N, u64 ld, double sigma, const double* sds, double sca, u64 K, u64 S,
                           uint64_t seed, double* y, double* delta);
 
+/* ---- Sobol sensitivity indices of a tensor-product model (DESIGN §3.10).  R_l(x, j) = basemat[x, col0 + j] scalemat[x, l]
+ * is the basis of dimension l at level j; the tables are its mean mu_l[j] and centred second moment C_l[j, j'] over the
+ * rows of X_q.  mu_l starts at mu_off of the mu table, C_l (mo x mo, column-major, symmetric) at c_off of the C table. */
+struct SobolDim { int col0, mo, mu_off, c_off; };
+constexpr int kSobolMomBlocks = 256; /* row slices of the moments kernel: partials per table entry */
+constexpr size_t kSobolStageBytes = 48 * 1024; /* the forms kernel stages the tables in shared memory up to this size */
+/* stage 0: musum[mu_off + j] = sum over the N rows of R_l(., j); stage 1: csum[c_off + j + mo j'] = sum of
+ * (R_l(., j) - mu[mu_off + j]) (R_l(., j') - mu[mu_off + j']).  Fixed row partition (kSobolMomBlocks slices of 32-row
+ * tiles), partials added in index order: the same bits on every run.  partial holds kSobolMomBlocks doubles per entry. */
+void launch_sobol_moments(Ctx& c, int stage, const double* basemat, const double* scalemat, u64 N, u64 ld,
+                          const std::vector<SobolDim>& dims, const SobolDim* dims_dev, const double* mu, double* partial,
+                          double* out);
+/* out[(b (2d + 1) + f)] for the B columns of coeff (K x B): f = 0 the variance form, 1 + l the first-order form of
+ * dimension l, 1 + d + l its total-effect form, each sum_{k <= k'} w theta_kb theta_k'b F_f(k, k') with w = 2 off the
+ * diagonal.  The pairs are cut into chunks and CTAs by K alone, so column b's result depends on nothing but column b
+ * and is the same bits on every run.  The tables (mu_n + c_n doubles) are staged in shared memory when they take at
+ * most kSobolStageBytes, read through the cache otherwise.  partial holds sobol_forms_partials(K) doubles per output. */
+u64 sobol_forms_partials(u64 K);
+void launch_sobol_forms(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                        const double* cov, u64 c_n, const double* coeff, u64 B, double* partial, double* out);
+
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {
   int kind; int m; int nh;

@@ -1644,6 +1644,212 @@ void launch_draws_perturb(Ctx& c, const double* y0, u64 N, u64 ld, double sigma,
   }
 }
 
+/* ---- Sobol indices (DESIGN §3.10) */
+constexpr int kSobolThreads = 256, kSobolRows = 32, kSobolTileLd = kSobolRows + 1; /* odd stride: no bank conflicts */
+
+/* grid (row slices, entry chunks of kSobolThreads, dimension).  Thread e of the chunk owns one table entry of the
+ * CTA's dimension and sums it over the CTA's 32-row tiles (t = blockIdx.x, + gridDim.x, ...) in row order; the tile of
+ * R_l (centred by the means in stage 1) is staged in shared memory.  R is rounded before the centring, as getbase
+ * forms it.  partial[entry * gridDim.x + blockIdx.x], entry = the output index of this stage. */
+__global__ void __launch_bounds__(kSobolThreads) sobol_moments_kernel(int stage, const double* __restrict__ basemat,
+                                                                      const double* __restrict__ scalemat, u64 N, u64 ld,
+                                                                      const SobolDim* __restrict__ dims,
+                                                                      const double* __restrict__ mu, double* __restrict__ partial) {
+  extern __shared__ double tile[]; /* mo x kSobolTileLd */
+  const SobolDim D = dims[blockIdx.z];
+  const int mo = D.mo, E = stage ? mo * mo : mo;
+  if ((int)blockIdx.y * kSobolThreads >= E) return; /* the whole CTA */
+  const int e = (int)blockIdx.y * kSobolThreads + (int)threadIdx.x;
+  const int j = e % mo, j2 = e / mo;
+  const double* scol = scalemat + (u64)blockIdx.z * ld;
+  const u64 ntiles = (N + kSobolRows - 1) / kSobolRows;
+  double acc = 0.0;
+  for (u64 t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    const u64 n0 = t * kSobolRows;
+    for (int i = threadIdx.x; i < mo * kSobolRows; i += kSobolThreads) {
+      const int r = i % kSobolRows, jj = i / kSobolRows;
+      const u64 n = n0 + r;
+      double v = 0.0;
+      if (n < N) {
+        v = __dmul_rn(basemat[n + (u64)(D.col0 + jj) * ld], scol[n]);
+        if (stage) v -= mu[D.mu_off + jj];
+      }
+      tile[jj * kSobolTileLd + r] = v;
+    }
+    __syncthreads();
+    if (e < E) {
+      const double* a = tile + j * kSobolTileLd;
+      if (stage) {
+        const double* b = tile + j2 * kSobolTileLd;
+#pragma unroll 8
+        for (int r = 0; r < kSobolRows; ++r) acc = fma(a[r], b[r], acc);
+      } else {
+#pragma unroll 8
+        for (int r = 0; r < kSobolRows; ++r) acc += a[r];
+      }
+    }
+    __syncthreads();
+  }
+  if (e < E) partial[(u64)((stage ? D.c_off : D.mu_off) + e) * gridDim.x + blockIdx.x] = acc;
+}
+
+void launch_sobol_moments(Ctx& c, int stage, const double* basemat, const double* scalemat, u64 N, u64 ld,
+                          const std::vector<SobolDim>& dims, const SobolDim* dims_dev, const double* mu, double* partial,
+                          double* out) {
+  int momax = 0;
+  u64 n_out = 0;
+  for (const SobolDim& D : dims) {
+    momax = std::max(momax, D.mo);
+    n_out += stage ? (u64)D.mo * D.mo : (u64)D.mo;
+  }
+  if (N == 0 || n_out == 0) return;
+  const u64 ntiles = (N + kSobolRows - 1) / kSobolRows;
+  const unsigned nb = (unsigned)std::min<u64>(ntiles, kSobolMomBlocks);
+  const u64 emax = stage ? (u64)momax * momax : (u64)momax;
+  const size_t smem = (size_t)momax * kSobolTileLd * sizeof(double);
+  set_smem(sobol_moments_kernel, smem);
+  sobol_moments_kernel<<<dim3(nb, (unsigned)((emax + kSobolThreads - 1) / kSobolThreads), (unsigned)dims.size()), kSobolThreads, smem,
+                         c.stream>>>(stage, basemat, scalemat, N, ld, dims_dev, mu, partial);
+  check_launch(c, "sobol_moments_kernel");
+  colsum_partials_kernel<<<(unsigned)n_out, 32, 0, c.stream>>>(partial, (int)nb, out);
+  check_launch(c, "colsum_partials_kernel");
+}
+
+/* pairs per chunk, columns per CTA (blockIdx.y), most CTAs over the pairs */
+constexpr int kSobolPairs = 128, kSobolCols = 32, kSobolFormBlocks = 1024;
+
+struct SobolFormsArgs {
+  const u64* terms; int K, d;
+  const SobolDim* dims;
+  const double* mu; const double* cov; int mu_n, c_n, staged;
+  const double* coeff; u64 B;
+  u64 npairs, nchunks;
+  double* partial;
+};
+
+/* pair q of the upper triangle in row-major order: row k holds (k, k .. K-1) and starts at k K - k (k - 1) / 2 */
+__device__ inline void sobol_pair(u64 q, u64 K, u64* k, u64* k2) {
+  auto start = [K](u64 r) { return r * K - r * (r - 1) / 2; };
+  const double b = 2.0 * (double)K + 1.0;
+  u64 r = (u64)fmax(0.0, floor((b - sqrt(fmax(0.0, b * b - 8.0 * (double)q))) * 0.5));
+  if (r >= K) r = K - 1;
+  while (r > 0 && start(r) > q) --r;
+  while (r + 1 < K && start(r + 1) <= q) ++r;
+  *k = r;
+  *k2 = r + (q - start(r));
+}
+
+/* grid (pair blocks, column blocks of kSobolCols).  Per chunk of kSobolPairs pairs: (A) thread p forms the 2d + 1 pair
+ * factors of its pair into F[p][.] -- prefix products of p_l and g_l on the way up, suffix products on the way down, so
+ * no division and no difference of products; (B) U[p][b] = w theta_kb theta_k'b; (C) output (f, b) adds
+ * F[p][f] U[p][b] over the chunk's pairs in order into acc (shared memory).  An output's sum runs over the same pairs
+ * in the same order whatever B is and whichever thread holds it. */
+__global__ void __launch_bounds__(kSobolThreads) sobol_forms_kernel(SobolFormsArgs a) {
+  extern __shared__ double sm[];
+  const int d = a.d, nf = 2 * d + 1;
+  const u64 K = (u64)a.K;
+  const u64 b0 = (u64)blockIdx.y * kSobolCols;
+  const int bc = a.B - b0 < (u64)kSobolCols ? (int)(a.B - b0) : kSobolCols;
+  double* F = sm;                          /* kSobolPairs x nf */
+  double* U = F + kSobolPairs * nf;        /* kSobolPairs x kSobolCols */
+  double* acc = U + kSobolPairs * kSobolCols; /* nf x kSobolCols */
+  const double* mu = a.mu;
+  const double* cov = a.cov;
+  if (a.staged) {
+    double* tab = acc + nf * kSobolCols;
+    for (int i = threadIdx.x; i < a.mu_n; i += kSobolThreads) tab[i] = a.mu[i];
+    for (int i = threadIdx.x; i < a.c_n; i += kSobolThreads) tab[a.mu_n + i] = a.cov[i];
+    mu = tab; cov = tab + a.mu_n;
+  }
+  for (int o = threadIdx.x; o < nf * bc; o += kSobolThreads) acc[o] = 0.0;
+  __syncthreads();
+  for (u64 ch = blockIdx.x; ch < a.nchunks; ch += gridDim.x) {
+    const u64 q0 = ch * kSobolPairs;
+    if (threadIdx.x < kSobolPairs) {
+      double* Fr = F + threadIdx.x * nf;
+      const u64 q = q0 + threadIdx.x;
+      if (q < a.npairs) {
+        u64 k, k2;
+        sobol_pair(q, K, &k, &k2);
+        double ppre = 1.0, gpre = 1.0;
+        for (int l = 0; l < d; ++l) {
+          const SobolDim D = a.dims[l];
+          const int t1 = (int)a.terms[k + l * K], t2 = (int)a.terms[k2 + l * K];
+          const double pl = mu[D.mu_off + t1] * mu[D.mu_off + t2], cl = cov[D.c_off + t1 + D.mo * t2];
+          Fr[1 + l] = ppre; Fr[1 + d + l] = gpre;
+          ppre *= pl; gpre *= cl + pl;
+        }
+        double psuf = 1.0, gsuf = 1.0, var = 0.0;
+        for (int l = d - 1; l >= 0; --l) {
+          const SobolDim D = a.dims[l];
+          const int t1 = (int)a.terms[k + l * K], t2 = (int)a.terms[k2 + l * K];
+          const double pl = mu[D.mu_off + t1] * mu[D.mu_off + t2], cl = cov[D.c_off + t1 + D.mo * t2];
+          var += Fr[1 + d + l] * cl * psuf;
+          Fr[1 + l] = cl * Fr[1 + l] * psuf;
+          Fr[1 + d + l] = cl * Fr[1 + d + l] * gsuf;
+          psuf *= pl; gsuf *= cl + pl;
+        }
+        Fr[0] = var;
+      } else {
+        for (int f = 0; f < nf; ++f) Fr[f] = 0.0;
+      }
+    }
+    for (int i = threadIdx.x; i < kSobolPairs * bc; i += kSobolThreads) {
+      const int p = i / bc, b = i % bc;
+      const u64 q = q0 + p;
+      double u = 0.0;
+      if (q < a.npairs) {
+        u64 k, k2;
+        sobol_pair(q, K, &k, &k2);
+        const double* th = a.coeff + (b0 + b) * K;
+        u = (k == k2 ? 1.0 : 2.0) * (th[k] * th[k2]);
+      }
+      U[p * kSobolCols + b] = u;
+    }
+    __syncthreads();
+    for (int o = threadIdx.x; o < nf * bc; o += kSobolThreads) {
+      const int f = o % nf, b = o / nf;
+      double s = acc[o];
+#pragma unroll 4
+      for (int p = 0; p < kSobolPairs; ++p) s = fma(F[p * nf + f], U[p * kSobolCols + b], s);
+      acc[o] = s;
+    }
+    __syncthreads();
+  }
+  for (int o = threadIdx.x; o < nf * bc; o += kSobolThreads) {
+    const int f = o % nf, b = o / nf;
+    a.partial[((b0 + b) * nf + f) * gridDim.x + blockIdx.x] = acc[o];
+  }
+}
+
+static u64 sobol_forms_chunks(u64 K) { return (K * (K + 1) / 2 + kSobolPairs - 1) / kSobolPairs; }
+u64 sobol_forms_partials(u64 K) { return std::max<u64>(1, std::min<u64>(sobol_forms_chunks(K), kSobolFormBlocks)); }
+
+void launch_sobol_forms(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                        const double* cov, u64 c_n, const double* coeff, u64 B, double* partial, double* out) {
+  if (K == 0 || B == 0) return;
+  if (K > 0x7FFFFFFFull) throw std::range_error("sobol: more terms than the forms kernel indexes");
+  const u64 nf = 2 * d + 1, ny = (B + kSobolCols - 1) / kSobolCols;
+  if (ny > 65535 || B * nf > 0x7FFFFFFFull) throw std::range_error("sobol: too many coefficient columns for one call");
+  SobolFormsArgs a{};
+  a.terms = terms; a.K = (int)K; a.d = (int)d; a.dims = dims_dev;
+  a.mu = mu; a.cov = cov; a.mu_n = (int)mu_n; a.c_n = (int)c_n;
+  a.coeff = coeff; a.B = B;
+  a.npairs = K * (K + 1) / 2; a.nchunks = sobol_forms_chunks(K);
+  a.partial = partial;
+  const size_t base = ((size_t)kSobolPairs * nf + (size_t)kSobolPairs * kSobolCols + nf * kSobolCols) * sizeof(double);
+  const size_t tab = (mu_n + c_n) * sizeof(double);
+  a.staged = tab <= kSobolStageBytes && base + tab <= c.smem_optin;
+  const size_t smem = base + (a.staged ? tab : 0);
+  if (smem > c.smem_optin) throw std::range_error("sobol: the model has more dimensions than the forms kernel holds");
+  const unsigned nblk = (unsigned)sobol_forms_partials(K);
+  set_smem(sobol_forms_kernel, smem);
+  sobol_forms_kernel<<<dim3(nblk, (unsigned)ny), kSobolThreads, smem, c.stream>>>(a);
+  check_launch(c, "sobol_forms_kernel");
+  colsum_partials_kernel<<<(unsigned)(B * nf), 32, 0, c.stream>>>(partial, (int)nblk, out);
+  check_launch(c, "colsum_partials_kernel");
+}
+
 void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd) {
   if (ld == 0) return;
   gda_obssd_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, c.stream>>>(phi2varc, N, ld, v0, v1, obssd);

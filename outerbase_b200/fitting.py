@@ -20,6 +20,8 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
   obpred        R/fitting.R:149-155
   obdraws                                 S joint posterior draws of a fitted model at new inputs (no reference
                                           counterpart)
+  obsobol                                 Sobol first-order and total indices of a fitted model, exact from its
+                                          coefficients, and of S posterior draws (no reference counterpart)
 """
 from __future__ import annotations
 
@@ -27,7 +29,7 @@ import math
 
 import numpy as np
 
-from .binding import gethyp, getpara, posterior_draws
+from .binding import gethyp, getpara, posterior_draws, sobol
 
 
 def _flatten(parlist):
@@ -432,3 +434,33 @@ def obdraws(obmodel, x, S=64, seed=0, tol=0.001, maxepch=100):
     at CG convergence; tol is the CG tolerance of the S solves).  Observation noise at x is not included."""
     draws = posterior_draws(obmodel["logpdf"]._lib, obmodel["logpdf"], S, seed).solve(tol, maxepch)
     return obmodel["y_cent"] + obmodel["y_sca"] * draws.predict(np.asfortranarray(np.asarray(x, dtype=float)))
+
+
+def _indices(r):
+    """first / var and total / var; a column whose variance is 0 gets NaN indices"""
+    var = np.asarray(r["var"], dtype=float)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        first = np.where(var != 0, r["first"] / np.where(var != 0, var, 1.0), np.nan)
+        total = np.where(var != 0, r["total"] / np.where(var != 0, var, 1.0), np.nan)
+    return first, total
+
+
+def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100):
+    """Sobol indices of the latent function of a model of obfit / obfit_gauss / obfit_multi under the product of the
+    empirical marginals of x's columns (binding.sobol: exact quadratic forms in the fitted coefficients).  Returns first and
+    total (the first-order and total indices, d or d x C), var (Var f in y's units, y_sca^2 var) and mean (y_cent +
+    y_sca E f).  S > 0 adds `draws`: the same four for each of S posterior draws (d x S, S), conditional on the
+    hyper-parameters, terms and para (posterior_draws; single-response models only)."""
+    logpdf = obmodel["logpdf"]
+    lib, om, terms = logpdf._lib, obmodel["om"], obmodel["terms"]
+    x = np.asfortranarray(np.asarray(x, dtype=float))
+    y_cent, y_sca = obmodel["y_cent"], obmodel["y_sca"]
+    r = sobol(lib, om, terms, logpdf.coeff, x)
+    first, total = _indices(r)
+    out = dict(first=first, total=total, var=y_sca ** 2 * r["var"], mean=y_cent + y_sca * r["mean"])
+    if S > 0:
+        draws = posterior_draws(lib, logpdf, S, seed).solve(tol, maxepch)
+        rd = sobol(lib, om, terms, draws.coeff, x)
+        fd, td = _indices(rd)
+        out["draws"] = dict(first=fd, total=td, var=y_sca ** 2 * rd["var"], mean=y_cent + y_sca * rd["mean"])
+    return out
