@@ -11,7 +11,7 @@ import subprocess
 from pathlib import Path
 
 from .binding import (Library, getpara, gethyp, header_symbols, loglik_gauss, loglik_gda, logpr_gauss, lpdf, lpdfvec,  # noqa: F401
-                      outerbase, outermod, predictor, setcovfs, setknot)
+                      outerbase, outermod, predictor, setcovfs, setknot, sobol, sobol_pairs)
 
 ROOT = Path(__file__).resolve().parent
 REPO = ROOT.parent
@@ -24,6 +24,7 @@ PERCOL_HEADER = REPO / "include" / "outerbase_b200_multi_percol.h"  # its per-co
 MULTI_GDA_HEADER = REPO / "include" / "outerbase_b200_multi_gda.h"  # multi-response loglik_gda (two-stage fits)
 DRAWS_HEADER = REPO / "include" / "outerbase_b200_draws.h"  # posterior draws of a fitted model
 SOBOL_HEADER = REPO / "include" / "outerbase_b200_sobol.h"  # Sobol sensitivity indices of a fitted model
+SOBOL_PAIRS_HEADER = REPO / "include" / "outerbase_b200_sobol_pairs.h"  # their second-order (input-pair) forms
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -37,7 +38,8 @@ def _stale() -> bool:
     if not LIBPATH.exists():
         return True
     t = LIBPATH.stat().st_mtime
-    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER, DRAWS_HEADER, SOBOL_HEADER]
+    deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER, DRAWS_HEADER, SOBOL_HEADER,
+                                   SOBOL_PAIRS_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

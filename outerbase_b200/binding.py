@@ -958,6 +958,41 @@ def sobol(lib, om, terms, coeff, x):
     return dict(mean=mean, var=var, first=first, total=total)
 
 
+def sobol_pairs(lib, om, terms, coeff, x):
+    """binding.sobol's four outputs (the same bits) and, for every input pair l < m, second (the pure second-order
+    variance sigma2_lm) and supset (Liu-Owen superset importance: the variance of every interaction that involves both)
+    (include/outerbase_b200_sobol_pairs.h).  second and supset are symmetric d x d for a K-vector coeff, d x d x B for a
+    K x B coeff, with NaN on the diagonal."""
+    t = _terms(terms)
+    K, d = t.shape
+    if d != om.d:
+        raise ValueError(f"terms has {d} columns, the outermod {om.d} dimensions")
+    x = _f64(x)
+    if x.ndim != 2 or x.shape[1] != d:
+        raise ValueError("x must be nq x d")
+    c = _f64(coeff)
+    vec = c.ndim == 1
+    if vec:
+        c = c.reshape((-1, 1), order="F")
+    if c.ndim != 2 or c.shape[0] != K:
+        raise ValueError("coeff must have one row per term")
+    B = c.shape[1]
+    P = d * (d - 1) // 2
+    mean, var = np.empty(B), np.empty(B)
+    first, total = np.empty((d, B), order="F"), np.empty((d, B), order="F")
+    second, supset = np.empty((max(P, 1), B), order="F"), np.empty((max(P, 1), B), order="F")
+    lib.call("sobol_pairs", lib.ctx, om._h, _p(t), _u(K), _p(c), _u(B), _p(x), _u(x.shape[0]), _p(mean), _p(var),
+             _p(first), _p(total), _p(second), _p(supset))
+    l, m = np.triu_indices(d, 1)  # row-major over l < m: row r of second / supset
+    S2, SU = np.full((d, d, B), np.nan), np.full((d, d, B), np.nan)
+    S2[l, m], S2[m, l] = second[:P], second[:P]
+    SU[l, m], SU[m, l] = supset[:P], supset[:P]
+    if vec:
+        return dict(mean=float(mean[0]), var=float(var[0]), first=first[:, 0].copy(), total=total[:, 0].copy(),
+                    second=S2[:, :, 0].copy(), supset=SU[:, :, 0].copy())
+    return dict(mean=mean, var=var, first=first, total=total, second=S2, supset=SU)
+
+
 class predictor(_Handle):
     """new(predictor, loglik) -- src/fit.h:352-361."""
     _destroy = "predictor_destroy"

@@ -9,6 +9,7 @@
 #include "../../include/outerbase_b200_multi_gda.h"
 #include "../../include/outerbase_b200_draws.h"
 #include "../../include/outerbase_b200_sobol.h"
+#include "../../include/outerbase_b200_sobol_pairs.h"
 
 #include "ob_engine.hpp"
 
@@ -700,6 +701,21 @@ int ob_sobol(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, co
   if (nq) need(xq, "xq");
   if (B) { need(mean, "mean"); need(var, "var"); need(first, "first"); need(total, "total"); }
   obe::sobol(ctx->c, &om->om, terms, K, coeff, B, xq, nq, mean, var, first, total);
+  OB_CATCH
+}
+
+int ob_sobol_pairs(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* coeff, uint64_t B,
+                   const double* xq, uint64_t nq, double* mean, double* var, double* first, double* total,
+                   double* second, double* supset) {
+  OB_TRY
+  need(ctx, "ctx"); need(om, "om");
+  if (K) { need(terms, "terms"); if (B) need(coeff, "coeff"); }
+  if (nq) need(xq, "xq");
+  if (B) {
+    need(mean, "mean"); need(var, "var"); need(first, "first"); need(total, "total");
+    if (om->om.d > 1) { need(second, "second"); need(supset, "supset"); }
+  }
+  obe::sobol_pairs(ctx->c, &om->om, terms, K, coeff, B, xq, nq, mean, var, first, total, second, supset);
   OB_CATCH
 }
 

@@ -381,6 +381,16 @@ void launch_sobol_moments(Ctx& c, int stage, const double* basemat, const double
 u64 sobol_forms_partials(u64 K);
 void launch_sobol_forms(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
                         const double* cov, u64 c_n, const double* coeff, u64 B, double* partial, double* out);
+/* Second-order forms (DESIGN §3.11), P = d (d - 1) / 2 input pairs (l, m), l < m, r = l d - l (l + 1) / 2 + m - l - 1:
+ * out[b 2P + 2 r] = sum_{k <= k'} w theta_kb theta_k'b c_l c_m prod_{j not in {l, m}} p_j (pure second-order variance)
+ * and out[b 2P + 2 r + 1] the same with g_j in the product (superset importance).  A GEMM over the term pairs on the
+ * FP64 tensor cores; the term-pair chunks and output blocks depend on K and d alone, so column b's result depends on
+ * nothing but column b and is the same bits on every run.  Nothing is launched when P = 0.  coeff_t holds the
+ * coefficients transposed (B x K column-major: the B columns of term k are adjacent).  partial holds
+ * sobol_pairs_partials(K, d) doubles per output. */
+u64 sobol_pairs_partials(u64 K, u64 d);
+void launch_sobol_pairs(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                        const double* cov, u64 c_n, const double* coeff_t, u64 B, double* partial, double* out);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

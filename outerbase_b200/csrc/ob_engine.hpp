@@ -2409,57 +2409,75 @@ struct Draws {
   }
 };
 
-/* ------------------------------------------------------------------ Sobol indices (DESIGN §3.10)
+/* ------------------------------------------------------------------ Sobol indices (DESIGN §3.10, §3.11)
  * f_b(x) = sum_k coeff[k, b] prod_l R_l(x_l, t_kl) under the product of the empirical marginals of X_q's columns:
  * mean[b], var[b], first[l + d b] = Var(E[f_b | x_l]) and total[l + d b] = E[Var(f_b | x_-l)], exact quadratic forms in
- * the coefficients built from the per-dimension tables mu_l and C_l (include/outerbase_b200_sobol.h).  X_q's basis is
- * built compact and without gradients, as Draws::predict builds its rows. */
-inline void sobol(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const double* coeff, u64 B, const double* xq,
-                  u64 nq, double* mean, double* var, double* first, double* total) {
+ * the coefficients built from the per-dimension tables mu_l and C_l (include/outerbase_b200_sobol.h); sobol_pairs adds
+ * the second-order forms of every input pair (include/outerbase_b200_sobol_pairs.h).  X_q's basis is built compact and
+ * without gradients, as Draws::predict builds its rows. */
+inline void sobol_check(const Ctx& ctx, u64 K, u64 B, u64 nq) {
   if (B == 0) throw std::invalid_argument("sobol: coeff must have at least one column");
   if (nq == 0) throw std::invalid_argument("sobol: X_q must have at least one row");
   if (K == 0) throw std::invalid_argument("sobol: the terms table is empty");
   if (ctx.nranks > 1)
     throw std::invalid_argument("sobol runs on one rank only (X_q's rows would be rank-local, so each rank would measure other marginals)");
-  OuterBase ob(ctx, om, xq, nq, /*dograd=*/false, terms, K);
-  ob.check_terms(terms, K);
-  const u64 d = ob.d;
-  std::vector<obd::SobolDim> dims(d);
-  u64 mu_n = 0, c_n = 0;
-  for (u64 l = 0; l < d; ++l) {
-    u64 mx = 0;
-    for (u64 k = 0; k < K; ++k) mx = std::max(mx, terms[k + l * K]);
-    dims[l] = obd::SobolDim{(int)ob.cst[l], (int)(mx + 1), (int)mu_n, (int)c_n};
-    mu_n += mx + 1;
-    c_n += (mx + 1) * (mx + 1);
-  }
+}
+
+/* The basis of X_q, the means and the centred moments on the device, the terms and the coefficients uploaded: what
+ * the forms kernels read. */
+struct SobolTables {
+  OuterBase ob;
+  u64 d = 0, mu_n = 0, c_n = 0;
+  std::vector<obd::SobolDim> dims;
+  std::vector<double> mu;
   DevBuf<obd::SobolDim> dims_dev;
-  DevBuf<double> part, mu_dev, c_dev, coeff_dev, out_dev;
+  DevBuf<double> part, mu_dev, c_dev, coeff_dev;
   DevBuf<u64> terms_dev;
-  dims_dev.upload(dims, ctx.stream);
-  part.ensure(std::max(c_n * obd::kSobolMomBlocks, B * (2 * d + 1) * obd::sobol_forms_partials(K)));
-  mu_dev.ensure(mu_n); c_dev.ensure(c_n);
-  /* the means first, then the moments centred at them: no E[R R'] - mu mu' */
-  obd::launch_sobol_moments(ctx, 0, ob.basemat.p, ob.scalemat.p, nq, ob.ld, dims, dims_dev.p, nullptr, part.p, mu_dev.p);
-  std::vector<double> mu(mu_n);
-  ob.d2h(mu.data(), mu_dev.p, mu_n);
-  for (double& v : mu) v /= double(nq);
-  mu_dev.upload(mu, ctx.stream);
-  obd::launch_sobol_moments(ctx, 1, ob.basemat.p, ob.scalemat.p, nq, ob.ld, dims, dims_dev.p, mu_dev.p, part.p, c_dev.p);
-  std::vector<double> cv(c_n);
-  ob.d2h(cv.data(), c_dev.p, c_n);
-  for (double& v : cv) v /= double(nq);
-  c_dev.upload(cv, ctx.stream);
-  terms_dev.upload(terms, K * d, ctx.stream);
-  coeff_dev.upload(coeff, K * B, ctx.stream);
+  SobolTables(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const double* coeff, u64 B, const double* xq, u64 nq)
+      : ob(ctx, om, xq, nq, /*dograd=*/false, terms, K) {
+    ob.check_terms(terms, K);
+    d = ob.d;
+    dims.resize(d);
+    for (u64 l = 0; l < d; ++l) {
+      u64 mx = 0;
+      for (u64 k = 0; k < K; ++k) mx = std::max(mx, terms[k + l * K]);
+      dims[l] = obd::SobolDim{(int)ob.cst[l], (int)(mx + 1), (int)mu_n, (int)c_n};
+      mu_n += mx + 1;
+      c_n += (mx + 1) * (mx + 1);
+    }
+    dims_dev.upload(dims, ctx.stream);
+    part.ensure(std::max(c_n * obd::kSobolMomBlocks, B * (2 * d + 1) * obd::sobol_forms_partials(K)));
+    mu_dev.ensure(mu_n); c_dev.ensure(c_n);
+    /* the means first, then the moments centred at them: no E[R R'] - mu mu' */
+    obd::launch_sobol_moments(ctx, 0, ob.basemat.p, ob.scalemat.p, nq, ob.ld, dims, dims_dev.p, nullptr, part.p, mu_dev.p);
+    mu.resize(mu_n);
+    ob.d2h(mu.data(), mu_dev.p, mu_n);
+    for (double& v : mu) v /= double(nq);
+    mu_dev.upload(mu, ctx.stream);
+    obd::launch_sobol_moments(ctx, 1, ob.basemat.p, ob.scalemat.p, nq, ob.ld, dims, dims_dev.p, mu_dev.p, part.p, c_dev.p);
+    std::vector<double> cv(c_n);
+    ob.d2h(cv.data(), c_dev.p, c_n);
+    for (double& v : cv) v /= double(nq);
+    c_dev.upload(cv, ctx.stream);
+    terms_dev.upload(terms, K * d, ctx.stream);
+    coeff_dev.upload(coeff, K * B, ctx.stream);
+  }
+};
+
+/* mean, var, first and total from the tables */
+inline void sobol_forms(Ctx& ctx, SobolTables& T, const u64* terms, u64 K, const double* coeff, u64 B, double* mean,
+                        double* var, double* first, double* total) {
+  const u64 d = T.d;
+  DevBuf<double> out_dev;
   out_dev.ensure(B * (2 * d + 1));
-  obd::launch_sobol_forms(ctx, terms_dev.p, K, d, dims_dev.p, mu_dev.p, mu_n, c_dev.p, c_n, coeff_dev.p, B, part.p, out_dev.p);
+  obd::launch_sobol_forms(ctx, T.terms_dev.p, K, d, T.dims_dev.p, T.mu_dev.p, T.mu_n, T.c_dev.p, T.c_n, T.coeff_dev.p, B,
+                          T.part.p, out_dev.p);
   std::vector<double> out(B * (2 * d + 1));
-  ob.d2h(out.data(), out_dev.p, out.size());
+  T.ob.d2h(out.data(), out_dev.p, out.size());
   /* the mean is O(K d B): on the host, from the same table */
   std::vector<double> pm(K, 1.0);
   for (u64 k = 0; k < K; ++k)
-    for (u64 l = 0; l < d; ++l) pm[k] *= mu[dims[l].mu_off + terms[k + l * K]];
+    for (u64 l = 0; l < d; ++l) pm[k] *= T.mu[T.dims[l].mu_off + terms[k + l * K]];
   for (u64 b = 0; b < B; ++b) {
     double s = 0.0;
     for (u64 k = 0; k < K; ++k) s += coeff[k + b * K] * pm[k];
@@ -2469,6 +2487,42 @@ inline void sobol(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const d
     std::copy(o + 1, o + 1 + d, first + b * d);
     std::copy(o + 1 + d, o + 1 + 2 * d, total + b * d);
   }
+}
+
+inline void sobol(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const double* coeff, u64 B, const double* xq,
+                  u64 nq, double* mean, double* var, double* first, double* total) {
+  sobol_check(ctx, K, B, nq);
+  SobolTables T(ctx, om, terms, K, coeff, B, xq, nq);
+  sobol_forms(ctx, T, terms, K, coeff, B, mean, var, first, total);
+}
+
+/* sobol's four outputs (the same bits: the same tables and forms launches) and, P = d (d - 1) / 2, second[r + P b]
+ * and supset[r + P b] of input pair r = (l, m), l < m, r = l d - l (l + 1) / 2 + m - l - 1 (DESIGN §3.11) */
+inline void sobol_pairs(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const double* coeff, u64 B,
+                        const double* xq, u64 nq, double* mean, double* var, double* first, double* total,
+                        double* second, double* supset) {
+  sobol_check(ctx, K, B, nq);
+  SobolTables T(ctx, om, terms, K, coeff, B, xq, nq);
+  sobol_forms(ctx, T, terms, K, coeff, B, mean, var, first, total);
+  const u64 d = T.d, P = d * (d - 1) / 2;
+  if (P == 0) return;
+  /* the pair kernel reads the B columns of a term together */
+  std::vector<double> ct(K * B);
+  for (u64 b = 0; b < B; ++b)
+    for (u64 k = 0; k < K; ++k) ct[b + B * k] = coeff[k + K * b];
+  DevBuf<double> part, out_dev, coeff_t;
+  coeff_t.upload(ct, ctx.stream);
+  part.ensure(B * 2 * P * obd::sobol_pairs_partials(K, d));
+  out_dev.ensure(B * 2 * P);
+  obd::launch_sobol_pairs(ctx, T.terms_dev.p, K, d, T.dims_dev.p, T.mu_dev.p, T.mu_n, T.c_dev.p, T.c_n, coeff_t.p, B,
+                          part.p, out_dev.p);
+  std::vector<double> out(B * 2 * P);
+  T.ob.d2h(out.data(), out_dev.p, out.size());
+  for (u64 b = 0; b < B; ++b)
+    for (u64 r = 0; r < P; ++r) {
+      second[r + P * b] = out[b * 2 * P + 2 * r];
+      supset[r + P * b] = out[b * 2 * P + 2 * r + 1];
+    }
 }
 
 } // namespace obe

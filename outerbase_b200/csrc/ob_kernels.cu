@@ -1850,6 +1850,232 @@ void launch_sobol_forms(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* 
   check_launch(c, "colsum_partials_kernel");
 }
 
+/* ---- second-order Sobol forms on the FP64 tensor cores (DESIGN §3.11).  out(f, b) = sum_q F[q, f] U[q, b] over the
+ * term pairs q = (k <= k'): a GEMM with the term pairs as the contraction dimension, F formed per chunk in shared
+ * memory and never stored in HBM.  A CTA owns an output block of kPairsMP input pairs (l, m) (2 kPairsMP factor rows:
+ * second and supset) and kPairsCols columns, and walks the term-pair chunks ch = blockIdx.x, + gridDim.x, ... */
+constexpr int kPairsQ = 16;                       /* term pairs per chunk: 4 k-steps of m8n8k4 */
+constexpr int kPairsMP = 64, kPairsRows = 2 * kPairsMP, kPairsCols = 64;
+constexpr int kPairsFS = kPairsRows + 4, kPairsUS = kPairsCols + 4; /* = 4 mod 16 doubles: see the fragment loads */
+constexpr int kPairsCTAs = 592;                   /* CTAs over (chunks x output blocks): two waves of 2 per SM */
+constexpr int kPairsVec = 7;                      /* per term pair and dimension: c, p, g, prefix p, prefix g, suffix p, suffix g */
+
+/* grid (chunk CTAs, output blocks, column blocks), 256 threads.  Per chunk of kPairsQ term pairs:
+ *   (A) c_j, p_j, g_j of every term pair and dimension;
+ *   (B) four scans per term pair: prefix products of p and g on the way up, suffix products on the way down; beside
+ *       them U[q][b] = w theta_kb theta_k'b (w = 2 off the diagonal), from a.coeff = the coefficients transposed (B x K);
+ *   (C) thread (q, h) forms the factors of input pairs 4h .. 4h+3 of the block: c_l c_m (pre_l mid_lm) suf_m for p
+ *       (second) and for g (supset), mid_lm = prod_{l<j<m} in ascending order, grown as m advances, so a factor is
+ *       the same bits whichever thread forms it and no division or difference of products appears.  Pair i = 4h + j
+ *       goes to tile row s kPairsMP + 16 j + h (s = 0 second, 1 supset): a store instruction writes 16 consecutive
+ *       doubles per term pair;
+ *   (D) warp w contracts tile rows 16w .. 16w+15 against the column tiles holding live columns: per k-step two A and
+ *       up to eight B fragments, two DMMAs per column tile.  Lane (g, k4) loads row k4 of a fragment at offset
+ *       k4 * stride + g; with strides of 4 mod 16 doubles the 16 lanes of a half-warp hit 16 different banks, the
+ *       minimum two wavefronts per load.
+ * Each D element depends on its own A row and B column only, the chunks follow in the same order whatever B is, so
+ * column b's result does not depend on the other columns.  The CTA's sum goes to partial[o * gridDim.x + blockIdx.x],
+ * o = b 2P + 2 r + s, added in index order by colsum_partials_kernel. */
+__global__ void __launch_bounds__(kSobolThreads) sobol_pairs_kernel(SobolFormsArgs a) {
+  extern __shared__ double sm[];
+  const int d = a.d, P = d * (d - 1) / 2;
+  const u64 K = (u64)a.K;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, k4 = lane & 3;
+  const u64 b0 = (u64)blockIdx.z * kPairsCols;
+  const int bc = a.B - b0 < (u64)kPairsCols ? (int)(a.B - b0) : kPairsCols;
+  const int ntc = (bc + 7) / 8;
+  const int r0 = (int)blockIdx.y * kPairsMP;
+  double* F = sm;                                   /* kPairsQ x kPairsFS */
+  double* U = F + kPairsQ * kPairsFS;               /* kPairsQ x kPairsUS */
+  double* V = U + kPairsQ * kPairsUS;               /* kPairsQ x kPairsVec d */
+  int* kq = reinterpret_cast<int*>(V + kPairsQ * kPairsVec * d); /* kPairsQ x 2: k, k' (-1: past the last pair) */
+  const double* mu = a.mu;
+  const double* cov = a.cov;
+  if (a.staged) {
+    double* tab = V + kPairsQ * kPairsVec * d + kPairsQ; /* kq takes kPairsQ doubles */
+    for (int i = tid; i < a.mu_n; i += kSobolThreads) tab[i] = a.mu[i];
+    for (int i = tid; i < a.c_n; i += kSobolThreads) tab[a.mu_n + i] = a.cov[i];
+    mu = tab; cov = tab + a.mu_n;
+  }
+  /* this thread's first input pair (l0, m0) in phase C; nv of its four are in the block */
+  const int qc = tid >> 4, h = tid & 15;
+  const int rs = r0 + 4 * h, nv = P - rs < 4 ? P - rs : 4;
+  int l0 = 0, m0 = 1;
+  for (int l = 0, r = rs; l < d - 1 && nv > 0; ++l) {
+    if (r < d - 1 - l) { l0 = l; m0 = l + 1 + r; break; }
+    r -= d - 1 - l;
+  }
+  double acc[2][kPairsCols / 8][2];
+#pragma unroll
+  for (int t = 0; t < 2; ++t)
+#pragma unroll
+    for (int n = 0; n < kPairsCols / 8; ++n) acc[t][n][0] = acc[t][n][1] = 0.0;
+
+  /* k and k' of the term pairs of chunk ch (-1 past the last pair or chunk) */
+  auto phase_kq = [&](u64 ch) {
+    if (tid < kPairsQ) {
+      const u64 q = ch * kPairsQ + tid;
+      int k = -1, k2 = -1;
+      if (ch < a.nchunks && q < a.npairs) {
+        u64 kk, kk2;
+        sobol_pair(q, K, &kk, &kk2);
+        k = (int)kk; k2 = (int)kk2;
+      }
+      kq[2 * tid] = k; kq[2 * tid + 1] = k2;
+    }
+  };
+  /* (A) */
+  auto phase_a = [&]() {
+    for (int i = tid; i < kPairsQ * d; i += kSobolThreads) {
+      const int q = i / d, l = i % d;
+      const int k = kq[2 * q], k2 = kq[2 * q + 1];
+      double cl = 0.0, pl = 0.0;
+      if (k >= 0) {
+        const SobolDim D = a.dims[l];
+        const int t1 = (int)a.terms[k + l * K], t2 = (int)a.terms[k2 + l * K];
+        pl = mu[D.mu_off + t1] * mu[D.mu_off + t2];
+        cl = cov[D.c_off + t1 + D.mo * t2];
+      }
+      double* Vq = V + q * kPairsVec * d;
+      Vq[l] = cl; Vq[d + l] = pl; Vq[2 * d + l] = cl + pl;
+    }
+  };
+  /* (B) warps 0-1; warps 2-7 write U from the transposed coefficients (row k holds the B columns: coalesced) */
+  auto phase_b = [&]() {
+    if (tid < 4 * kPairsQ) {
+      const int q = tid >> 2, kind = tid & 3;
+      double* Vq = V + q * kPairsVec * d;
+      const double* src = Vq + ((kind & 1) ? 2 * d : d);
+      double* dst = Vq + (3 + kind) * d;
+      double x = 1.0;
+      if (kind < 2) {
+        for (int l = 0; l < d; ++l) { dst[l] = x; x *= src[l]; }
+      } else {
+        for (int l = d - 1; l >= 0; --l) { dst[l] = x; x *= src[l]; }
+      }
+    } else {
+      for (int i = tid - 4 * kPairsQ; i < kPairsQ * kPairsCols; i += kSobolThreads - 4 * kPairsQ) {
+        const int q = i / kPairsCols, b = i % kPairsCols;
+        const int k = kq[2 * q], k2 = kq[2 * q + 1];
+        double u = 0.0;
+        if (k >= 0 && b < bc) u = (k == k2 ? 1.0 : 2.0) * (a.coeff[(u64)k * a.B + b0 + b] * a.coeff[(u64)k2 * a.B + b0 + b]);
+        U[q * kPairsUS + b] = u;
+      }
+    }
+  };
+  /* (C) */
+  auto phase_c = [&]() {
+    const double* c = V + qc * kPairsVec * d;
+    const double *p = c + d, *gg = c + 2 * d, *pp = c + 3 * d, *pg = c + 4 * d, *sp = c + 5 * d, *sg = c + 6 * d;
+    double* Fq = F + qc * kPairsFS;
+    int l = l0, m = m0;
+    double mp = 1.0, mg = 1.0;
+    if (nv > 0)
+      for (int j = l + 1; j < m; ++j) { mp *= p[j]; mg *= gg[j]; }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      double fs = 0.0, fu = 0.0;
+      if (j < nv) {
+        const double cc = c[l] * c[m];
+        fs = cc * ((pp[l] * mp) * sp[m]);
+        fu = cc * ((pg[l] * mg) * sg[m]);
+        if (m + 1 < d) { mp *= p[m]; mg *= gg[m]; ++m; }
+        else { ++l; m = l + 1; mp = 1.0; mg = 1.0; }
+      }
+      Fq[16 * j + h] = fs;
+      Fq[kPairsMP + 16 * j + h] = fu;
+    }
+  };
+  /* (D) */
+  auto phase_d = [&]() {
+#pragma unroll
+    for (int ks = 0; ks < kPairsQ / 4; ++ks) {
+      const double* Fk = F + (ks * 4 + k4) * kPairsFS + warp * 16 + g;
+      const double* Uk = U + (ks * 4 + k4) * kPairsUS + g;
+      const double a0 = Fk[0], a1 = Fk[8];
+#pragma unroll
+      for (int n = 0; n < kPairsCols / 8; ++n) {
+        if (n < ntc) {
+          const double bv = Uk[n * 8];
+          dmma_f64(acc[0][n][0], acc[0][n][1], a0, bv);
+          dmma_f64(acc[1][n][0], acc[1][n][1], a1, bv);
+        }
+      }
+    }
+  };
+
+  /* software pipeline, three barriers per chunk: the DMMAs of chunk ch run beside (A) of the next chunk, which reads
+   * the tables through the cache and writes V only; (B) and (C) of the next chunk follow once F and U are consumed */
+  const u64 G = gridDim.x;
+  phase_kq(blockIdx.x);
+  __syncthreads(); /* and the staged tables are visible */
+  phase_a();
+  __syncthreads();
+  phase_b();
+  __syncthreads();
+  phase_c();
+  phase_kq(blockIdx.x + G);
+  __syncthreads();
+  for (u64 ch = blockIdx.x; ch < a.nchunks; ch += G) {
+    phase_d();
+    phase_a();
+    __syncthreads();
+    phase_b();
+    __syncthreads();
+    phase_c();
+    phase_kq(ch + 2 * G);
+    __syncthreads();
+  }
+  /* C fragment: lane (g, k4) holds rows 16 warp + 8 t + g, columns 8 n + 2 k4 + e */
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {
+    const int row = warp * 16 + t * 8 + g;
+    const int s = row / kPairsMP, jj = (row % kPairsMP) >> 4, hh = row & 15;
+    const int r = r0 + 4 * hh + jj;
+    if (r >= P) continue;
+#pragma unroll
+    for (int n = 0; n < kPairsCols / 8; ++n)
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        const int b = n * 8 + 2 * k4 + e;
+        if (b < bc) a.partial[(((b0 + b) * (u64)(2 * P) + 2 * r + s) * gridDim.x) + blockIdx.x] = acc[t][n][e];
+      }
+  }
+}
+
+static u64 sobol_pairs_chunks(u64 K) { return (K * (K + 1) / 2 + kPairsQ - 1) / kPairsQ; }
+static u64 sobol_pairs_blocks(u64 d) { return (d * (d - 1) / 2 + kPairsMP - 1) / kPairsMP; }
+u64 sobol_pairs_partials(u64 K, u64 d) {
+  const u64 ny = std::max<u64>(1, sobol_pairs_blocks(d));
+  return std::max<u64>(1, std::min<u64>(sobol_pairs_chunks(K), std::max<u64>(1, kPairsCTAs / ny)));
+}
+
+void launch_sobol_pairs(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                        const double* cov, u64 c_n, const double* coeff_t, u64 B, double* partial, double* out) {
+  const u64 P = d * (d - 1) / 2;
+  if (K == 0 || B == 0 || P == 0) return;
+  if (K > 0x7FFFFFFFull) throw std::range_error("sobol_pairs: more terms than the pair kernel indexes");
+  const u64 nz = (B + kPairsCols - 1) / kPairsCols;
+  if (nz > 65535 || B * 2 * P > 0x7FFFFFFFull) throw std::range_error("sobol_pairs: too many coefficient columns for one call");
+  SobolFormsArgs a{};
+  a.terms = terms; a.K = (int)K; a.d = (int)d; a.dims = dims_dev;
+  a.mu = mu; a.cov = cov; a.mu_n = (int)mu_n; a.c_n = (int)c_n;
+  a.coeff = coeff_t; a.B = B;
+  a.npairs = K * (K + 1) / 2; a.nchunks = sobol_pairs_chunks(K);
+  a.partial = partial;
+  const size_t base = ((size_t)kPairsQ * (kPairsFS + kPairsUS + kPairsVec * d) + kPairsQ) * sizeof(double);
+  const size_t tab = (mu_n + c_n) * sizeof(double);
+  a.staged = tab <= kSobolStageBytes && base + tab <= c.smem_optin;
+  const size_t smem = base + (a.staged ? tab : 0);
+  if (smem > c.smem_optin) throw std::range_error("sobol_pairs: the model has more dimensions than the pair kernel holds");
+  const unsigned nx = (unsigned)sobol_pairs_partials(K, d), ny = (unsigned)sobol_pairs_blocks(d);
+  set_smem(sobol_pairs_kernel, smem);
+  sobol_pairs_kernel<<<dim3(nx, ny, (unsigned)nz), kSobolThreads, smem, c.stream>>>(a);
+  check_launch(c, "sobol_pairs_kernel");
+  colsum_partials_kernel<<<(unsigned)(B * 2 * P), 32, 0, c.stream>>>(partial, (int)nx, out);
+  check_launch(c, "colsum_partials_kernel");
+}
+
 void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd) {
   if (ld == 0) return;
   gda_obssd_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, c.stream>>>(phi2varc, N, ld, v0, v1, obssd);

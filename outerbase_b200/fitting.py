@@ -21,7 +21,8 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
   obdraws                                 S joint posterior draws of a fitted model at new inputs (no reference
                                           counterpart)
   obsobol                                 Sobol first-order and total indices of a fitted model, exact from its
-                                          coefficients, and of S posterior draws (no reference counterpart)
+                                          coefficients, optionally the second-order indices of every input pair, and
+                                          of S posterior draws (no reference counterpart)
 """
 from __future__ import annotations
 
@@ -29,7 +30,7 @@ import math
 
 import numpy as np
 
-from .binding import gethyp, getpara, posterior_draws, sobol
+from .binding import gethyp, getpara, posterior_draws, sobol, sobol_pairs
 
 
 def _flatten(parlist):
@@ -445,22 +446,41 @@ def _indices(r):
     return first, total
 
 
-def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100):
+def _pair_indices(r):
+    """second / var, closed = (first_l + first_m + second_lm) / var and supset / var (d x d or d x d x B, NaN on the
+    diagonal); a column whose variance is 0 gets NaN indices"""
+    var = np.asarray(r["var"], dtype=float)
+    f = np.asarray(r["first"], dtype=float)
+    closed = f[:, None] + f[None, :] + r["second"]
+    den = np.where(var != 0, var, 1.0)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return {k: np.where(var != 0, v / den, np.nan) for k, v in (("second", r["second"]), ("closed", closed),
+                                                                    ("supset", r["supset"]))}
+
+
+def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100, second=False):
     """Sobol indices of the latent function of a model of obfit / obfit_gauss / obfit_multi under the product of the
     empirical marginals of x's columns (binding.sobol: exact quadratic forms in the fitted coefficients).  Returns first and
     total (the first-order and total indices, d or d x C), var (Var f in y's units, y_sca^2 var) and mean (y_cent +
-    y_sca E f).  S > 0 adds `draws`: the same four for each of S posterior draws (d x S, S), conditional on the
+    y_sca E f).  second=True adds, from binding.sobol_pairs, the input-pair indices second (pure second-order), closed
+    (first_l + first_m + second_lm) and supset (superset importance), each d x d or d x d x C with NaN on the diagonal.
+    S > 0 adds `draws`: the same keys for each of S posterior draws (d x S, d x d x S, S), conditional on the
     hyper-parameters, terms and para (posterior_draws; single-response models only)."""
     logpdf = obmodel["logpdf"]
     lib, om, terms = logpdf._lib, obmodel["om"], obmodel["terms"]
     x = np.asfortranarray(np.asarray(x, dtype=float))
     y_cent, y_sca = obmodel["y_cent"], obmodel["y_sca"]
-    r = sobol(lib, om, terms, logpdf.coeff, x)
-    first, total = _indices(r)
-    out = dict(first=first, total=total, var=y_sca ** 2 * r["var"], mean=y_cent + y_sca * r["mean"])
+    forms = sobol_pairs if second else sobol
+
+    def indices(coeff):
+        r = forms(lib, om, terms, coeff, x)
+        first, total = _indices(r)
+        out = dict(first=first, total=total, var=y_sca ** 2 * r["var"], mean=y_cent + y_sca * r["mean"])
+        if second:
+            out.update(_pair_indices(r))
+        return out
+
+    out = indices(logpdf.coeff)
     if S > 0:
-        draws = posterior_draws(lib, logpdf, S, seed).solve(tol, maxepch)
-        rd = sobol(lib, om, terms, draws.coeff, x)
-        fd, td = _indices(rd)
-        out["draws"] = dict(first=fd, total=td, var=y_sca ** 2 * rd["var"], mean=y_cent + y_sca * rd["mean"])
+        out["draws"] = indices(posterior_draws(lib, logpdf, S, seed).solve(tol, maxepch).coeff)
     return out
