@@ -286,12 +286,22 @@ extern "C" void run_d(const double* tile, const double* as_, const double* gmat,
 """
 
 
-@pytest.mark.parametrize("K,d,unused_dim,nh", [(160, 8, False, 2), (160, 8, True, 2), (160, 8, False, 1), (160, 8, True, 3), (2000, 10, False, 2)])
-def test_generated_hyper_gradient_sweep(product_symbols, tmp_path, K, d, unused_dim, nh):
+_SWEEP_CASES = [(160, 8, False, 2, True), (160, 8, True, 2, True), (160, 8, False, 1, True), (160, 8, True, 3, True),
+                (2000, 10, False, 2, True), (120, 32, False, 2, True), (160, 8, False, 2, False)]
+
+
+@pytest.mark.parametrize("K,d,unused_dim,nh,root", _SWEEP_CASES,
+                         ids=["-".join(map(str, c[:4])) + ("" if c[4] else "-rootless") for c in _SWEEP_CASES])
+def test_generated_hyper_gradient_sweep(product_symbols, tmp_path, K, d, unused_dim, nh, root):
     """phi_d_spec's generated body + epilogue macros (lifted to host C++) against the definition of prodmmge_'s outge
     (src/linalg.cpp:139-163, 273-276) for one row, plain and squared (basematsq_gradhyp = 2 G % B, modandbase.cpp:588-590);
-    the last case has the size of BASELINE config C3's table."""
+    2000 x 10 has the size of BASELINE config C3's table, 32 dimensions with two hyper-parameters each fill DotParams'
+    fixed arrays (hst[33], gest[65], kst[33]) to the last entry, and `root = False` drops the constant term."""
     terms, rng = _terms(product_symbols, K, d)
+    if not root:
+        assert not terms[0].any()
+        terms = np.asfortranarray(terms[1:])
+        K -= 1
     if unused_dim:  # a dimension no term uses: its hyper-parameters still see G_h[:,0] * yhat
         terms = np.asfortranarray(np.hstack([terms, np.zeros((K, 1), dtype=terms.dtype)]))
         d += 1
