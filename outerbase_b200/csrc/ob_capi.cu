@@ -408,7 +408,6 @@ int ob_lpdf_debug_build_geometry(ob_lpdf* l, int* out) {
   OB_TRY
   need(l, "l"); need(out, "out");
   if (auto* lik = dynamic_cast<obe::DevLik*>(l->p.get())) build_geometry(lik->ob, out);
-  else if (auto* gda = dynamic_cast<obe::LoglikGda*>(l->p.get())) build_geometry(gda->ob, out);
   else throw std::invalid_argument("only a likelihood holds a basis");
   OB_CATCH
 }
@@ -484,7 +483,7 @@ int ob_loglik_gda_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, ui
   need(ctx, "ctx"); need(om, "om");
   auto* h = new ob_lpdf();
   h->ctx = ctx;
-  try { h->p.reset(new obe::LoglikGda(ctx->c, &om->om, terms, K, y, x, N)); } catch (...) { delete h; throw; }
+  try { h->p.reset(new obe::LoglikGda(ctx->c, &om->om, terms, K, y, 1, x, N, /*multi=*/false)); } catch (...) { delete h; throw; }
   *out = h;
   OB_CATCH
 }
@@ -519,7 +518,7 @@ int ob_loglik_gda_multi_create(ob_ctx* ctx, ob_outermod* om, const uint64_t* ter
   if (C == 0) throw std::invalid_argument("ncol must be at least 1");
   auto* h = new ob_lpdf();
   h->ctx = ctx;
-  try { h->p.reset(new obe::LoglikGdaMulti(ctx->c, &om->om, terms, K, Y, C, x, N)); } catch (...) { delete h; throw; }
+  try { h->p.reset(new obe::LoglikGda(ctx->c, &om->om, terms, K, Y, C, x, N, /*multi=*/true)); } catch (...) { delete h; throw; }
   *out = h;
   OB_CATCH
 }
@@ -576,9 +575,9 @@ int ob_lpdf_set_flag(ob_lpdf* l, const char* which, int value) {
     if (!v) throw std::invalid_argument("domarg is a field of lpdfvec");
     v->domargadj = value;
   } else if (w == "dodiag") { /* R field name of loglik_gda::doda, interfaceR.cpp:748 */
-    if (auto* v = dynamic_cast<obe::LoglikGda*>(l->p.get())) { v->doda = value; v->redostd = true; }
-    else if (auto* m = dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) { m->doda = value; m->redostd = true; }
-    else throw std::invalid_argument("dodiag is a field of loglik_gda / loglik_gda_multi");
+    auto* v = dynamic_cast<obe::LoglikGda*>(l->p.get());
+    if (!v) throw std::invalid_argument("dodiag is a field of loglik_gda / loglik_gda_multi");
+    v->doda = value; v->redostd = true;
   } else throw std::invalid_argument("unknown flag " + w);
   OB_CATCH
 }
@@ -604,13 +603,12 @@ int ob_lpdf_get(ob_lpdf* l, const char* which, double* out, uint64_t* n) {
   } else if (w == "ncol") v = {double(l->p->ncol())};
   else if (w == "predvar_ncol") {
     if (auto* g = dynamic_cast<obe::LoglikGaussBase*>(l->p.get())) v = {double(g->predvar_ncol())};
-    else if (dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) v = {1.0};
-    else throw std::invalid_argument("predvar_ncol is a field of loglik_gauss / loglik_gauss_multi / loglik_gda_multi");
+    else if (dynamic_cast<obe::LoglikGda*>(l->p.get())) v = {1.0};
+    else throw std::invalid_argument("predvar_ncol is a field of loglik_gauss / loglik_gauss_multi / loglik_gda / loglik_gda_multi");
   }
   else if (w == "yhat") {
     if (auto* g = dynamic_cast<obe::LoglikGauss*>(l->p.get())) v = g->get_yhat();
-    else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(l->p.get())) v = g2->yhat;
-    else if (auto* g3 = dynamic_cast<obe::LoglikGdaMulti*>(l->p.get())) v = g3->get_yhat();
+    else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(l->p.get())) v = g2->get_yhat();
     else throw std::invalid_argument("yhat is a field of loglik_gauss / loglik_gda / loglik_gda_multi");
   } else if (w == "coeffsd") {
     auto* g = dynamic_cast<obe::LogprGauss*>(l->p.get());
@@ -630,7 +628,6 @@ int ob_predictor_create(ob_lpdf* loglik, ob_predictor** out) {
     if (auto* g3 = dynamic_cast<obe::LoglikStd*>(loglik->p.get())) h->p.reset(new obe::PredrStd(*g3)); /* before its base class */
     else if (auto* g = dynamic_cast<obe::LoglikGaussBase*>(loglik->p.get())) h->p.reset(new obe::PredGauss(*g));
     else if (auto* g2 = dynamic_cast<obe::LoglikGda*>(loglik->p.get())) h->p.reset(new obe::PredGda(*g2));
-    else if (auto* g4 = dynamic_cast<obe::LoglikGdaMulti*>(loglik->p.get())) h->p.reset(new obe::PredGda(*g4));
     else throw std::invalid_argument("cannot produce a predictor from this obj.");
   } catch (...) { delete h; throw; }
   *out = h;

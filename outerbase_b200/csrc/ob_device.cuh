@@ -319,8 +319,6 @@ void launch_cg_stage(Ctx& c, const CgParams& p, u64 ncol = 1);
  * when set, gives row i of every column the sd sd_rows[i] (loglik_gda's per-row noise) instead of either. */
 void launch_resid_multi(Ctx& c, const double* yhat, const double* y, double* w, u64 N, u64 ld, u64 C, double sd, bool update,
                         DevBuf<double>& partial, double* ssq_out, const double* sd_cols = nullptr, const double* sd_rows = nullptr);
-/* loglik_gda's obssd on the device: obssd[i] = sqrt(v0 + v1 (1 - phi2varc[i])) (phi2varc null: sqrt(v0)), pad rows 1 */
-void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd);
 
 /* ---- standard normals of the posterior draws (DESIGN §3.9), the same on the host and the device.
  * Philox4x32-10 (Salmon, Moraes, Dror, Shaw, SC'11; the constants of Random123) with key (seed low 32, seed high 32) and

@@ -7,10 +7,10 @@
  *   LoglikGaussBase   loglik_gauss      src/lpdfs/loglik_gauss.cpp:41-179  (N-length work on the GPU) on C responses;
  *                                       the products: LoglikGauss (one response), LoglikGaussMulti (C columns)
  *   LoglikStd         loglik_std        src/lpdfs/loglik_std.cpp:41-203
- *   LoglikGda         loglik_gda        src/lpdfs/loglik_gda.cpp:47-239
  *   LogprGaussMulti   logpr_gauss on each of C columns
- *   LoglikGdaMulti    loglik_gda on each of C columns (obfit_multi's stage 1)
- *   DevLik            what the device CG needs of a likelihood: LoglikGaussBase and LoglikGdaMulti derive from it
+ *   LoglikGda         loglik_gda        src/lpdfs/loglik_gda.cpp:47-239 on C responses (C = 1: loglik_gda itself;
+ *                                       C columns: obfit_multi's stage 1)
+ *   DevLik            what the device CG needs of a likelihood: LoglikGaussBase and LoglikGda derive from it
  *   LpdfVec           lpdfvec           src/fit.cpp:174-267,310-428,557-607 (diagonal branch), 269-299 (full branch)
  *   Pred              the predictors PredGauss (pred_gauss, loglik_gauss.cpp:196-227), PredrStd, PredGda
  *
@@ -696,6 +696,10 @@ struct OuterBase {
 };
 
 /* ------------------------------------------------------------------ lpdf family */
+[[noreturn]] inline void refuse_multi(const char* what) {
+  throw std::invalid_argument(std::string(what) + " is not available for multi-response objects");
+}
+
 struct Lpdf {
   double val = 0;
   std::vector<double> grad, gradhyp, gradpara, para, coeff, totdiaghess, para0, paravar;
@@ -735,11 +739,11 @@ struct Lpdf {
   virtual bool diaghessgradpara_dot(const std::vector<double>&, std::vector<double>&) { return false; }
   virtual void settotdiaghess(const std::vector<double>& dh) { totdiaghess = dh; didfulltothess = false; didnotothess = false; }
   /* full Hessian, fit.h:81-88: K x K, K x K x H, K x K x npara (column-major, slice after slice); empty when the
-   * object has none (loglik_gauss, loglik_gda) */
+   * object has none (loglik_gauss, loglik_gda); refused for multi-response objects */
   virtual void settothess(const std::vector<double>& h) { tothess = h; didfulltothess = true; didnotothess = false; }
-  virtual std::vector<double> hess() { return {}; }
-  virtual std::vector<double> hessgradhyp() { return {}; }
-  virtual std::vector<double> hessgradpara() { return {}; }
+  virtual std::vector<double> hess() { if (multi()) refuse_multi("the full Hessian"); return {}; }
+  virtual std::vector<double> hessgradhyp() { if (multi()) refuse_multi("the full Hessian"); return {}; }
+  virtual std::vector<double> hessgradpara() { if (multi()) refuse_multi("the full Hessian"); return {}; }
   virtual u64 nhyp() const { return 0; }
   virtual u64 nrow() const { return 0; }
   /* multi-response objects (loglik_gauss_multi, logpr_gauss_multi, an lpdfvec of them): ncol responses, coefficients
@@ -793,6 +797,7 @@ struct Lpdf {
 
   /* lpdf::optnewton, fit.cpp:98-131: one Newton step on the full Hessian */
   virtual void optnewton() {
+    if (multi()) refuse_multi("optnewton");
     fullhess = true;
     compute_val = true; compute_grad = true; compute_gradhyp = false; compute_gradpara = false;
     if (coeff.size() != nterms) coeff.assign(nterms, 0.0);
@@ -810,6 +815,7 @@ struct Lpdf {
   /* lpdf::optcg, fit.cpp:37-96.  The K-length algebra runs on the host in the
    * reference's order (Armadillo's two-accumulator accu); update/hessmult are the GPU. */
   virtual void optcg(double tol, u64 maxepch) {
+    if (multi()) refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi or loglik_gda_multi)");
     fullhess = false;
     compute_val = true; compute_grad = true; compute_gradhyp = false; compute_gradpara = false;
     if (coeff.size() != nterms) coeff.assign(nterms, 0.0);
@@ -949,9 +955,6 @@ struct LogprGauss : Lpdf { /* logpr_gauss.cpp:41-145 */
   u64 nhyp() const override { return om->nhyp(); }
 };
 
-[[noreturn]] inline void refuse_multi(const char* what) {
-  throw std::invalid_argument(std::string(what) + " is not available for multi-response objects");
-}
 /* K x S -> (K C) x S: each length-K column repeated C times */
 inline std::vector<double> tile_cols(const std::vector<double>& v, u64 K, u64 C) {
   const u64 S = K ? v.size() / K : 0;
@@ -1277,9 +1280,6 @@ struct LoglikGauss : LoglikGaussBase {
   }
 };
 
-/* loglik_gda (src/lpdfs/loglik_gda.cpp:47-239): the stage-1 likelihood of obfit, built on a <= 3*numb-row subsample
- * (R/fitting.R:79-84).  Every Phi-type product runs on the GPU kernels through the outerbase operators; the
- * N-vector bookkeeping around them (per-row noise scale and its derivatives) follows the reference on the host. */
 /* loglik_std, src/lpdfs/loglik_std.cpp:41-203: loglik_gauss's model (same value, gradients, Hessian products and
  * diagonals -- the formulas of :100-165 are loglik_gauss.cpp:110-179's) plus the full K x K Hessian that lpdf::optnewton
  * and the full branch of lpdfvec::buildhess need.  The reference keeps the explicit N x K basis and its N x K x H cube
@@ -1324,161 +1324,6 @@ struct LoglikStd : LoglikGauss {
     for (double& v : o) v = -2 * v;
     return o;
   }
-};
-
-/* loglik_gda's per-row noise sd and the host work that depends on it only, not on the response (shared by LoglikGda and
- * LoglikGdaMulti): the sd's derivatives (loglik_gda.cpp:226-235) and the Hessian diagonals (:172-211), all K- or
- * N-sized on the host around the GPU products, in the reference's operation order */
-struct GdaSd {
-  std::vector<double> obssd, obssd_gradhyp, obssd_gradpara;
-  /* from obssd and rterms = residvar (read only with doda) */
-  void sd_grads(OuterBase& ob, const u64* terms, u64 K, const std::vector<double>& para, bool doda, const std::vector<double>& rterms) {
-    const u64 N = obssd.size(), H = ob.H;
-    if (doda) {
-      obssd_gradhyp.resize(N * H);
-      ob.residvar_gradhyp(terms, K, obssd_gradhyp.data());
-      for (u64 h = 0; h < H; ++h)
-        for (u64 i = 0; i < N; ++i) obssd_gradhyp[i + h * N] *= (std::exp(2 * para[1]) * 0.5) / obssd[i];
-    }
-    obssd_gradpara.assign(N * 2, 0.0);
-    for (u64 i = 0; i < N; ++i) {
-      obssd_gradpara[i] = std::exp(2 * para[0]) / obssd[i];
-      obssd_gradpara[i + N] = doda ? std::exp(2 * para[1]) * rterms[i] / obssd[i] : 0.0;
-    }
-  }
-  std::vector<double> gda_diaghess(OuterBase& ob, const u64* terms, u64 K) const { /* :172-175 */
-    const u64 N = obssd.size();
-    std::vector<double> t(N), o(K);
-    for (u64 i = 0; i < N; ++i) t[i] = 1 / (obssd[i] * obssd[i]);
-    ob.tmm(1, terms, K, t.data(), o.data());
-    return o;
-  }
-  std::vector<double> gda_diaghessgradhyp(OuterBase& ob, const u64* terms, u64 K, bool doda) const { /* :182-196 */
-    const u64 N = obssd.size(), H = ob.H;
-    std::vector<double> temp(N), lh(K * H);
-    for (u64 i = 0; i < N; ++i) temp[i] = 1 / (obssd[i] * obssd[i]);
-    ob.tmm_gradhyp(1, terms, K, temp.data(), nullptr, lh.data());
-    for (u64 i = 0; i < N; ++i) temp[i] *= -2 / obssd[i];
-    if (doda) {
-      std::vector<double> t2(obssd_gradhyp), add(K * H);
-      for (u64 h = 0; h < H; ++h)
-        for (u64 i = 0; i < N; ++i) t2[i + h * N] *= temp[i];
-      ob.tmm_mat(1, terms, K, t2.data(), H, add.data());
-      for (u64 i = 0; i < K * H; ++i) lh[i] += add[i];
-    }
-    return lh;
-  }
-  std::vector<double> gda_diaghessgradpara(OuterBase& ob, const u64* terms, u64 K) const { /* :203-211 */
-    const u64 N = obssd.size();
-    std::vector<double> t2(obssd_gradpara), o(K * 2);
-    for (u64 q = 0; q < 2; ++q)
-      for (u64 i = 0; i < N; ++i) t2[i + q * N] *= (1 / (obssd[i] * obssd[i])) * (-2 / obssd[i]);
-    ob.tmm_mat(1, terms, K, t2.data(), 2, o.data());
-    return o;
-  }
-  /* Armadillo's two-accumulator dot */
-  static double dot2(const double* a, const double* b, u64 n) {
-    double s1 = 0, s2 = 0;
-    u64 j;
-    for (j = 1; j < n; j += 2) { s1 += a[j - 1] * b[j - 1]; s2 += a[j] * b[j]; }
-    if ((j - 1) < n) s1 += a[j - 1] * b[j - 1];
-    return s1 + s2;
-  }
-};
-
-struct LoglikGda : Lpdf, GdaSd {
-  Ctx& ctx;
-  const OuterMod* om;
-  OuterBase ob;
-  std::vector<double> x_host, y;
-  u64 N = 0;
-  bool doda = true, redostd = true;
-  std::vector<double> yhat, yhatge, residtemp, residtemp2;
-
-  LoglikGda(Ctx& c, const OuterMod* om_, const u64* t, u64 K, const double* yh, const double* xh, u64 N_)
-      : ctx(c), om(om_), ob(c, om_, xh, N_, true, t, K), N(N_) {
-    if (ctx.nranks > 1) throw std::logic_error("loglik_gda is the single-rank subsample model of obfit stage 1");
-    d = om->d; npara = 2;
-    terms.assign(t, t + K * d);
-    nterms = K;
-    x_host.assign(xh, xh + N * d);
-    y.assign(yh, yh + N);
-    para0 = {0.5 * std::log(0.01 * DevLik::arma_var(yh, N)), 0.0};
-    paravar = {4, 4};
-    para = para0;
-    buildstd();
-  }
-  void setnthreads(int k) override { ob.nthreads = k; }
-  void updateom() override { ob.build(); if (doda) redostd = true; }
-  void updatepara(const double* p, u64 n) override { para.assign(p, p + n); redostd = true; }
-  void updateterms(const u64* t, u64 K) override { terms.assign(t, t + K * d); nterms = K; if (doda) redostd = true; }
-  void buildstd() { /* :217-236 */
-    if (redostd) {
-      const u64 K = nterms;
-      std::vector<double> rterms(N);
-      ob.residvar(terms.data(), K, rterms.data());
-      obssd.resize(N);
-      for (u64 i = 0; i < N; ++i) {
-        double v = std::exp(2 * para[0]);
-        if (doda) v += std::exp(2 * para[1]) * rterms[i];
-        obssd[i] = std::sqrt(v);
-      }
-      sd_grads(ob, terms.data(), K, para, doda, rterms);
-    }
-    redostd = false;
-  }
-  void update(const std::vector<double>& c) override { /* :116-149 */
-    coeff = c;
-    const u64 K = nterms, H = ob.H;
-    if (c.size() != K) throw std::range_error("coeff must have one entry per term");
-    yhat.resize(N);
-    if (compute_gradhyp) { yhatge.resize(N * H); ob.mm_gradhyp(0, terms.data(), K, coeff.data(), yhat.data(), yhatge.data()); }
-    else ob.mm(0, terms.data(), K, coeff.data(), yhat.data());
-    buildstd();
-    residtemp.resize(N); residtemp2.resize(N);
-    for (u64 i = 0; i < N; ++i) { residtemp[i] = (yhat[i] - y[i]) / obssd[i]; residtemp2[i] = residtemp[i] * residtemp[i]; }
-    if (compute_val) {
-      std::vector<double> t(N);
-      for (u64 i = 0; i < N; ++i) t[i] = std::log(obssd[i]);
-      val = -0.5 * obh::sum2(residtemp2.data(), N) - obh::sum2(t.data(), N);
-    }
-    if (compute_grad) {
-      std::vector<double> inv(N);
-      for (u64 i = 0; i < N; ++i) { residtemp[i] = -1. * (residtemp[i] / obssd[i]); residtemp2[i] /= obssd[i]; inv[i] = 1 / obssd[i]; }
-      grad.resize(K);
-      ob.tmm(0, terms.data(), K, residtemp.data(), grad.data());
-      if (compute_gradhyp) {
-        gradhyp.assign(H, 0.0);
-        for (u64 h = 0; h < H; ++h) {
-          gradhyp[h] = dot2(residtemp.data(), yhatge.data() + h * N, N);
-          if (doda) {
-            gradhyp[h] += dot2(residtemp2.data(), obssd_gradhyp.data() + h * N, N);
-            gradhyp[h] -= dot2(inv.data(), obssd_gradhyp.data() + h * N, N);
-          }
-        }
-      }
-      if (compute_gradpara) {
-        gradpara.assign(2, 0.0);
-        for (u64 q = 0; q < 2; ++q) {
-          gradpara[q] = dot2(residtemp2.data(), obssd_gradpara.data() + q * N, N);
-          gradpara[q] -= dot2(inv.data(), obssd_gradpara.data() + q * N, N);
-        }
-      }
-    }
-  }
-  std::vector<double> hessmult(const std::vector<double>& g) override { /* :156-164 */
-    const u64 K = nterms;
-    std::vector<double> yt(N), o(K);
-    ob.mm(0, terms.data(), K, g.data(), yt.data());
-    for (u64 i = 0; i < N; ++i) { yt[i] /= obssd[i]; yt[i] /= obssd[i]; }
-    ob.tmm(0, terms.data(), K, yt.data(), o.data());
-    return o;
-  }
-  std::vector<double> diaghess() override { return gda_diaghess(ob, terms.data(), nterms); }
-  std::vector<double> diaghessgradhyp() override { return gda_diaghessgradhyp(ob, terms.data(), nterms, doda); }
-  std::vector<double> diaghessgradpara() override { return gda_diaghessgradpara(ob, terms.data(), nterms); }
-  u64 nhyp() const override { return ob.H; }
-  u64 nrow() const override { return N; }
 };
 
 /* ------------------------------------------------------------------ multi-response: C responses observed at the same rows
@@ -1602,11 +1447,6 @@ struct LogprGaussMulti : Lpdf {
     }
     return true;
   }
-  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
-  void optnewton() override { refuse_multi("optnewton"); }
-  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi)"); }
 };
 
 /* the matrix path, also for C = 1: mm_mat_dev / tmm_mat_dev (the FP64 tensor-core kernels for C >= 8 on a specialised
@@ -1671,31 +1511,29 @@ struct LoglikGaussMulti : LoglikGaussBase {
       for (u64 c = 0; c < C; ++c) for (u64 h = 0; h < H; ++h) gradhyp[h] += r[c * H + h];
     }
   }
-  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
-  void optnewton() override { refuse_multi("optnewton"); }
-  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gauss_multi)"); }
 };
 
-/* loglik_gda (loglik_gda.cpp:47-239) on C responses observed at the same rows: column c is loglik_gda on Y[:,c].  The
- * columns share the basis, the terms table, the hyper-parameters, dodiag and both para entries, so the per-row noise
- * sd obssd is one N-vector; it is formed on the device (gda_obssd_kernel) from the squared product residvar runs, and
- * rebuilt where LoglikGda sets redostd.  val, gradhyp and gradpara are the sums over the columns (in column order) of
- * loglik_gda's, grad is K x C, hessmult is block-diagonal, and the Hessian diagonals, which do not depend on the
- * response, are loglik_gda's computed once and repeated C times.  The products are the matrix path of LoglikGaussMulti:
- * mm_mat_dev | resid_multi with the per-row sd | tmm_mat_dev; the sd's hyper-gradient bookkeeping stays on the host as in
- * LoglikGda and runs once per update with gradients.  Para is never per column; one rank only (obfit's stage-1
- * subsample). */
-struct LoglikGdaMulti : DevLik, GdaSd {
+/* loglik_gda (loglik_gda.cpp:47-239), the stage-1 likelihood of obfit on a <= 3*numb-row subsample (R/fitting.R:79-84),
+ * on C responses observed at the same rows: column c is loglik_gda on Y[:,c].  The columns share the basis, the terms
+ * table, the hyper-parameters, dodiag and both para entries, so the per-row noise sd obssd is one N-vector, formed on
+ * the host in the reference's operation order and uploaded for the residual pass.  val, gradhyp and gradpara are the
+ * sums over the columns (in column order) of loglik_gda's, grad is K x C, hessmult is block-diagonal, and the Hessian
+ * diagonals, which do not depend on the response, are loglik_gda's computed once and repeated C times.  The products
+ * are the matrix path of LoglikGaussMulti: mm_mat_dev | resid_multi with the per-row sd | tmm_mat_dev; the sd's
+ * derivatives and the Hessian diagonals are N- and K-sized host work around the GPU products, in the reference's
+ * order.  Para is never per column; one rank only (obfit's stage-1 subsample).
+ * multi: the multi-response object at every C (loglik_gda_multi, paired with logpr_gauss_multi); otherwise C = 1 and
+ * the object is the single-response loglik_gda (paired with logpr_gauss, optimised by the host CG loop). */
+struct LoglikGda : DevLik {
+  bool is_multi;
   bool doda = true, redostd = true;
   double sumlogsd = 0; /* sum_i log obssd_i in obh::sum2 order: the likelihood's constant, the same for every column */
-  std::vector<double> y_host;
-  DevBuf<double> sd, phi2, ssq, partial, gh;
+  std::vector<double> y_host, obssd, obssd_gradhyp, obssd_gradpara;
+  DevBuf<double> sd, ssq, partial, gh;
 
-  LoglikGdaMulti(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_)
-      : DevLik(c, om_, t, K_, yh, C_, xh, N_) {
-    if (ctx.nranks > 1) throw std::logic_error("loglik_gda_multi is the single-rank subsample model of obfit stage 1");
+  LoglikGda(Ctx& c, const OuterMod* om_, const u64* t, u64 K_, const double* yh /* N x C */, u64 C_, const double* xh, u64 N_, bool multi_)
+      : DevLik(c, om_, t, K_, yh, C_, xh, N_), is_multi(multi_) {
+    if (ctx.nranks > 1) throw std::logic_error("loglik_gda is the single-rank subsample model of obfit stage 1");
     npara = 2;
     y_host.assign(yh, yh + N * C);
     double vs = 0; /* para0[0] = 0.5 log(0.01 mean_c var(Y[:,c])), loglik_gda.cpp:59 on the mean variance */
@@ -1706,7 +1544,7 @@ struct LoglikGdaMulti : DevLik, GdaSd {
     ssq.ensure(C);
     buildstd();
   }
-  bool multi() const override { return true; }
+  bool multi() const override { return is_multi; }
   void updateom() override { ob.build(); if (doda) redostd = true; }
   void updatepara(const double* p, u64 n) override {
     if (n != 2) throw std::range_error("para must have two entries");
@@ -1714,25 +1552,38 @@ struct LoglikGdaMulti : DevLik, GdaSd {
     redostd = true;
   }
   void updateterms(const u64* t, u64 K_) override { terms.assign(t, t + K_ * d); K = K_; nterms = K * C; if (doda) redostd = true; }
+  /* Armadillo's two-accumulator dot */
+  static double dot2(const double* a, const double* b, u64 n) {
+    double s1 = 0, s2 = 0;
+    u64 j;
+    for (j = 1; j < n; j += 2) { s1 += a[j - 1] * b[j - 1]; s2 += a[j] * b[j]; }
+    if ((j - 1) < n) s1 += a[j - 1] * b[j - 1];
+    return s1 + s2;
+  }
   void buildstd() { /* loglik_gda.cpp:217-236 */
     if (!redostd) return;
-    const u64 ld = ob.ld;
-    std::vector<double> rterms;
-    sd.ensure(std::max<u64>(ld, 1));
-    if (doda) { /* residvar = 1 - Phi^2 varc */
-      std::vector<double> varc(K);
-      om->getvar(terms.data(), K, varc.data());
-      kbuf.upload(varc, ctx.stream);
-      phi2.ensure(std::max<u64>(ld, 1));
-      ob.mm_dev(terms.data(), K, 1, kbuf.p, phi2.p);
-      rterms.resize(N);
-      ob.d2h(rterms.data(), phi2.p, N);
-      for (u64 i = 0; i < N; ++i) rterms[i] = 1 - rterms[i];
-    }
-    obd::launch_gda_obssd(ctx, doda ? phi2.p : nullptr, N, ld, std::exp(2 * para[0]), std::exp(2 * para[1]), sd.p);
+    const u64 H = ob.H;
+    std::vector<double> rterms(N);
+    if (doda) ob.residvar(terms.data(), K, rterms.data());
     obssd.resize(N);
-    ob.d2h(obssd.data(), sd.p, N);
-    sd_grads(ob, terms.data(), K, para, doda, rterms);
+    for (u64 i = 0; i < N; ++i) {
+      double v = std::exp(2 * para[0]);
+      if (doda) v += std::exp(2 * para[1]) * rterms[i];
+      obssd[i] = std::sqrt(v);
+    }
+    sd.upload(obssd, ctx.stream);
+    ctx.sync(); /* obssd may change at the next buildstd */
+    if (doda) { /* :226-235 */
+      obssd_gradhyp.resize(N * H);
+      ob.residvar_gradhyp(terms.data(), K, obssd_gradhyp.data());
+      for (u64 h = 0; h < H; ++h)
+        for (u64 i = 0; i < N; ++i) obssd_gradhyp[i + h * N] *= (std::exp(2 * para[1]) * 0.5) / obssd[i];
+    }
+    obssd_gradpara.assign(N * 2, 0.0);
+    for (u64 i = 0; i < N; ++i) {
+      obssd_gradpara[i] = std::exp(2 * para[0]) / obssd[i];
+      obssd_gradpara[i + N] = doda ? std::exp(2 * para[1]) * rterms[i] / obssd[i] : 0.0;
+    }
     std::vector<double> t(N);
     for (u64 i = 0; i < N; ++i) t[i] = std::log(obssd[i]);
     sumlogsd = obh::sum2(t.data(), N);
@@ -1816,14 +1667,34 @@ struct LoglikGdaMulti : DevLik, GdaSd {
     for (u64 c = 0; c < C; ++c) ob.d2h(o.data() + c * N, yhat.p + c * ob.ld, N);
     return o;
   }
-  std::vector<double> diaghess() override { return tile_cols(gda_diaghess(ob, terms.data(), K), K, C); }
-  std::vector<double> diaghessgradhyp() override { return tile_cols(gda_diaghessgradhyp(ob, terms.data(), K, doda), K, C); }
-  std::vector<double> diaghessgradpara() override { return tile_cols(gda_diaghessgradpara(ob, terms.data(), K), K, C); }
-  std::vector<double> hess() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradhyp() override { refuse_multi("the full Hessian"); }
-  std::vector<double> hessgradpara() override { refuse_multi("the full Hessian"); }
-  void optnewton() override { refuse_multi("optnewton"); }
-  void optcg(double, u64) override { refuse_multi("optcg outside lpdfvec(logpr_gauss_multi, loglik_gda_multi)"); }
+  std::vector<double> diaghess() override { /* :172-175 */
+    std::vector<double> t(N), o(K);
+    for (u64 i = 0; i < N; ++i) t[i] = 1 / (obssd[i] * obssd[i]);
+    ob.tmm(1, terms.data(), K, t.data(), o.data());
+    return tile_cols(o, K, C);
+  }
+  std::vector<double> diaghessgradhyp() override { /* :182-196 */
+    const u64 H = ob.H;
+    std::vector<double> temp(N), lh(K * H);
+    for (u64 i = 0; i < N; ++i) temp[i] = 1 / (obssd[i] * obssd[i]);
+    ob.tmm_gradhyp(1, terms.data(), K, temp.data(), nullptr, lh.data());
+    for (u64 i = 0; i < N; ++i) temp[i] *= -2 / obssd[i];
+    if (doda) {
+      std::vector<double> t2(obssd_gradhyp), add(K * H);
+      for (u64 h = 0; h < H; ++h)
+        for (u64 i = 0; i < N; ++i) t2[i + h * N] *= temp[i];
+      ob.tmm_mat(1, terms.data(), K, t2.data(), H, add.data());
+      for (u64 i = 0; i < K * H; ++i) lh[i] += add[i];
+    }
+    return tile_cols(lh, K, C);
+  }
+  std::vector<double> diaghessgradpara() override { /* :203-211 */
+    std::vector<double> t2(obssd_gradpara), o(K * 2);
+    for (u64 q = 0; q < 2; ++q)
+      for (u64 i = 0; i < N; ++i) t2[i + q * N] *= (1 / (obssd[i] * obssd[i])) * (-2 / obssd[i]);
+    ob.tmm_mat(1, terms.data(), K, t2.data(), 2, o.data());
+    return tile_cols(o, K, C);
+  }
 };
 
 struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
@@ -1840,7 +1711,7 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   LpdfVec(Lpdf* a, Lpdf* b) {
     if (a->multi() != b->multi() || a->ncol() != b->ncol())
       throw std::invalid_argument("lpdfvec: children must both be single-response, or multi-response with the same number of columns");
-    if ((dynamic_cast<LoglikGdaMulti*>(a) && b->para_per_column()) || (dynamic_cast<LoglikGdaMulti*>(b) && a->para_per_column()))
+    if ((dynamic_cast<LoglikGda*>(a) && b->para_per_column()) || (dynamic_cast<LoglikGda*>(b) && a->para_per_column()))
       throw std::invalid_argument("lpdfvec: loglik_gda_multi pairs with a shared-para logpr_gauss_multi only");
     kid[0] = a; kid[1] = b;
     terms = a->terms; d = a->d;
@@ -2104,7 +1975,9 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
     }
     Ctx& ctx = lk->ctx;
     const u64 K = lk->K, C = lk->C, NS = obd::CG_NSCAL;
-    if (!mult && (!ctx.device_cg || K == 0 || lk->N == 0 || !lk->ob.spec_for(terms.data(), K))) return false;
+    /* the single-response loglik_gda (a DevLik too) keeps the host loop */
+    if (!mult && (!dynamic_cast<LoglikGaussBase*>(lk) || !ctx.device_cg || K == 0 || lk->N == 0 || !lk->ob.spec_for(terms.data(), K)))
+      return false;
     compute_val = true; compute_grad = true; compute_gradhyp = false; compute_gradpara = false;
     if (coeff.size() != nterms) coeff.assign(nterms, 0.0);
     update(std::vector<double>(coeff));
@@ -2190,10 +2063,6 @@ struct LpdfVec : Lpdf { /* fit.cpp:174-267,310-428,557-607 */
   void optcg(double tol, u64 maxepch) override {
     fullhess = false; /* fit.cpp:38 */
     if (!optcg_device(tol, maxepch)) Lpdf::optcg(tol, maxepch);
-  }
-  void optnewton() override {
-    if (multi()) refuse_multi("optnewton");
-    Lpdf::optnewton();
   }
   bool multi() const override { return kid[0]->multi(); }
   u64 ncol() const override { return kid[0]->ncol(); }
@@ -2306,13 +2175,12 @@ struct PredrStd : Pred { /* loglik_std.cpp:219-257 */
   }
 };
 
-/* multi-response (LoglikGdaMulti): the mean is N x C, the variance one N-vector for all columns from the first K entries
- * of 1 / totdiaghess (its column blocks are equal) */
+/* the mean is N x C, the variance one N-vector for all columns from the first K entries of 1 / totdiaghess (its column
+ * blocks are equal) */
 struct PredGda : Pred { /* loglik_gda.cpp:249-283 */
   std::vector<double> coeffvar;
   bool doda;
-  PredGda(LoglikGda& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.nterms), coeffvar(inv_totdiaghess(lk)), doda(lk.doda) {}
-  PredGda(LoglikGdaMulti& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.K, lk.C), coeffvar(inv_totdiaghess(lk)), doda(lk.doda) {}
+  PredGda(LoglikGda& lk) : Pred(lk.ctx, lk.om, lk, lk.x_host, lk.N, lk.K, lk.C), coeffvar(inv_totdiaghess(lk)), doda(lk.doda) {}
   void var(double* out) override {
     ob->mm(1, terms.data(), K, coeffvar.data(), out);
     std::vector<double> rv(ob->N);

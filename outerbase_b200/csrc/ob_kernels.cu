@@ -558,19 +558,6 @@ __global__ void __launch_bounds__(kResidThreads) resid_multi_kernel(const double
   if (threadIdx.x == 0) partial[col * gridDim.x + blockIdx.x] = sm[0];
 }
 
-/* loglik_gda's per-row noise sd (LoglikGda::buildstd): v = v0, plus v1 (1 - phi2varc[i]) when phi2varc is set (dodiag;
- * phi2varc = Phi^2 varc, so that 1 - phi2varc is OuterBase::residvar), obssd = sqrt(v); rows N .. ld-1 are 1 */
-__global__ void gda_obssd_kernel(const double* __restrict__ phi2varc, u64 N, u64 ld, double v0, double v1, double* __restrict__ obssd) {
-  const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= ld) return;
-  double v = 1.0;
-  if (i < N) {
-    v = v0;
-    if (phi2varc) v += v1 * (1 - phi2varc[i]);
-  }
-  obssd[i] = sqrt(v);
-}
-
 __global__ void getmat_kernel(const double* const* load_src, const int* col_op, const uint32_t* csr_ptr,
                               const uint32_t* csr_col, int K, const double* scale, int sq, unsigned long long N,
                               double* out, unsigned long long ldo) {
@@ -2074,12 +2061,6 @@ void launch_sobol_pairs(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* 
   check_launch(c, "sobol_pairs_kernel");
   colsum_partials_kernel<<<(unsigned)(B * 2 * P), 32, 0, c.stream>>>(partial, (int)nx, out);
   check_launch(c, "colsum_partials_kernel");
-}
-
-void launch_gda_obssd(Ctx& c, const double* phi2varc, u64 N, u64 ld, double v0, double v1, double* obssd) {
-  if (ld == 0) return;
-  gda_obssd_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, c.stream>>>(phi2varc, N, ld, v0, v1, obssd);
-  check_launch(c, "gda_obssd_kernel");
 }
 
 void launch_fill(Ctx& c, double* p, u64 n, double v) {

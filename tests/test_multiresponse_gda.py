@@ -1,5 +1,6 @@
 """Multi-response loglik_gda: C responses on one basis with one per-row noise scale (include/outerbase_b200_multi_gda.h,
-ob_engine.hpp LoglikGdaMulti), and the two-stage fitting.obfit_multi it makes possible.
+ob_engine.hpp LoglikGda, the object behind both loglik_gda and loglik_gda_multi), and the two-stage fitting.obfit_multi
+it makes possible.
 
 The reference is the definition itself: C single-response oracle loglik_gda objects and loops over them
 (tests/multiresponse_gda_reference.py).  GPU: the product's column-batched objects and CG against it."""
@@ -137,6 +138,33 @@ def test_gpu_likelihood_matches_the_reference(gpu, oracle, families, spec, dodia
     assert relerr(g["yhat"], o["yhat"]) < 1e-8
     assert relerr(g["hm"], o["hm"]) < 1e-8 and relerr(g["dh"], o["dh"]) < 1e-8
     assert relerr(g["dhh"], o["dhh"]) < 1e-7 and relerr(g["dhp"], o["dhp"]) < 1e-8
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("spec", [0, 1])
+@pytest.mark.parametrize("dodiag", [True, False])
+def test_gpu_one_column_is_loglik_gda_bit_for_bit(gpu, families, spec, dodiag):
+    """loglik_gda_multi at C = 1 is loglik_gda: the same bits for every likelihood output"""
+    families(spec)
+    res = {}
+    for name in ("single", "multi"):
+        om, x, Y, terms, rng = gda_objects(gpu, 1)
+        lk = gpu.loglik_gda(om, terms, Y[:, 0], x) if name == "single" else gpu.loglik_gda_multi(om, terms, Y, x)
+        lk.dodiag = dodiag
+        para0 = np.array(lk.para)
+        lk.updatepara([np.log(0.2), -0.5])
+        a = rng.normal(size=K_GDA) / 50
+        g = rng.normal(size=K_GDA)
+        _flags(lk)
+        lk.update(a)
+        res[name] = dict(para0=para0, val=lk.val, grad=np.ravel(lk.grad), gh=np.array(lk.gradhyp), gp=np.array(lk.gradpara),
+                         yhat=np.ravel(lk.yhat), hm=lk.hessmult(g), dh=lk.diaghess(), dhh=lk.diaghessgradhyp(),
+                         dhp=lk.diaghessgradpara())
+        if name == "single":
+            with pytest.raises(ValueError):  # para has two entries
+                lk.updatepara([0.0])
+    for k, v in res["single"].items():
+        np.testing.assert_array_equal(v, res["multi"][k], err_msg=k)
 
 
 def test_reference_default_para_is_the_mean_variance(oracle):
