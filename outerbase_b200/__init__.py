@@ -11,7 +11,8 @@ import subprocess
 from pathlib import Path
 
 from .binding import (Library, getpara, gethyp, header_symbols, loglik_gauss, loglik_gda, logpr_gauss, lpdf, lpdfvec,  # noqa: F401
-                      outerbase, outermod, predictor, setcovfs, setknot, sobol, sobol_pairs)
+                      outerbase, outermod, predictor, setcovfs, setknot, sobol, sobol_pairs,
+                      sobol_shapley)
 
 ROOT = Path(__file__).resolve().parent
 REPO = ROOT.parent
@@ -25,6 +26,7 @@ MULTI_GDA_HEADER = REPO / "include" / "outerbase_b200_multi_gda.h"  # multi-resp
 DRAWS_HEADER = REPO / "include" / "outerbase_b200_draws.h"  # posterior draws of a fitted model
 SOBOL_HEADER = REPO / "include" / "outerbase_b200_sobol.h"  # Sobol sensitivity indices of a fitted model
 SOBOL_PAIRS_HEADER = REPO / "include" / "outerbase_b200_sobol_pairs.h"  # their second-order (input-pair) forms
+SOBOL_SHAPLEY_HEADER = REPO / "include" / "outerbase_b200_sobol_shapley.h"  # Shapley effects of a fitted model
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -39,7 +41,7 @@ def _stale() -> bool:
         return True
     t = LIBPATH.stat().st_mtime
     deps = list(CSRC.glob("*")) + [HEADER, MULTI_HEADER, PERCOL_HEADER, MULTI_GDA_HEADER, DRAWS_HEADER, SOBOL_HEADER,
-                                   SOBOL_PAIRS_HEADER]
+                                   SOBOL_PAIRS_HEADER, SOBOL_SHAPLEY_HEADER]
     return any(p.stat().st_mtime > t for p in deps)
 
 

@@ -993,6 +993,35 @@ def sobol_pairs(lib, om, terms, coeff, x):
     return dict(mean=mean, var=var, first=first, total=total, second=S2, supset=SU)
 
 
+def sobol_shapley(lib, om, terms, coeff, x):
+    """binding.sobol's four outputs (the same bits) and shapley, the Shapley effect of every input: the variance of
+    each ANOVA component split equally among its inputs, sum_{u containing l} sigma2_u / |u|
+    (include/outerbase_b200_sobol_shapley.h).  shapley has d entries for a K-vector coeff, d x B for a K x B coeff; it
+    adds up to var, and first <= shapley <= total."""
+    t = _terms(terms)
+    K, d = t.shape
+    if d != om.d:
+        raise ValueError(f"terms has {d} columns, the outermod {om.d} dimensions")
+    x = _f64(x)
+    if x.ndim != 2 or x.shape[1] != d:
+        raise ValueError("x must be nq x d")
+    c = _f64(coeff)
+    vec = c.ndim == 1
+    if vec:
+        c = c.reshape((-1, 1), order="F")
+    if c.ndim != 2 or c.shape[0] != K:
+        raise ValueError("coeff must have one row per term")
+    B = c.shape[1]
+    mean, var = np.empty(B), np.empty(B)
+    first, total, shapley = (np.empty((d, B), order="F") for _ in range(3))
+    lib.call("sobol_shapley", lib.ctx, om._h, _p(t), _u(K), _p(c), _u(B), _p(x), _u(x.shape[0]), _p(mean), _p(var),
+             _p(first), _p(total), _p(shapley))
+    if vec:
+        return dict(mean=float(mean[0]), var=float(var[0]), first=first[:, 0].copy(), total=total[:, 0].copy(),
+                    shapley=shapley[:, 0].copy())
+    return dict(mean=mean, var=var, first=first, total=total, shapley=shapley)
+
+
 class predictor(_Handle):
     """new(predictor, loglik) -- src/fit.h:352-361."""
     _destroy = "predictor_destroy"

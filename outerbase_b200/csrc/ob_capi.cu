@@ -10,6 +10,7 @@
 #include "../../include/outerbase_b200_draws.h"
 #include "../../include/outerbase_b200_sobol.h"
 #include "../../include/outerbase_b200_sobol_pairs.h"
+#include "../../include/outerbase_b200_sobol_shapley.h"
 
 #include "ob_engine.hpp"
 
@@ -713,6 +714,18 @@ int ob_sobol_pairs(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t
     if (om->om.d > 1) { need(second, "second"); need(supset, "supset"); }
   }
   obe::sobol_pairs(ctx->c, &om->om, terms, K, coeff, B, xq, nq, mean, var, first, total, second, supset);
+  OB_CATCH
+}
+
+int ob_sobol_shapley(ob_ctx* ctx, ob_outermod* om, const uint64_t* terms, uint64_t K, const double* coeff, uint64_t B,
+                     const double* xq, uint64_t nq, double* mean, double* var, double* first, double* total,
+                     double* shapley) {
+  OB_TRY
+  need(ctx, "ctx"); need(om, "om");
+  if (K) { need(terms, "terms"); if (B) need(coeff, "coeff"); }
+  if (nq) need(xq, "xq");
+  if (B) { need(mean, "mean"); need(var, "var"); need(first, "first"); need(total, "total"); need(shapley, "shapley"); }
+  obe::sobol_shapley(ctx->c, &om->om, terms, K, coeff, B, xq, nq, mean, var, first, total, shapley);
   OB_CATCH
 }
 

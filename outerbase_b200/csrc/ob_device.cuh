@@ -389,6 +389,15 @@ void launch_sobol_forms(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* 
 u64 sobol_pairs_partials(u64 K, u64 d);
 void launch_sobol_pairs(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
                         const double* cov, u64 c_n, const double* coeff_t, u64 B, double* partial, double* out);
+/* Shapley effects (DESIGN §3.12): out[b d + l] = sum_{k <= k'} w theta_kb theta_k'b c_l sum_i w_i prod_{j != l} h_j(z_i),
+ * h_j(z) = p_j + z c_j, with nodes = z_0 .. z_{n-1}, w_0 .. w_{n-1} (device memory) a quadrature rule on [0, 1] exact
+ * for degree d - 1.  A GEMM over the term pairs on the FP64 tensor cores; the term-pair chunks and the k-step split
+ * depend on K and d alone, so column b's result depends on nothing but column b and is the same bits on every run.
+ * coeff_t as launch_sobol_pairs.  partial holds sobol_shapley_partials(K) doubles per output. */
+u64 sobol_shapley_partials(u64 K);
+void launch_sobol_shapley(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                          const double* cov, u64 c_n, const double* coeff_t, u64 B, const double* nodes, u64 n,
+                          double* partial, double* out);
 
 /* basis build: cov(x, knots) . rotmat, normalise (modandbase.cpp:285-327, 547-626) */
 struct BuildDims {

@@ -2277,11 +2277,12 @@ struct Draws {
   }
 };
 
-/* ------------------------------------------------------------------ Sobol indices (DESIGN §3.10, §3.11)
+/* ------------------------------------------------------------------ Sobol indices (DESIGN §3.10, §3.11, §3.12)
  * f_b(x) = sum_k coeff[k, b] prod_l R_l(x_l, t_kl) under the product of the empirical marginals of X_q's columns:
  * mean[b], var[b], first[l + d b] = Var(E[f_b | x_l]) and total[l + d b] = E[Var(f_b | x_-l)], exact quadratic forms in
  * the coefficients built from the per-dimension tables mu_l and C_l (include/outerbase_b200_sobol.h); sobol_pairs adds
- * the second-order forms of every input pair (include/outerbase_b200_sobol_pairs.h).  X_q's basis is built compact and
+ * the second-order forms of every input pair (include/outerbase_b200_sobol_pairs.h), sobol_shapley the Shapley effects
+ * (include/outerbase_b200_sobol_shapley.h).  X_q's basis is built compact and
  * without gradients, as Draws::predict builds its rows. */
 inline void sobol_check(const Ctx& ctx, u64 K, u64 B, u64 nq) {
   if (B == 0) throw std::invalid_argument("sobol: coeff must have at least one column");
@@ -2391,6 +2392,61 @@ inline void sobol_pairs(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, c
       second[r + P * b] = out[b * 2 * P + 2 * r];
       supset[r + P * b] = out[b * 2 * P + 2 * r + 1];
     }
+}
+
+/* The n-node Gauss-Legendre rule mapped to [0, 1], nodes ascending: zw[i] = z_i, zw[n + i] = w_i.  Newton's method on
+ * the three-term recurrence of P_n in long double, from Tricomi's initial guesses; exact for polynomials of degree
+ * 2n - 1, the weights positive and adding up to 1. */
+inline std::vector<double> gauss_legendre01(u64 n) {
+  std::vector<double> zw(2 * n);
+  const long double pi = 3.141592653589793238462643383279502884L;
+  for (u64 i = 0; i < n; ++i) {
+    /* P_n(x) and P_n'(x) = n (x P_n - P_{n-1}) / (x^2 - 1) */
+    auto legendre = [n](long double x, long double* dp) {
+      long double p0 = 1.0L, p1 = x;
+      for (u64 k = 2; k <= n; ++k) {
+        const long double p2 = ((2.0L * k - 1.0L) * x * p1 - (k - 1.0L) * p0) / (long double)k;
+        p0 = p1; p1 = p2;
+      }
+      *dp = (long double)n * (x * p1 - p0) / (x * x - 1.0L);
+      return p1;
+    };
+    long double x = std::cos(pi * ((long double)i + 0.75L) / ((long double)n + 0.5L)), dp = 1.0L;
+    for (int it = 0; it < 100; ++it) {
+      const long double dx = legendre(x, &dp) / dp;
+      x -= dx;
+      if (std::fabs(dx) <= 4 * std::numeric_limits<long double>::epsilon()) break;
+    }
+    legendre(x, &dp);
+    zw[i] = (double)((1.0L - x) / 2.0L); /* x descends with i: z ascends */
+    zw[n + i] = (double)(1.0L / ((1.0L - x * x) * dp * dp));
+  }
+  return zw;
+}
+
+/* sobol's four outputs (the same bits) and the Shapley effect of every input, shapley[l + d b] =
+ * sum_{u containing l} sigma2_u / |u|, by the ceil(d / 2)-node Gauss-Legendre rule, exact for the degree d - 1
+ * polynomial in z it integrates (DESIGN §3.12) */
+inline void sobol_shapley(Ctx& ctx, const OuterMod* om, const u64* terms, u64 K, const double* coeff, u64 B,
+                          const double* xq, u64 nq, double* mean, double* var, double* first, double* total,
+                          double* shapley) {
+  sobol_check(ctx, K, B, nq);
+  SobolTables T(ctx, om, terms, K, coeff, B, xq, nq);
+  sobol_forms(ctx, T, terms, K, coeff, B, mean, var, first, total);
+  const u64 d = T.d, n = std::max<u64>(1, (d + 1) / 2);
+  /* the Shapley kernel reads the B columns of a term together */
+  std::vector<double> ct(K * B);
+  for (u64 b = 0; b < B; ++b)
+    for (u64 k = 0; k < K; ++k) ct[b + B * k] = coeff[k + K * b];
+  const std::vector<double> zw = gauss_legendre01(n);
+  DevBuf<double> part, out_dev, coeff_t, nodes;
+  coeff_t.upload(ct, ctx.stream);
+  nodes.upload(zw, ctx.stream);
+  part.ensure(B * d * obd::sobol_shapley_partials(K));
+  out_dev.ensure(B * d);
+  obd::launch_sobol_shapley(ctx, T.terms_dev.p, K, d, T.dims_dev.p, T.mu_dev.p, T.mu_n, T.c_dev.p, T.c_n, coeff_t.p, B,
+                            nodes.p, n, part.p, out_dev.p);
+  T.ob.d2h(shapley, out_dev.p, B * d); /* out[b d + l] is shapley's layout */
 }
 
 } // namespace obe

@@ -2063,6 +2063,222 @@ void launch_sobol_pairs(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* 
   check_launch(c, "colsum_partials_kernel");
 }
 
+/* ---- Shapley effects on the FP64 tensor cores (DESIGN §3.12).  out(l, b) = sum_q F[q, l] U[q, b] over the term pairs
+ * q = (k <= k'), F[q, l] = c_l sum_i w_i prod_{j != l} h_j(z_i) with h_j(z) = p_j + z c_j and (z_i, w_i) the n-node
+ * Gauss-Legendre rule on [0, 1]: a GEMM with the term pairs as the contraction dimension, F formed per chunk in shared
+ * memory and never stored in HBM.  One CTA holds all d <= 80 output rows (mt = ceil(d / 8) row tiles) and kShapCols
+ * columns, and walks the term-pair chunks ch = blockIdx.x, + gridDim.x, ... */
+constexpr int kShapQ = 32;                        /* term pairs per chunk: 8 k-steps of m8n8k4, 8 threads per pair */
+constexpr int kShapCols = 64, kShapUS = kShapCols + 4; /* = 4 mod 16 doubles, as kPairsUS */
+constexpr int kShapTiles = 10;                    /* most (row tile, column tile) accumulators of a warp: mt ksplit */
+constexpr int kShapCTAs = 296;                    /* CTAs over the chunks: two per SM */
+
+struct SobolShapleyArgs {
+  SobolFormsArgs f;
+  const double* nodes; /* z_0 .. z_{n-1}, then w_0 .. w_{n-1} */
+  int n;
+};
+
+/* k-step groups of the contraction: 8 / ksplit warps per group, group kg takes k-steps kg, kg + ksplit, ... of every
+ * chunk, and the groups' sums are added in kg order at the end.  A warp holds at most mt ksplit <= kShapTiles tiles, so
+ * at small d the k-steps spread the DMMAs over all eight warps instead of leaving warps without rows.  mt alone decides
+ * the split: a column's sum order does not depend on B. */
+__host__ __device__ inline int shapley_ksplit(int mt) { return mt == 1 ? 8 : mt == 2 ? 4 : mt <= 5 ? 2 : 1; }
+/* F's row stride: the smallest = 4 mod 16 doubles above the 8 mt rows */
+__host__ __device__ inline int shapley_fs(int mt) { return (8 * mt + 15) / 16 * 16 + 4; }
+
+/* grid (chunk CTAs, 1, column blocks), 256 threads, LM >= ceil(d / 8), NT >= mt ksplit tiles per warp.  Per chunk of kShapQ term pairs, double-buffered
+ * with one barrier per chunk:
+ *   (A) thread (q, s) = (tid / 8, tid % 8) finds term pair q's (k, k'), writes U[q][s + 8 j] = w theta_kb theta_k'b
+ *       (w = 2 off the diagonal) from a.coeff = the coefficients transposed (B x K), and loads c_j, p_j of its segment
+ *       of inputs j = s L .. s L + L - 1, L = ceil(d / 8), into registers;
+ *   (B) per node z_i in ascending order: h_j = p_j + z_i c_j, the segment's prefix products in ascending j, the
+ *       segment products of the eight lanes exchanged by shuffles and multiplied in ascending (before the segment) and
+ *       descending (after it) lane order, then acc_j += w_i (pre_s suf_s) (lpre_j lsuf_j) with the segment's suffix
+ *       grown in descending j.  F[q][j] = c_j acc_j.  No division and no difference of products; the segments depend
+ *       on d alone, so a factor is the same bits whichever thread forms it;
+ *   (C) warp w = (kg, wg) contracts its tiles t = wg, wg + 8 / ksplit, ... (row tile t % mt, column tile t / mt, the
+ *       column tiles holding live columns) over its group's k-steps, one DMMA per tile and k-step.
+ * Each D element depends on its own A row and B column only and the chunks and k-steps follow in an order fixed by K
+ * and d, so column b's result does not depend on the other columns.  The CTA's sum goes to
+ * partial[(b d + l) gridDim.x + blockIdx.x], added in index order by colsum_partials_kernel. */
+template <int LM, int NT>
+__global__ void __launch_bounds__(kSobolThreads) sobol_shapley_kernel(SobolShapleyArgs sa) {
+  extern __shared__ double sm[];
+  const SobolFormsArgs& a = sa.f;
+  const int d = a.d, n = sa.n;
+  const u64 K = (u64)a.K;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, k4 = lane & 3;
+  const u64 b0 = (u64)blockIdx.z * kShapCols;
+  const int bc = a.B - b0 < (u64)kShapCols ? (int)(a.B - b0) : kShapCols;
+  const int mt = (d + 7) / 8, FS = shapley_fs(mt), ntile = mt * ((bc + 7) / 8);
+  const int ksplit = shapley_ksplit(mt), nwg = 8 / ksplit, kg = warp / nwg, wg = warp % nwg;
+  double* F = sm;                                   /* 2 x kShapQ x FS */
+  double* U = F + 2 * kShapQ * FS;                  /* 2 x kShapQ x kShapUS */
+  double* zw = U + 2 * kShapQ * kShapUS;            /* 2 n */
+  const double* mu = a.mu;
+  const double* cov = a.cov;
+  if (a.staged) {
+    double* tab = zw + 2 * n;
+    for (int i = tid; i < a.mu_n; i += kSobolThreads) tab[i] = a.mu[i];
+    for (int i = tid; i < a.c_n; i += kSobolThreads) tab[a.mu_n + i] = a.cov[i];
+    mu = tab; cov = tab + a.mu_n;
+  }
+  for (int i = tid; i < 2 * n; i += kSobolThreads) zw[i] = sa.nodes[i];
+  for (int i = tid; i < 2 * kShapQ * FS; i += kSobolThreads) F[i] = 0.0; /* rows d .. 8 mt - 1 stay zero */
+  const int q = tid >> 3, s = tid & 7;
+  const int L = (d + 7) / 8, j0 = s * L;
+  const int ns = d - j0 < 0 ? 0 : d - j0 < L ? d - j0 : L;
+  double acc[NT][2];
+#pragma unroll
+  for (int i = 0; i < NT; ++i) acc[i][0] = acc[i][1] = 0.0;
+  __syncthreads();
+
+  int buf = 0;
+  for (u64 ch = blockIdx.x; ch < a.nchunks; ch += gridDim.x, buf ^= 1) {
+    double* Fb = F + buf * kShapQ * FS;
+    double* Ub = U + buf * kShapQ * kShapUS;
+    /* (A) */
+    const u64 qq = ch * kShapQ + q;
+    int k = -1, k2 = -1;
+    if (qq < a.npairs) {
+      u64 kk, kk2;
+      sobol_pair(qq, K, &kk, &kk2);
+      k = (int)kk; k2 = (int)kk2;
+    }
+#pragma unroll
+    for (int j = 0; j < kShapCols / 8; ++j) {
+      const int b = s + 8 * j;
+      double u = 0.0;
+      if (k >= 0 && b < bc) u = (k == k2 ? 1.0 : 2.0) * (a.coeff[(u64)k * a.B + b0 + b] * a.coeff[(u64)k2 * a.B + b0 + b]);
+      Ub[q * kShapUS + b] = u;
+    }
+    double c[LM], p[LM], lpre[LM], f[LM];
+#pragma unroll
+    for (int j = 0; j < LM; ++j) {
+      c[j] = p[j] = f[j] = 0.0;
+      if (j < ns && k >= 0) {
+        const int l = j0 + j;
+        const SobolDim D = a.dims[l];
+        const int t1 = (int)a.terms[k + l * K], t2 = (int)a.terms[k2 + l * K];
+        p[j] = mu[D.mu_off + t1] * mu[D.mu_off + t2];
+        c[j] = cov[D.c_off + t1 + D.mo * t2];
+      }
+    }
+    /* (B) */
+    for (int i = 0; i < n; ++i) {
+      const double z = zw[i], w = zw[n + i];
+      double x = 1.0;
+#pragma unroll
+      for (int j = 0; j < LM; ++j)
+        if (j < ns) { lpre[j] = x; x *= fma(z, c[j], p[j]); }
+      double pre = 1.0, suf = 1.0;
+#pragma unroll
+      for (int t = 0; t < 8; ++t) {
+        const double v = __shfl_sync(0xffffffffu, x, (lane & ~7) | t);
+        if (t < s) pre *= v;
+      }
+#pragma unroll
+      for (int t = 7; t >= 0; --t) {
+        const double v = __shfl_sync(0xffffffffu, x, (lane & ~7) | t);
+        if (t > s) suf *= v;
+      }
+      const double ww = w * (pre * suf);
+      double y = 1.0;
+#pragma unroll
+      for (int j = LM - 1; j >= 0; --j)
+        if (j < ns) { f[j] = fma(ww, lpre[j] * y, f[j]); y *= fma(z, c[j], p[j]); }
+    }
+#pragma unroll
+    for (int j = 0; j < LM; ++j)
+      if (j < ns) Fb[q * FS + j0 + j] = c[j] * f[j];
+    __syncthreads();
+    /* (C) */
+    for (int ks = kg; ks < kShapQ / 4; ks += ksplit) {
+      const double* Fk = Fb + (ks * 4 + k4) * FS + g;
+      const double* Uk = Ub + (ks * 4 + k4) * kShapUS + g;
+#pragma unroll
+      for (int i = 0; i < NT; ++i) {
+        const int t = wg + nwg * i;
+        if (t < ntile) dmma_f64(acc[i][0], acc[i][1], Fk[(t % mt) * 8], Uk[(t / mt) * 8]);
+      }
+    }
+  }
+  /* the k-step groups, added in kg order through shared memory (F and U are free once every warp is past its last
+   * contraction); C fragment: lane (g, k4) holds row 8 (t % mt) + g, columns 8 (t / mt) + 2 k4 + e */
+  __syncthreads();
+  double* red = sm; /* (ksplit - 1) x 8 mt tiles x 64: at most 7 x 8 x 64 doubles, below F and U's 2 kShapQ (20 + 68) */
+  if (kg > 0) {
+#pragma unroll
+    for (int i = 0; i < NT; ++i) {
+      const int t = wg + nwg * i;
+      if (t < ntile) {
+        double* r = red + ((size_t)(kg - 1) * 8 * mt + t) * 64 + 2 * lane;
+        r[0] = acc[i][0]; r[1] = acc[i][1];
+      }
+    }
+  }
+  __syncthreads();
+  if (kg > 0) return;
+#pragma unroll
+  for (int i = 0; i < NT; ++i) {
+    const int t = wg + nwg * i;
+    if (t >= ntile) continue;
+    for (int gg = 1; gg < ksplit; ++gg) {
+      const double* r = red + ((size_t)(gg - 1) * 8 * mt + t) * 64 + 2 * lane;
+      acc[i][0] += r[0]; acc[i][1] += r[1];
+    }
+    const int l = (t % mt) * 8 + g;
+    if (l >= d) continue;
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const int b = (t / mt) * 8 + 2 * k4 + e;
+      if (b < bc) a.partial[((b0 + b) * (u64)d + l) * gridDim.x + blockIdx.x] = acc[i][e];
+    }
+  }
+}
+
+static u64 sobol_shapley_chunks(u64 K) { return (K * (K + 1) / 2 + kShapQ - 1) / kShapQ; }
+u64 sobol_shapley_partials(u64 K) { return std::max<u64>(1, std::min<u64>(sobol_shapley_chunks(K), kShapCTAs)); }
+
+void launch_sobol_shapley(Ctx& c, const u64* terms, u64 K, u64 d, const SobolDim* dims_dev, const double* mu, u64 mu_n,
+                          const double* cov, u64 c_n, const double* coeff_t, u64 B, const double* nodes, u64 n,
+                          double* partial, double* out) {
+  if (K == 0 || B == 0 || d == 0) return;
+  if (K > 0x7FFFFFFFull) throw std::range_error("sobol_shapley: more terms than the Shapley kernel indexes");
+  if (d > 8 * kShapTiles) throw std::range_error("sobol_shapley: the model has more dimensions than the Shapley kernel holds");
+  const u64 nz = (B + kShapCols - 1) / kShapCols;
+  if (nz > 65535 || B * d > 0x7FFFFFFFull) throw std::range_error("sobol_shapley: too many coefficient columns for one call");
+  SobolShapleyArgs sa{};
+  SobolFormsArgs& a = sa.f;
+  a.terms = terms; a.K = (int)K; a.d = (int)d; a.dims = dims_dev;
+  a.mu = mu; a.cov = cov; a.mu_n = (int)mu_n; a.c_n = (int)c_n;
+  a.coeff = coeff_t; a.B = B;
+  a.npairs = K * (K + 1) / 2; a.nchunks = sobol_shapley_chunks(K);
+  a.partial = partial;
+  sa.nodes = nodes; sa.n = (int)n;
+  const int mt = (int)(d + 7) / 8;
+  const size_t base = ((size_t)2 * kShapQ * (shapley_fs(mt) + kShapUS) + 2 * n) * sizeof(double);
+  const size_t tab = (mu_n + c_n) * sizeof(double);
+  a.staged = tab <= kSobolStageBytes && base + tab <= c.smem_optin;
+  const size_t smem = base + (a.staged ? tab : 0);
+  if (smem > c.smem_optin) throw std::range_error("sobol_shapley: the model has more dimensions than the Shapley kernel holds");
+  const unsigned nx = (unsigned)sobol_shapley_partials(K);
+  const dim3 grid(nx, 1, (unsigned)nz);
+  /* registers per thread follow the segment length ceil(d / 8) and the tiles per warp (8 up to mt = 4): 124 up to
+   * d = 24, two CTAs per SM; 246 above, one CTA per SM (a segment of 5 in 128 registers would spill) */
+  auto launch = [&](auto kernel) {
+    set_smem(kernel, smem);
+    kernel<<<grid, kSobolThreads, smem, c.stream>>>(sa);
+  };
+  if (d <= 16) launch(sobol_shapley_kernel<2, 8>);
+  else if (d <= 24) launch(sobol_shapley_kernel<3, 8>);
+  else launch(sobol_shapley_kernel<10, kShapTiles>);
+  check_launch(c, "sobol_shapley_kernel");
+  colsum_partials_kernel<<<(unsigned)(B * d), 32, 0, c.stream>>>(partial, (int)nx, out);
+  check_launch(c, "colsum_partials_kernel");
+}
+
 void launch_fill(Ctx& c, double* p, u64 n, double v) {
   if (n == 0) return;
   fill_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c.stream>>>(p, n, v);

@@ -21,8 +21,8 @@ on both.  Nothing N-sized happens in this file: every objective evaluation is
   obdraws                                 S joint posterior draws of a fitted model at new inputs (no reference
                                           counterpart)
   obsobol                                 Sobol first-order and total indices of a fitted model, exact from its
-                                          coefficients, optionally the second-order indices of every input pair, and
-                                          of S posterior draws (no reference counterpart)
+                                          coefficients, optionally the second-order indices of every input pair and
+                                          the Shapley effects, and of S posterior draws (no reference counterpart)
 """
 from __future__ import annotations
 
@@ -30,7 +30,7 @@ import math
 
 import numpy as np
 
-from .binding import gethyp, getpara, posterior_draws, sobol, sobol_pairs
+from .binding import gethyp, getpara, posterior_draws, sobol, sobol_pairs, sobol_shapley
 
 
 def _flatten(parlist):
@@ -458,12 +458,21 @@ def _pair_indices(r):
                                                                     ("supset", r["supset"]))}
 
 
-def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100, second=False):
+def _shapley_indices(r):
+    """shapley / var (d or d x B, adding up to 1); a column whose variance is 0 gets NaN"""
+    var = np.asarray(r["var"], dtype=float)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return np.where(var != 0, r["shapley"] / np.where(var != 0, var, 1.0), np.nan)
+
+
+def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100, second=False, shapley=False):
     """Sobol indices of the latent function of a model of obfit / obfit_gauss / obfit_multi under the product of the
     empirical marginals of x's columns (binding.sobol: exact quadratic forms in the fitted coefficients).  Returns first and
     total (the first-order and total indices, d or d x C), var (Var f in y's units, y_sca^2 var) and mean (y_cent +
     y_sca E f).  second=True adds, from binding.sobol_pairs, the input-pair indices second (pure second-order), closed
     (first_l + first_m + second_lm) and supset (superset importance), each d x d or d x d x C with NaN on the diagonal.
+    shapley=True adds, from binding.sobol_shapley, shapley: the Shapley effects over the variance (d or d x C), which
+    add up to 1 and lie between first and total.
     S > 0 adds `draws`: the same keys for each of S posterior draws (d x S, d x d x S, S), conditional on the
     hyper-parameters, terms and para (posterior_draws; single-response models only)."""
     logpdf = obmodel["logpdf"]
@@ -478,6 +487,8 @@ def obsobol(obmodel, x, S=0, seed=0, tol=0.001, maxepch=100, second=False):
         out = dict(first=first, total=total, var=y_sca ** 2 * r["var"], mean=y_cent + y_sca * r["mean"])
         if second:
             out.update(_pair_indices(r))
+        if shapley:
+            out["shapley"] = _shapley_indices(sobol_shapley(lib, om, terms, coeff, x))
         return out
 
     out = indices(logpdf.coeff)
